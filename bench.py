@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the two hot paths (contract in the task statement; metric from BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3] [--impl reference] [--no-extras]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3] [--impl reference] [--no-extras] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...      (N > 1)
 
 Primary line: Hamming mAP@k queries/s on the MS-COCO shape (BASELINE.json configs[2]: 5k queries x 117k database rows,
@@ -21,10 +21,13 @@ and exchanges the per-query results the same way: total work is fixed, so "scali
 `roofline`: the dominant kernel of the step, its stage time measured with CUDA events in an eager re-run of the same
             kernels on the same inputs (a graph replay cannot be timed stage by stage), plus flat copies of the numbers
             the other workloads produce (`c5_*`: BASELINE configs[4] at this N; `swt_*`: configs[0] / [3]).
-`extras`  : everything else (other Hamming shapes, cosine k-NN, SWT grid, DSCH metrics, DWT, fix_size) at N = 1.
+`extras`  : everything else (other Hamming shapes, cosine k-NN, SWT grid, DSCH metrics, DWT, fix_size) at N = 1, printed
+            as a JSON line of its own on stderr.
 `--impl reference` times the reference's own CPU implementation: the REAL ``CustomCalculator.calculate_maphashing`` loaded
 from /root/reference when that tree is readable (kind "reference"), else the literal torch restatement of it (kind "port";
 the reference's third-party stack is not installable offline, see DESIGN.md §3) — on a bounded query sample.
+`--dump-outputs DIR` writes what the last timed step of the main workload computed (map.npy, and the per-query ap.npy and
+hits.npy, float64); the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import ctypes
@@ -243,7 +246,19 @@ POPC_PER_PAIR = {1: 2, 2: 3, 4: 4}        # select kernel: carry-save adders in 
 XU_LANES_PER_CLK_PER_SM = 16.0              # POPC is a quarter-rate XU instruction (measured: tools/ubench_int.cu)
 
 
-def bench_map(name, args, world, rank, device, dist, engine, with_e2e=True, with_cpu=True, check=True):
+def dump_outputs(out_dir, engine, m):
+    """Write what the last timed step computed as ``out_dir/<name>.npy``: the mAP and the per-query AP and hit counts that
+    ``evaluate(details=True)`` hands a caller, read from the engine's result region after that step (float64)."""
+    st = engine._last
+    arrays = {"map": np.array([m], dtype=np.float64),
+              "ap": engine._result(st, st.off_ap, torch.float64, st.nq).cpu().numpy(),
+              "hits": engine._result(st, st.off_tsum, torch.int32, st.nq).cpu().numpy().astype(np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for key, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{key}.npy"), a)
+
+
+def bench_map(name, args, world, rank, device, dist, engine, with_e2e=True, with_cpu=True, check=True, dump_dir=None):
     """One Hamming-mAP workload through HammingMapEngine at this world size."""
     from image_retrieval_wavelet_b200 import _cabi
     from image_retrieval_wavelet_b200.engine.dist import shard_bounds
@@ -292,6 +307,8 @@ def bench_map(name, args, world, rank, device, dist, engine, with_e2e=True, with
     if dist is not None:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_per_step = float(t.item()) / args.steps
+    if dump_dir is not None and rank == 0:
+        dump_outputs(dump_dir, engine, out[0])
     # keep the GPU busy a little longer (about 0.25 s) so that the clock sampler sees the kernels under load; the count
     # comes from the all-reduced time, so every rank runs the SAME number of steps (they contain barriers)
     for _ in range(int(min(400, max(3, 250.0 / max(ms_per_step, 1e-3))))):
@@ -678,7 +695,7 @@ def run_own(args):
     from image_retrieval_wavelet_b200.engine.map_engine import HammingMapEngine
 
     engine = HammingMapEngine()
-    main = bench_map(args.workload, args, world, rank, device, dist, engine)
+    main = bench_map(args.workload, args, world, rank, device, dist, engine, dump_dir=args.dump_outputs)
     engine.close()
     small = argparse.Namespace(**{**vars(args), "steps": min(args.steps, 10)})
     flat = {}                     # scalar copies for the retained `roofline` object (the driver drops `extras`)
@@ -766,8 +783,12 @@ def run_own(args):
             "data": "synthetic", "config": main["config"], "clocks": main["clocks"], "e2e": main.get("e2e"),
             "gpu_launches": main["gpu_launches"], "roofline": roofline, "cpu_baseline": main.get("cpu_baseline"),
             "stage_ms": main["stage_ms"], "map": main["map"], "checked": main["checked"], "run": main["run"], "plan": main["plan"],
-            "steps_redone_with_full_sequence": main["steps_redone_with_full_sequence"], "scaleout": scaleout, "extras": extras,
+            "steps_redone_with_full_sequence": main["steps_redone_with_full_sequence"], "scaleout": scaleout,
         }
+        if extras:
+            # about 14 KB: on a line of their own (stderr), so that readers with a line-length limit still parse the result
+            # line; `roofline` keeps flat copies of their headline figures
+            print(json.dumps({"extras": extras}), file=sys.stderr)
         print(json.dumps(line))
     if dist is not None:
         dist.barrier()
@@ -782,7 +803,11 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="c3", choices=sorted(WORKLOADS))
     ap.add_argument("--no-extras", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step of the main workload as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
     if args.impl == "reference":
         run_reference(args)
     else:

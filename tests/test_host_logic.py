@@ -150,7 +150,8 @@ class _FakeDataset:
 
 def test_build_fast_eval_subset_mirror():
     """batch_map.py:39-91: deterministic, de-duplicated, at most `size` images, groups below min_per_class skipped; against
-    the reference's own function when /root/reference is readable."""
+    the recorded selections of tests/golden/subset_golden.npz, and against the reference's own function when its tree is
+    readable."""
     from image_retrieval_wavelet_b200.engine import build_fast_eval_subset
 
     ds = _FakeDataset(300, 12, 1)
@@ -163,6 +164,10 @@ def test_build_fast_eval_subset_mirror():
         build_fast_eval_subset(ds, 8, min_per_class=10 ** 6)
     with pytest.raises(AttributeError):
         build_fast_eval_subset(object(), 8)
+    want = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "subset_golden.npz"))
+    for size, seed in ((64, 3), (17, 0), (10 ** 6, 9)):
+        got = [ds.paths.index(p) for p in build_fast_eval_subset(ds, size, seed=seed).paths]
+        assert got == want[f"size{size}_seed{seed}"].tolist(), (size, seed)
     from oracle import ref_loader
 
     if ref_loader.available():
