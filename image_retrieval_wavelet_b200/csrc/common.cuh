@@ -61,6 +61,22 @@ __host__ __device__ constexpr T round_up(T a, T b) {
     return ceil_div(a, b) * b;
 }
 
+// ---- order-preserving float -> uint32 key of the k-NN selections: a larger key ranks first.  largest: larger floats get
+// larger keys, else smaller floats do.  -0.0 folds into +0.0, so equal scores are ordered by index alone, and NaN gets
+// key 0, the worst in either direction (no number maps to 0 or its complement).
+__device__ __forceinline__ uint32_t rank_key(float f, bool largest) {
+    if (f != f) return 0u;
+    const uint32_t u = __float_as_uint(f + 0.f);          // -0.0 + 0.0 = +0.0 (IEEE, round to nearest)
+    const uint32_t m = (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+    return largest ? m : ~m;
+}
+// the score of a key (key 0: NaN; -0.0 comes back as +0.0)
+__device__ __forceinline__ float rank_key_inv(uint32_t key, bool largest) {
+    if (key == 0u) return __uint_as_float(0x7fffffffu);
+    const uint32_t m = largest ? key : ~key;
+    return __uint_as_float((m & 0x80000000u) ? (m & 0x7fffffffu) : ~m);
+}
+
 // ---- streaming global accesses (read-once inputs / write-once outputs must not pollute L1)
 __device__ __forceinline__ uint4 ldg_stream_u4(const void *p) {
     uint4 r;

@@ -98,21 +98,13 @@ __global__ void __launch_bounds__(256) knn_scores_kernel(const float *__restrict
             const long long n = n0 + tx * 8 + j;
             if (n >= N) continue;
             float v = acc[i][j];
-            if (l2) v = sqrtf(fmaxf(qn[m] + rn[n] - 2.f * v, 0.f));
+            if (l2) {
+                const float d2 = qn[m] + rn[n] - 2.f * v;
+                v = d2 != d2 ? d2 : sqrtf(fmaxf(d2, 0.f));        // fmaxf would turn NaN into distance 0
+            }
             S[static_cast<size_t>(m) * ldS + n] = v;
         }
     }
-}
-
-// order-preserving float -> uint32 (larger float <=> larger key); NaN sorts last for "largest first"
-__device__ __forceinline__ uint32_t mono_key(float f) {
-    if (f != f) return 0u;
-    const uint32_t u = __float_as_uint(f);
-    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-__device__ __forceinline__ float mono_inv(uint32_t k) {
-    const uint32_t u = (k & 0x80000000u) ? (k & 0x7fffffffu) : ~k;
-    return __uint_as_float(u);
 }
 
 // MSB-first radix select, one digit: given the 256-bin histogram of the keys that still match the prefix, the largest
@@ -146,8 +138,8 @@ __device__ __forceinline__ void radix_pick_digit(const uint32_t *hist, uint32_t 
     }
 }
 
-// One CTA (256 threads) per query row: the k largest keys (key = mono(score), or ~mono(distance) for L2), ties to
-// the smaller index, sorted best-first.
+// One CTA (256 threads) per query row: the k largest keys (rank_key: larger scores first, or smaller distances for L2;
+// NaN last), ties to the smaller index, sorted best-first.
 // Lists longer than kKnnMaxK come out in passes of <= kKnnMaxK ranks: pass p only sees the entries that rank strictly
 // after the last entry of pass p - 1 (k_done > 0: that entry is idx_out / score_out[k_done - 1] of the row), writes ranks
 // k_done .. k_done + k - 1 of the ldo-wide output rows.  gate (or null): the launch does nothing while *gate == 0.
@@ -171,17 +163,13 @@ __global__ void __launch_bounds__(256) knn_select_kernel(const float *__restrict
     // legal key (NaN), so eligibility is carried separately
     unsigned long long bound = ~0ull;                     // exclusive upper bound on (key << 32 | ~idx)
     if (k_done > 0) {
-        const uint32_t bu = mono_key(orow_score[-1]);
-        bound = (static_cast<unsigned long long>(l2 ? ~bu : bu) << 32) | (0xffffffffu - static_cast<uint32_t>(orow_idx[-1]));
+        bound = (static_cast<unsigned long long>(rank_key(orow_score[-1], !l2)) << 32) | (0xffffffffu - static_cast<uint32_t>(orow_idx[-1]));
     }
     const uint32_t bkey = static_cast<uint32_t>(bound >> 32), bnidx = static_cast<uint32_t>(bound);
     auto eligible = [&](uint32_t u, long long n) {
         return k_done == 0 || u < bkey || (u == bkey && (0xffffffffu - static_cast<uint32_t>(n)) < bnidx);
     };
-    auto key_of = [&](long long n) {
-        const uint32_t u = mono_key(row[n]);
-        return l2 ? ~u : u;
-    };
+    auto key_of = [&](long long n) { return rank_key(row[n], !l2); };
     // ---- fast path: a threshold from a sorted sample that, with overwhelming probability, is not above the k-th
     // largest key and admits at most kKnnCand candidates; ONE pass over the row collects every key >= threshold, the
     // candidates are sorted exactly (ties by index).  Any miss (too few / too many candidates) falls through to the
@@ -229,8 +217,7 @@ __global__ void __launch_bounds__(256) knn_select_kernel(const float *__restrict
                 const float e[4] = {v[b].x, v[b].y, v[b].z, v[b].w};
 #pragma unroll
                 for (int j = 0; j < 4; ++j) {
-                    const uint32_t u = mono_key(e[j]);
-                    keys[4 * b + j] = l2 ? ~u : u;
+                    keys[4 * b + j] = rank_key(e[j], !l2);
                     if (base + b * 256 < n4 && keys[4 * b + j] >= thr && eligible(keys[4 * b + j], 4 * (base + b * 256) + j))
                         mask |= 1u << (4 * b + j);
                 }
@@ -300,7 +287,7 @@ __global__ void __launch_bounds__(256) knn_select_kernel(const float *__restrict
                 const unsigned long long pr = s_top[i];
                 const uint32_t u = static_cast<uint32_t>(pr >> 32);
                 orow_idx[i] = static_cast<int64_t>(0xffffffffu - static_cast<uint32_t>(pr));
-                orow_score[i] = mono_inv(l2 ? ~u : u);
+                orow_score[i] = rank_key_inv(u, !l2);
             }
             return;
         }
@@ -384,7 +371,7 @@ __global__ void __launch_bounds__(256) knn_select_kernel(const float *__restrict
         const uint32_t u = static_cast<uint32_t>(pr >> 32);
         const uint32_t n = 0xffffffffu - static_cast<uint32_t>(pr);
         orow_idx[i] = static_cast<int64_t>(n);
-        orow_score[i] = mono_inv(l2 ? ~u : u);
+        orow_score[i] = rank_key_inv(u, !l2);
     }
 }
 
@@ -453,7 +440,7 @@ __global__ void __launch_bounds__(256) knn_select_cand_kernel(const unsigned lon
     for (int i = tid; i < k; i += 256) {
         const unsigned long long pr = s_top[i];
         idx_out[static_cast<size_t>(blockIdx.x) * k + i] = static_cast<int64_t>(0xffffffffu - static_cast<uint32_t>(pr));
-        score_out[static_cast<size_t>(blockIdx.x) * k + i] = mono_inv(static_cast<uint32_t>(pr >> 32));
+        score_out[static_cast<size_t>(blockIdx.x) * k + i] = rank_key_inv(static_cast<uint32_t>(pr >> 32), true);
     }
 }
 

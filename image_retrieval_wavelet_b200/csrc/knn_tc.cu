@@ -65,12 +65,6 @@ struct TcFilter {
     const uint32_t *gate;            // or null: when given and zero the kernel returns at once (fallback launches)
 };
 
-__device__ __forceinline__ uint32_t tc_mono_key(float f) {       // order-preserving float -> uint32 (as knn.cu: mono_key)
-    if (f != f) return 0u;
-    const uint32_t u = __float_as_uint(f);
-    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-
 __global__ void __launch_bounds__(kTcThreads, 1) knn_scores_tc_kernel(const __grid_constant__ TcMaps maps, float *__restrict__ S,
                                                                        int M, long long N, long long ldS, int Dp,
                                                                        const TcFilter filt) {
@@ -177,7 +171,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) knn_scores_tc_kernel(const __gr
                                 if ((hit >> j) & 1u) {
                                     if (pos < filt.cap)
                                         filt.cand[static_cast<size_t>(m) * filt.cap + pos] =
-                                            (static_cast<unsigned long long>(tc_mono_key(__uint_as_float(r[j]))) << 32) |
+                                            (static_cast<unsigned long long>(rank_key(__uint_as_float(r[j]), true)) << 32) |
                                             (0xffffffffu - static_cast<uint32_t>(nb + j));
                                     ++pos;
                                 }

@@ -4,7 +4,9 @@
 keeps the reference's signature and return order ``(indices, distances)``; ``with_faiss`` is accepted and ignored
 (there is one implementation).  "hamming"/"cosine" rank by inner product, largest first; anything else by L2 distance,
 smallest first — exactly the branches of ``get_knn_torch`` (:60-71) / ``get_knn_faiss`` (:27-57).  Ties go to the smaller
-index (torch.topk / faiss leave the tie order unspecified).
+index (torch.topk / faiss leave the tie order unspecified).  -0.0 and +0.0 are the same score (reported as +0.0), and a
+NaN score or distance ranks after every number for both metrics.  ±inf coordinates are supported for L2 only: the
+inner-product scorer's bf16 hi/lo split turns them into NaN (inf - inf).
 """
 import logging
 
@@ -86,7 +88,7 @@ def get_knn(references, queries, num_k, embeddings_come_from_same_source, with_f
 
 def select_topk(scores, k, largest=True):
     """Row-wise top-k of a float32 device matrix by ``b200_select_topk_f32``: ``(values [Q, k], columns int64 [Q, k])``,
-    ties to the smaller column."""
+    ties to the smaller column; -0.0 equals +0.0 and NaN ranks last for either ``largest``."""
     _cabi.require_cuda()
     s = torch.as_tensor(scores)
     if s.dim() != 2 or not s.is_cuda:
@@ -117,8 +119,12 @@ def merge_knn_shards(shard_scores, shard_indices, num_k, distance_metric="l2"):
     cat_s = sc.permute(1, 0, 2).reshape(q, n_sh * ks).contiguous().float()
     cat_i = ix.permute(1, 0, 2).reshape(q, n_sh * ks).contiguous()
     largest = distance_metric in ("hamming", "cosine")
-    pad = torch.finfo(torch.float32).min if largest else torch.finfo(torch.float32).max
-    cat_s = torch.where(cat_i < 0, torch.full_like(cat_s, pad), cat_s)                 # negative index = padding of a short shard
+    # negative index = padding of a short shard.  No score ranks after a real NaN, so the padding moves behind every real
+    # entry (a stable sort keeps their order) and reads as NaN: ties go to the smaller column, so it is never chosen
+    # while a real entry remains.
+    order = torch.sort((cat_i < 0).to(torch.uint8), dim=1, stable=True).indices
+    cat_s, cat_i = torch.gather(cat_s, 1, order), torch.gather(cat_i, 1, order)
+    cat_s = cat_s.masked_fill(cat_i < 0, float("nan"))
     val, col = select_topk(cat_s, num_k, largest)
     return torch.gather(cat_i, 1, col), val
 

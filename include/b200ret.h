@@ -284,7 +284,9 @@ int b200_curve_accumulate(const uint32_t *cum, int Q, long long k, const uint8_t
 
 /* Continuous-embedding k-NN, get_knn.py:9-24,60-71: top-k by inner product (cosine / "hamming" metrics,
  * largest first) or by L2 distance (smallest first), ties by index.  refs float32 [N][D], queries float32
- * [Q][D] device; idx int64 [Q][k], score float32 [Q][k] (inner product, or L2 distance). */
+ * [Q][D] device; idx int64 [Q][k], score float32 [Q][k] (inner product, or L2 distance).  -0.0 equals +0.0 (reported
+ * as +0.0); a NaN score or distance ranks after every number for both metrics.  +-inf coordinates: L2 only (the
+ * tensor-core scorer's bf16 hi/lo split makes an inner product with them NaN). */
 size_t b200_knn_workspace_bytes(int Q, long long N, int D, int k);
 int b200_knn_topk(const float *refs, const float *queries, int Q, long long N, int D, int k, int metric_l2,
                   int64_t *idx, float *score, void *workspace, size_t workspace_bytes, b200_stream_t stream);
@@ -337,7 +339,8 @@ int b200_comm_destroy(b200_comm *comm);
 
 /* Top-k of every row of a float32 matrix on the device (row stride ldS, a multiple of 4; 16-byte aligned base):
  * idx int64 [Q][k] = column numbers, score float32 [Q][k]; largest != 0: largest first, else smallest first; ties to
- * the smaller column; any k <= N.  The merge step of the database-sharded k-NN (get_knn.py:41-44: faiss merges its
+ * the smaller column, -0.0 equals +0.0 (reported as +0.0), NaN ranks after every number for either `largest`;
+ * any k <= N.  The merge step of the database-sharded k-NN (get_knn.py:41-44: faiss merges its
  * shards on the host): per-shard (score, index) lists concatenated in shard order are such a matrix. */
 int b200_select_topk_f32(const float *S, int Q, long long N, long long ldS, int k, int largest, int64_t *idx, float *score,
                          b200_stream_t stream);

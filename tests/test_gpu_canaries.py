@@ -99,15 +99,28 @@ def test_select_pool_overflow_stays_inside_the_pool(monkeypatch):
     assert int(ts.view(torch.int32)[3]) == hits and abs(float(ap.view(torch.float64)[3]) - want) <= 1e-6
 
 
-@pytest.mark.parametrize("fused,k,n", [("1", 1000, 70000), ("0", 1000, 70000), ("1", 5000, 20000)])
-def test_knn_topk_stays_inside_its_buffers(monkeypatch, fused, k, n):
+@pytest.mark.parametrize("fused,k,n,top_tie", [pytest.param("1", 1000, 70000, False, id="1-1000-70000"),
+                                               pytest.param("0", 1000, 70000, False, id="0-1000-70000"),
+                                               pytest.param("1", 5000, 20000, False, id="1-5000-20000"),
+                                               pytest.param("1", 2048, 70001, True, id="1-2048-70001-top_tie")])
+def test_knn_topk_stays_inside_its_buffers(monkeypatch, fused, k, n, top_tie):
+    """top_tie: every 7th row is the best row of every query (integer inputs, 10 001 exact ties): the fused path's
+    candidate lists and the select kernel's candidate buffer overflow, and the fallbacks run."""
     from image_retrieval_wavelet_b200 import _cabi
 
     monkeypatch.setenv("B200_KNN_FUSED", fused)
     g = torch.Generator().manual_seed(n)
     nq, d = 70, 64
-    refs = torch.nn.functional.normalize(torch.randn(n, d, generator=g), dim=1).cuda()
-    qs = torch.nn.functional.normalize(torch.randn(nq, d, generator=g), dim=1).cuda()
+    if top_tie:
+        refs = torch.randint(-3, 4, (n, d), generator=g).float()
+        qs = torch.randint(-3, 4, (nq, d), generator=g).float()
+        qs[:, 0] = 100
+        refs[::7] = 0
+        refs[::7, 0] = 100
+        refs, qs = refs.cuda(), qs.cuda()
+    else:
+        refs = torch.nn.functional.normalize(torch.randn(n, d, generator=g), dim=1).cuda()
+        qs = torch.nn.functional.normalize(torch.randn(nq, d, generator=g), dim=1).cuda()
     lib = _cabi.load()
     nbytes = lib.b200_knn_workspace_bytes(nq, n, d, k)
     ws, idx, score = Guarded(nbytes), Guarded(nq * k * 8), Guarded(nq * k * 4)
@@ -117,6 +130,8 @@ def test_knn_topk_stays_inside_its_buffers(monkeypatch, fused, k, n):
     assert ws.intact() and idx.intact() and score.intact(), "b200_knn_topk wrote outside a buffer"
     want = torch.topk(qs.double() @ refs.double().T, k, dim=1).values
     assert (score.view(torch.float32).reshape(nq, k).double() - want).abs().max().item() <= 1e-5
+    if top_tie:                                            # the tied rows in index order
+        assert torch.equal(idx.view(torch.int64).reshape(nq, k).cpu(), torch.arange(0, 7 * k, 7).expand(nq, k))
 
 
 @pytest.mark.parametrize("rw", ["0", "1", "2"])
