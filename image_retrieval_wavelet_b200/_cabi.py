@@ -46,6 +46,9 @@ SIGNATURES = {
     "b200_swt2_fwd_host": (c_int, [c_void_p, c_int, c_int, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_int, c_int]),
     "b200_resize_workspace_bytes": (c_size_t, [c_ll, c_int, c_int, c_int, c_int, c_int]),
     "b200_resize_u8": (c_int, [c_void_p, c_void_p, c_ll, c_int, c_int, c_int, c_int, c_int, c_void_p, c_size_t, c_void_p]),
+    "b200_resize_crop_workspace_bytes": (c_size_t, [c_int, c_void_p, c_int, c_int, c_int, c_int]),
+    "b200_resize_crop_u8": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_size_t,
+                                    c_void_p]),
     "b200_dwt2_workspace_bytes": (c_size_t, [c_ll, c_int, c_int, c_int, c_int]),
     "b200_dwt2_fwd": (c_int, [c_void_p, c_int, c_void_p, c_ll, c_int, c_int, c_void_p, c_void_p, c_int, c_int, c_void_p, c_size_t,
                               c_void_p]),

@@ -100,6 +100,23 @@ size_t b200_resize_workspace_bytes(long long planes, int H, int W, int Hout, int
 int b200_resize_u8(const uint8_t *in, uint8_t *out, long long planes, int H, int W, int Hout, int Wout, int filter,
                    void *workspace, size_t workspace_bytes, b200_stream_t stream);
 
+/* Resize + crop of a ragged batch of decoded images in one launch: the eval transform Resize(256) -> CenterCrop(224)
+ * (config/transform/basic_swt.yaml) applied to every image, bit-identical to torchvision on PIL images.
+ * in           : device; image i is HWC-interleaved uint8 [H_i][W_i][C] (row pitch W_i * C bytes) at byte
+ *                offsets_host[i] of `in`.  `in` and every offset must be multiples of 4 (B200_ERR_ALIGNMENT).
+ * geom_host    : HOST int [n][6] = H, W, RH, RW, top, left per image: the resized size (Pillow's Image.resize with
+ *                `filter`, exactly as b200_resize_u8) and the crop origin inside it; 0 <= top <= RH - Hc and
+ *                0 <= left <= RW - Wc (B200_ERR_INVALID_ARG otherwise).  The size and crop rules of torchvision stay with
+ *                the caller.
+ * out          : device uint8 [n][C][Hc][Wc] (planar, the layout b200_swt2_fwd takes);  C in 1..4.
+ * workspace    : device scratch of b200_resize_crop_workspace_bytes() (per-image descriptors and the weight tables of the
+ *                crop windows, built on the host per call and copied with one H2D copy).
+ * B200_ERR_UNSUPPORTED when a window is wider than 64 taps (a reduction of more than ~31x bilinear / ~15x bicubic).
+ * n = 0 is a no-op; the workspace query returns 0 for n < 1 and for arguments the call rejects. */
+size_t b200_resize_crop_workspace_bytes(int n, const int *geom_host, int C, int Hc, int Wc, int filter);
+int b200_resize_crop_u8(const uint8_t *in, const long long *offsets_host, const int *geom_host, int n, int C, int Hc, int Wc,
+                        int filter, uint8_t *out, void *workspace, size_t workspace_bytes, b200_stream_t stream);
+
 /* ---- the decimated transform next to the SWT (SURVEY.md §8 f4)
  * DWTTransform._apply_wavelet, main/transforms/custom_transforms.py:196-200: pywt.wavedec2(channel, wavelet, level)
  * in PyWavelets' default 'symmetric' mode, keeping the coarsest level: out [planes][4][H_L][W_L] = (cA, cH, cV, cD),
