@@ -82,22 +82,18 @@ struct HostLoadTile {
 template <int F>
 static void run_swt_level(const SwtGeom &g, const void *in, float *out, SwtTileId id, float *smem, HostExec ex) {
     switch (g.level) {
-        case 1:
-            if (g.rw == 1) swt_tile_program<F, 1, 1, 0>(g, in, out, id, smem, ex, HostStore{}, HostLoad{});
-            else if (g.rw == 2) (g.vs ? swt_tile_program<F, 1, 2, 1>(g, in, out, id, smem, ex, HostStore{}, HostLoad{}) : swt_tile_program<F, 1, 2, 0>(g, in, out, id, smem, ex, HostStore{}, HostLoad{}));
-            else (g.vs ? swt_tile_program<F, 1, 0, 1>(g, in, out, id, smem, ex, HostStore{}, HostLoad{}) : swt_tile_program<F, 1, 0, 0>(g, in, out, id, smem, ex, HostStore{}, HostLoad{}));
-            break;
-        case 2:
-            if (g.rw == 1) swt_tile_program<F, 2, 1, 0>(g, in, out, id, smem, ex, HostStore{}, HostLoad{});
-            else if (g.rw == 2) (g.vs ? swt_tile_program<F, 2, 2, 1>(g, in, out, id, smem, ex, HostStore{}, HostLoad{}) : swt_tile_program<F, 2, 2, 0>(g, in, out, id, smem, ex, HostStore{}, HostLoad{}));
-            else (g.vs ? swt_tile_program<F, 2, 0, 1>(g, in, out, id, smem, ex, HostStore{}, HostLoad{}) : swt_tile_program<F, 2, 0, 0>(g, in, out, id, smem, ex, HostStore{}, HostLoad{}));
-            break;
-        case 3:
-            if (g.rw == 1) swt_tile_program<F, 3, 1, 0>(g, in, out, id, smem, ex, HostStore{}, HostLoad{});
-            else if (g.rw == 2) (g.vs ? swt_tile_program<F, 3, 2, 1>(g, in, out, id, smem, ex, HostStore{}, HostLoad{}) : swt_tile_program<F, 3, 2, 0>(g, in, out, id, smem, ex, HostStore{}, HostLoad{}));
-            else (g.vs ? swt_tile_program<F, 3, 0, 1>(g, in, out, id, smem, ex, HostStore{}, HostLoad{}) : swt_tile_program<F, 3, 0, 0>(g, in, out, id, smem, ex, HostStore{}, HostLoad{}));
-            break;
+        case 1: swt_tile_program<F, 1>(g, in, out, id, smem, ex, HostStore{}, HostLoad{}); break;
+        case 2: swt_tile_program<F, 2>(g, in, out, id, smem, ex, HostStore{}, HostLoad{}); break;
+        case 3: swt_tile_program<F, 3>(g, in, out, id, smem, ex, HostStore{}, HostLoad{}); break;
     }
+}
+
+// The pass form the launcher runs: swt_rw_form (-1: the generic program), swt_vs_form, and the uint8 staging units.
+static void swt_plan_forms(const SwtGeom &g, int *rw, int *vs, int *u8_stage) {
+    const bool fast = swt_fast_path(g.F, g.level);
+    *rw = fast ? swt_rw_form(g.F, g.level) : -1;
+    *vs = fast ? swt_vs_form(g.F, g.level) : 0;
+    *u8_stage = g.u8_stage;
 }
 
 template <int CW, int LW, bool EQ>
@@ -185,14 +181,14 @@ extern "C" {
 
 // Same planner, same tile programs as b200_swt2_fwd; host pointers.
 int sim_swt2_fwd(const void *in, int in_is_u8, float *out, int B, int C, int H, int W, const float *lo, const float *hi, int F,
-                 int level, int num_sms, int *plan_out /* TH, TW, vec, threads, run, RH, RWp or NULL */) {
+                 int level, int num_sms, int *plan_out /* TH, TW, rw form, threads, vs form, RH, RWp, u8_stage or NULL */) {
     SwtGeom g;
     const int rc = swt_plan(g, B, C, H, W, F, level, in_is_u8, lo, hi, num_sms);
     if (rc == -1) return B200_ERR_INVALID_ARG;
     if (rc) return B200_ERR_UNSUPPORTED;
     if (plan_out) {
-        plan_out[0] = g.TH, plan_out[1] = g.TW, plan_out[2] = 4, plan_out[3] = g.threads, plan_out[4] = kSwtR;
-        plan_out[5] = g.RH, plan_out[6] = g.RWp;
+        plan_out[0] = g.TH, plan_out[1] = g.TW, plan_out[3] = g.threads, plan_out[5] = g.RH, plan_out[6] = g.RWp;
+        swt_plan_forms(g, plan_out + 2, plan_out + 4, plan_out + 7);
     }
     std::vector<float> smem(swt_smem_bytes(g) / sizeof(float));
     std::vector<unsigned char> states;
@@ -220,15 +216,17 @@ int sim_swt2_fwd(const void *in, int in_is_u8, float *out, int B, int C, int H, 
 // The uint8 -> [0, 1] conversion of the staging phase (must equal b / 255.0f bit for bit).
 float sim_u8_unit(unsigned b) { return swt_u8_unit(b); }
 
-// Planner only: TH, TW, vec, threads, run, RH, RWp, smem bytes, CTAs.
+// Planner only: TH, TW, rw form, threads, vs form, RH, RWp, smem bytes, CTAs, u8_stage (forms: swt_plan_forms).
 int sim_swt2_plan(int B, int C, int H, int W, int F, int level, int in_is_u8, int num_sms, long long *plan_out) {
     SwtGeom g;
     float z[20] = {0};
     const int rc = swt_plan(g, B, C, H, W, F, level, in_is_u8, z, z, num_sms);
     if (rc) return rc;
-    plan_out[0] = g.TH, plan_out[1] = g.TW, plan_out[2] = 4, plan_out[3] = g.threads, plan_out[4] = kSwtR;
+    int rw, vs, u8_stage;
+    swt_plan_forms(g, &rw, &vs, &u8_stage);
+    plan_out[0] = g.TH, plan_out[1] = g.TW, plan_out[2] = rw, plan_out[3] = g.threads, plan_out[4] = vs;
     plan_out[5] = g.RH, plan_out[6] = g.RWp, plan_out[7] = static_cast<long long>(swt_smem_bytes(g));
-    plan_out[8] = static_cast<long long>(B) * C * g.tiles_y * g.tiles_x;
+    plan_out[8] = static_cast<long long>(B) * C * g.tiles_y * g.tiles_x, plan_out[9] = u8_stage;
     return 0;
 }
 

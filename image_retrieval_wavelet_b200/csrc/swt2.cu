@@ -121,29 +121,13 @@ __device__ __forceinline__ SwtTileId swt_block_tile() {
 }
 
 // Register budgets are part of the design: a 256-thread CTA at 64 registers fits 4 per SM, at 65-72 only 3 — measured
-// 0.74 vs 0.64 of the HBM roofline for haar level 2 — so F <= 4 is pinned to 64 registers and F = 6, 8 to 80 (F = 8 with 2 output rows per vertical unit; F = 10 spills there).
-template <int F, int LEVEL, int VS>
-__global__ void __launch_bounds__(256, (F <= 4 ? 4 : (F <= 8 ? ((VS && LEVEL == 1) ? 4 : 3) : 2))) swt2_tile_kernel(const __grid_constant__ SwtGeom g, const void *__restrict__ in,
-                                                           float *__restrict__ out) {
-    extern __shared__ __align__(16) float swt_smem[];
-    swt_tile_program<F, LEVEL, 0, VS>(g, in, out, swt_block_tile(), swt_smem, SwtDeviceExec{}, DevStore{}, DevLoad{});
-}
-
-// Register-window form (swt_rw_*): a unit keeps a window of F horizontally filtered rows and its output accumulators in
-// registers, so the budget is 128 registers at <= 256 threads (2 CTAs of 256, or 4 of 128, per SM).
+// 0.74 vs 0.64 of the HBM roofline for haar level 2 — so F <= 4 and the sliding F = 8 level-1 kernel are pinned to 64
+// registers and F = 6, 8 to 80 (F = 8 with 2 output rows per vertical unit; F = 10 spills there).
 template <int F, int LEVEL>
-__global__ void __launch_bounds__(256, 2) swt2_rw_kernel(const __grid_constant__ SwtGeom g, const void *__restrict__ in,
-                                                         float *__restrict__ out) {
+__global__ void __launch_bounds__(256, ((F <= 4 || swt_vs_form(F, LEVEL)) ? 4 : (F <= 8 ? 3 : 2)))
+    swt2_tile_kernel(const __grid_constant__ SwtGeom g, const void *__restrict__ in, float *__restrict__ out) {
     extern __shared__ __align__(16) float swt_smem[];
-    swt_tile_program<F, LEVEL, 1, 0>(g, in, out, swt_block_tile(), swt_smem, SwtDeviceExec{}, DevStore{}, DevLoad{});
-}
-
-// Register-window intermediate levels, two-pass last level: the budgets of the two-pass kernel.
-template <int F, int LEVEL, int VS>
-__global__ void __launch_bounds__(256, (F <= 4 ? 4 : (F <= 8 ? 3 : 2))) swt2_rwll_kernel(const __grid_constant__ SwtGeom g, const void *__restrict__ in,
-                                                                                          float *__restrict__ out) {
-    extern __shared__ __align__(16) float swt_smem[];
-    swt_tile_program<F, LEVEL, 2, VS>(g, in, out, swt_block_tile(), swt_smem, SwtDeviceExec{}, DevStore{}, DevLoad{});
+    swt_tile_program<F, LEVEL>(g, in, out, swt_block_tile(), swt_smem, SwtDeviceExec{}, DevStore{}, DevLoad{});
 }
 
 __global__ void __launch_bounds__(256) swt2_generic_kernel(const __grid_constant__ SwtGeom g, const void *__restrict__ in,
@@ -168,22 +152,23 @@ __global__ void __launch_bounds__(256) raw_stack_kernel(const void *__restrict__
 
 using swt_fn = void (*)(const SwtGeom, const void *, float *);
 
-template <int F, int VS>
-static swt_fn pick_level(int level, int rw) {
+// the fast-path kernel of (F, level): the only 15 instantiations of swt2_tile_kernel
+template <int F>
+static swt_fn pick_level(int level) {
     switch (level) {
-        case 1: return rw == 1 ? swt2_rw_kernel<F, 1> : swt2_tile_kernel<F, 1, VS>;
-        case 2: return rw == 1 ? swt2_rw_kernel<F, 2> : (rw == 2 ? swt2_rwll_kernel<F, 2, VS> : swt2_tile_kernel<F, 2, VS>);
-        case 3: return rw == 1 ? swt2_rw_kernel<F, 3> : (rw == 2 ? swt2_rwll_kernel<F, 3, VS> : swt2_tile_kernel<F, 3, VS>);
+        case 1: return swt2_tile_kernel<F, 1>;
+        case 2: return swt2_tile_kernel<F, 2>;
+        case 3: return swt2_tile_kernel<F, 3>;
     }
     return nullptr;
 }
-static swt_fn pick_swt(int F, int level, int rw, int vs) {
+static swt_fn pick_swt(int F, int level) {
     switch (F) {
-        case 2: return vs ? pick_level<2, 1>(level, rw) : pick_level<2, 0>(level, rw);
-        case 4: return vs ? pick_level<4, 1>(level, rw) : pick_level<4, 0>(level, rw);
-        case 6: return vs ? pick_level<6, 1>(level, rw) : pick_level<6, 0>(level, rw);
-        case 8: return vs ? pick_level<8, 1>(level, rw) : pick_level<8, 0>(level, rw);
-        case 10: return vs ? pick_level<10, 1>(level, rw) : pick_level<10, 0>(level, rw);
+        case 2: return pick_level<2>(level);
+        case 4: return pick_level<4>(level);
+        case 6: return pick_level<6>(level);
+        case 8: return pick_level<8>(level);
+        case 10: return pick_level<10>(level);
     }
     return nullptr;
 }
@@ -197,7 +182,7 @@ int swt2_launch(const void *in, int in_is_u8, float *out, int B, int C, int H, i
     const size_t smem = swt_smem_bytes(g);
     const long long planes = static_cast<long long>(B) * C;
     if (planes > 0x7fffffffll || g.tiles_y > 65535) return B200_ERR_UNSUPPORTED;
-    swt_fn fn = swt_fast_path(F, level) ? pick_swt(F, level, g.rw, g.vs) : swt2_generic_kernel;
+    swt_fn fn = swt_fast_path(F, level) ? pick_swt(F, level) : swt2_generic_kernel;
     if (!fn) return B200_ERR_UNSUPPORTED;
     B200_CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void *>(fn), cudaFuncAttributeMaxDynamicSharedMemorySize,
                                        static_cast<int>(smem)));

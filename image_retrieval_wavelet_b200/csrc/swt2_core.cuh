@@ -45,17 +45,23 @@ struct SwtGeom {
     int RH, RWp;             // staged rows, padded row stride in floats (multiple of 4)
     int RHv;                 // rows of the last level's horizontal outputs = TH + 2^(L-1) * (F-1)
     int threads;             // CTA size
-    int nbuf;                // generic program: 3 full buffers; fast program: buffer A + buffer B (off_b)
     int off_b;               // float offset of buffer B from the start of shared memory
-    int smem_floats;
     uint32_t m_load;         // multiply-high reciprocals of the unit -> row divisors (0: divisor 1)
     uint32_t m_load8;        // same for the uint8 staging units (8 buffer columns each)
-    int u8_stage;            // uint8 staging: 1 = 8-pixel units (default), 0 = the 4-pixel units shared with float32 (A/B)
-    int rw;                  // 1: register-window passes (swt_rw_*): no horizontal-pass planes in shared memory
-    int vs;                  // 1: sliding last vertical pass (swt_vpass_final_slide); TH % (kVsR * 2^(level-1)) == 0
+    int u8_stage;            // uint8 staging: 1 = 8-pixel units, 0 = the 4-pixel units shared with float32 (chosen from W)
     uint32_t m_lvl[kSwtMaxLevelFast];
     float lo[20], hi[20];
+    // host only, behind the taps: ptxas merges the kernels' tap loads at 16-byte boundaries of the parameter block, so
+    // lo / hi keep the offset (12 mod 16) the kernels were measured with
+    int nbuf;                // generic program: 3 full buffers; fast program: buffer A + buffer B (off_b)
+    int smem_floats;
 };
+
+// Pass form of the fast path, a function of (F, level) alone (measurements: swt2_plan.h, DESIGN.md §4.1).
+// 2: register-window intermediate levels (swt_rw_ll) + two-pass last level; 0: two-pass levels.
+__host__ __device__ constexpr int swt_rw_form(int F, int level) { return level >= 2 && F <= 4 ? 2 : 0; }
+// 1: sliding last vertical pass (swt_vpass_final_slide; TH % (kVsR * 2^(level-1)) == 0); 0: blocked (swt_vpass_final).
+__host__ __device__ constexpr int swt_vs_form(int F, int level) { return level == 1 && F == 8 ? 1 : 0; }
 
 __host__ __device__ __forceinline__ uint32_t swt_magic(uint32_t d) {      // host planner only (64-bit division)
     return d <= 1 ? 0u : static_cast<uint32_t>(((1ull << 32) + d - 1) / d);
@@ -411,7 +417,7 @@ __host__ __device__ __forceinline__ void swt_vpass_final(const SwtGeom &g, const
     }
 }
 
-// Sliding form of the last level's vertical pass (g.vs): a unit is 4 columns x kVsR output rows of one residue class of
+// Sliding form of the last level's vertical pass (swt_vs_form): a unit is 4 columns x kVsR output rows of one residue class of
 // ONE sub-band (band = 2 * (hh ? 1 : 0) + (dec_hi along H ? 1 : 0) = its output plane).  The unit walks its
 // kVsR + F - 1 source rows top to bottom through a register window of F rows: every row is loaded once per kVsR outputs
 // whatever F is (the blocked form above re-loads (R + F - 1) / R rows per output with R = 2 for the 8-tap filters: 4.5
@@ -475,12 +481,12 @@ __host__ __device__ __forceinline__ void swt_vpass_final_slide(const SwtGeom &g,
 }
 
 // ---------------------------------------------------------------------------------------------- register-window passes
-// One level as ONE pass: a unit is 4 adjacent columns x kRwR output rows of one residue class mod S.  The unit walks its
-// kRwR + F - 1 source rows top to bottom; each row is filtered horizontally in registers (aligned 128-bit shared loads,
-// FFMA2 over pixel pairs) into a window of the last F filtered rows, and every new row completes one output row, which
-// is filtered vertically straight out of that window.  The horizontal outputs never go to shared memory (the two-pass
-// form above stores and re-loads two planes of them per level, with the unit -> (row, column) index arithmetic of two
-// more sweeps), at the price of (kRwR + F - 1) / kRwR times the horizontal FMAs.
+// An intermediate level as ONE pass (swt_rw_form 2): a unit is 4 adjacent columns x kRwR output rows of one residue
+// class mod S.  The unit walks its kRwR + F - 1 source rows top to bottom; each row is filtered horizontally in registers
+// (aligned 128-bit shared loads, FFMA2 over pixel pairs) into a window of the last F filtered rows, and every new row
+// completes one output row, which is filtered vertically straight out of that window.  The horizontal outputs never go
+// to shared memory (the two-pass form above stores and re-loads a plane of them per level, with the unit -> (row,
+// column) index arithmetic of two more sweeps), at the price of (kRwR + F - 1) / kRwR times the horizontal FMAs.
 constexpr int kRwR = 8;
 
 // Keeps the compiler from hoisting the shared loads of later rows of a (fully unrolled) unit above this point: without
@@ -557,68 +563,6 @@ __host__ __device__ __forceinline__ void swt_rw_ll(const SwtGeom &g, const float
     }
 }
 
-// Last level: the four bands of the TH x TW tile straight from the level's input buffer to global memory.
-// src: RH x stride, buffer row `row_b0` / column `col_b0` = tile row / column 0.  Two sweeps per unit: the dec_lo rows
-// give cA, cH (planes 0, 1), the dec_hi rows cV, cD (planes 2, 3) — one 4-wide window at a time keeps the unit within
-// ~96 registers.
-template <int F, int S, bool ALIGNED, typename Store>
-__host__ __device__ __forceinline__ void swt_rw_final(const SwtGeom &g, const float *src, int stride, int row_b0, int col_b0,
-                                                      float *out_plane, int row_g0, int col_g0, int ncg, uint32_t magic,
-                                                      int tid, int nthreads, Store store) {
-    constexpr int R = kRwR;
-    const int nblk = g.TH / (S * R);
-    const uint32_t units = static_cast<uint32_t>(ncg) * S * nblk;
-    const size_t plane = static_cast<size_t>(g.H) * g.W;
-#pragma unroll 1
-    for (uint32_t u = tid; u < units; u += nthreads) {
-        const int rest = static_cast<int>(swt_div(u, magic));
-        const int cg = static_cast<int>(u) - rest * ncg;
-        const int rho = rest % S, b = rest / S;
-        const int o0 = rho + S * R * b;                     // first tile-local output row of the unit
-        const int gc = col_g0 + 4 * cg;
-        if (gc >= g.W || row_g0 + o0 >= g.H) continue;
-        const int n = g.W - gc >= 4 ? 4 : g.W - gc;          // W is even: n is 4 or 2
-        const int j0 = col_b0 + 4 * cg;
-        const float *base = src + (row_b0 + o0 - S * (F / 2 - 1)) * stride;
-#pragma unroll 1
-        for (int half = 0; half < 2; ++half) {
-            float f[F];                                  // this sweep's horizontal taps
-#pragma unroll
-            for (int t = 0; t < F; ++t) f[t] = half ? g.hi[t] : g.lo[t];
-            float win[F][4];
-#pragma unroll
-            for (int k = 0; k < R + F - 1; ++k) {
-                swt_rw_hrow<F, S>(base + S * k * stride, j0, f, win[k % F]);
-                if (k >= F - 1) {
-                    const int m = k - (F - 1);
-                    float a[4] = {0.f, 0.f, 0.f, 0.f}, d[4] = {0.f, 0.f, 0.f, 0.f};
-#pragma unroll
-                    for (int t = 0; t < F; ++t) {
-                        const float *x = win[(m + F - 1 - t) % F];
-                        swt_fma2<true>(g.lo[t], x[0], x[1], a[0], a[1]);      // lo along H
-                        swt_fma2<true>(g.lo[t], x[2], x[3], a[2], a[3]);
-                        swt_fma2<true>(g.hi[t], x[0], x[1], d[0], d[1]);      // hi along H
-                        swt_fma2<true>(g.hi[t], x[2], x[3], d[2], d[3]);
-                    }
-                    const int gr = row_g0 + o0 + S * m;
-                    if (gr < g.H) {
-                        // dec_lo along W: cA (LL) = plane 0, cH 'da' (LH) = plane 1; dec_hi along W: cV 'ad' (HL) = 2, cD (HH) = 3
-                        float *o = out_plane + (half ? 2 * plane : 0) + static_cast<size_t>(gr) * g.W + gc;
-                        if constexpr (ALIGNED) {
-                            store.vec4(o, a);
-                            store.vec4(o + plane, d);
-                        } else {
-                            store(o, a, n);
-                            store(o + plane, d, n);
-                        }
-                    }
-                }
-                swt_rw_fence();
-            }
-        }
-    }
-}
-
 // ---------------------------------------------------------------------------------------------- tile programs
 // The per-CTA program is written once, as a sequence of phases handed to `exec`: on the device a phase runs as
 // phase(threadIdx.x, blockDim.x) followed by __syncthreads(); the CPU simulator runs it for tid = 0..nthreads-1.
@@ -635,11 +579,12 @@ __host__ __device__ __forceinline__ void swt_level_cols(const SwtGeom &g, int lv
     ncg = (ce + 3) / 4 - c0g;
 }
 
-// RW (g.rw, chosen by the planner): 0 two-pass levels, 1 register-window passes, 2 register-window intermediate levels +
-// two-pass last level — a template parameter so that each kernel is compiled and register-allocated for one form only.
-template <int F, int LEVEL, int RW, int VS, typename Exec, typename Store, typename Ld>
+// One program per (F, LEVEL): the pass form follows from them (swt_rw_form, swt_vs_form), so that each kernel is
+// compiled and register-allocated for one form only.
+template <int F, int LEVEL, typename Exec, typename Store, typename Ld>
 __host__ __device__ __forceinline__ void swt_tile_program(const SwtGeom &g, const void *in, float *out, SwtTileId id,
                                                           float *smem, Exec exec, Store store, Ld ld) {
+    constexpr int RW = swt_rw_form(F, LEVEL), VS = swt_vs_form(F, LEVEL);
     const size_t plane_px = static_cast<size_t>(g.H) * g.W;
     const void *in_plane = g.in_is_u8 ? static_cast<const void *>(static_cast<const uint8_t *>(in) + id.plane * plane_px)
                                       : static_cast<const void *>(static_cast<const float *>(in) + id.plane * plane_px);
@@ -661,72 +606,41 @@ __host__ __device__ __forceinline__ void swt_tile_program(const SwtGeom &g, cons
     constexpr int hb = F / 2 - 1, ha = F / 2;          // halo of a dilation-1 step
     int vb = 0, ve = g.RH;                             // valid rows of the current approximation
     int c0g, ncg;
-    if constexpr (RW != 0) {
-        // register-window form: one pass per level, the approximations ping-pong between the two buffers
-        float *cur = stage, *other = stage == a ? b : a;
-        if constexpr (LEVEL >= 2) {
-            swt_level_cols(g, 1, c0g, ncg);
+    // The intermediate levels leave the approximation in `cur` and the free buffer in `other`: a register-window level
+    // is one pass that swaps them, a two-pass level filters cur -> other (horizontal) -> cur (vertical).
+    float *cur = stage, *other = stage == a ? b : a;
+    if constexpr (LEVEL >= 2) {
+        swt_level_cols(g, 1, c0g, ncg);
+        if constexpr (RW != 0) {
             vb += hb, ve -= ha;
             exec([&](int tid, int n) { swt_rw_ll<F, 1>(g, cur, other, g.RWp, vb, ve, c0g, ncg, g.m_lvl[0], tid, n); });
             float *t = cur;
             cur = other, other = t;
+        } else {
+            exec([&](int tid, int n) { swt_hpass<F, 1, false>(g, cur, g.RWp, other, nullptr, g.RWp, vb, ve, c0g, ncg, g.m_lvl[0], 0, 0, tid, n); });
+            vb += hb, ve -= ha;
+            exec([&](int tid, int n) { swt_vpass_ll<F, 1>(g, other, cur, g.RWp, vb, ve, c0g, ncg, g.m_lvl[0], tid, n); });
         }
-        if constexpr (LEVEL >= 3) {
-            swt_level_cols(g, 2, c0g, ncg);
+    }
+    if constexpr (LEVEL >= 3) {
+        swt_level_cols(g, 2, c0g, ncg);
+        if constexpr (RW != 0) {
             vb += 2 * hb, ve -= 2 * ha;
             exec([&](int tid, int n) { swt_rw_ll<F, 2>(g, cur, other, g.RWp, vb, ve, c0g, ncg, g.m_lvl[1], tid, n); });
             float *t = cur;
             cur = other, other = t;
-        }
-        constexpr int SL = 1 << (LEVEL - 1);
-        if constexpr (RW == 1) {
-            const int twp4 = (g.TW + 3) / 4;
-            exec([&](int tid, int n) {
-                if ((g.W & 3) == 0)
-                    swt_rw_final<F, SL, true>(g, cur, g.RWp, g.top, g.padL, out_plane, id.ty * g.TH, id.tx * g.TW, twp4, g.m_lvl[LEVEL - 1], tid, n, store);
-                else
-                    swt_rw_final<F, SL, false>(g, cur, g.RWp, g.top, g.padL, out_plane, id.ty * g.TH, id.tx * g.TW, twp4, g.m_lvl[LEVEL - 1], tid, n, store);
-            });
         } else {
-            const int twp = (g.TW + 3) / 4 * 4;
-            float *hl = other, *hh = other + static_cast<size_t>(g.RHv) * twp;
-            const int r0 = g.top - SL * hb;
-            exec([&](int tid, int n) {
-                swt_hpass<F, SL, true>(g, cur, g.RWp, hl, hh, twp, r0, r0 + g.RHv, g.padL / 4, twp / 4, g.m_lvl[LEVEL - 1], r0, g.padL, tid, n);
-            });
-            exec([&](int tid, int n) {
-                if constexpr (VS != 0) {
-                    if ((g.W & 3) == 0)
-                        swt_vpass_final_slide<F, SL, true>(g, hl, hh, twp, out_plane, id.ty * g.TH, id.tx * g.TW, twp / 4, g.m_lvl[LEVEL - 1], tid, n, store);
-                    else
-                        swt_vpass_final_slide<F, SL, false>(g, hl, hh, twp, out_plane, id.ty * g.TH, id.tx * g.TW, twp / 4, g.m_lvl[LEVEL - 1], tid, n, store);
-                } else {
-                    if ((g.W & 3) == 0)
-                        swt_vpass_final<F, SL, true>(g, hl, hh, twp, out_plane, id.ty * g.TH, id.tx * g.TW, twp / 4, g.m_lvl[LEVEL - 1], tid, n, store);
-                    else
-                        swt_vpass_final<F, SL, false>(g, hl, hh, twp, out_plane, id.ty * g.TH, id.tx * g.TW, twp / 4, g.m_lvl[LEVEL - 1], tid, n, store);
-                }
-            });
+            exec([&](int tid, int n) { swt_hpass<F, 2, false>(g, cur, g.RWp, other, nullptr, g.RWp, vb, ve, c0g, ncg, g.m_lvl[1], 0, 0, tid, n); });
+            vb += 2 * hb, ve -= 2 * ha;
+            exec([&](int tid, int n) { swt_vpass_ll<F, 2>(g, other, cur, g.RWp, vb, ve, c0g, ncg, g.m_lvl[1], tid, n); });
         }
-    } else {
-    if constexpr (LEVEL >= 2) {
-        swt_level_cols(g, 1, c0g, ncg);
-        exec([&](int tid, int n) { swt_hpass<F, 1, false>(g, a, g.RWp, b, nullptr, g.RWp, vb, ve, c0g, ncg, g.m_lvl[0], 0, 0, tid, n); });
-        vb += hb, ve -= ha;
-        exec([&](int tid, int n) { swt_vpass_ll<F, 1>(g, b, a, g.RWp, vb, ve, c0g, ncg, g.m_lvl[0], tid, n); });
-    }
-    if constexpr (LEVEL >= 3) {
-        swt_level_cols(g, 2, c0g, ncg);
-        exec([&](int tid, int n) { swt_hpass<F, 2, false>(g, a, g.RWp, b, nullptr, g.RWp, vb, ve, c0g, ncg, g.m_lvl[1], 0, 0, tid, n); });
-        vb += 2 * hb, ve -= 2 * ha;
-        exec([&](int tid, int n) { swt_vpass_ll<F, 2>(g, b, a, g.RWp, vb, ve, c0g, ncg, g.m_lvl[1], tid, n); });
     }
     constexpr int S = 1 << (LEVEL - 1);
     const int twp = (g.TW + 3) / 4 * 4;
-    float *hl = b, *hh = b + static_cast<size_t>(g.RHv) * twp;
+    float *hl = other, *hh = other + static_cast<size_t>(g.RHv) * twp;
     const int r0 = g.top - S * hb;
     exec([&](int tid, int n) {
-        swt_hpass<F, S, true>(g, a, g.RWp, hl, hh, twp, r0, r0 + g.RHv, g.padL / 4, twp / 4, g.m_lvl[LEVEL - 1], r0, g.padL, tid, n);
+        swt_hpass<F, S, true>(g, cur, g.RWp, hl, hh, twp, r0, r0 + g.RHv, g.padL / 4, twp / 4, g.m_lvl[LEVEL - 1], r0, g.padL, tid, n);
     });
     exec([&](int tid, int n) {
         if constexpr (VS != 0) {
@@ -741,7 +655,6 @@ __host__ __device__ __forceinline__ void swt_tile_program(const SwtGeom &g, cons
                 swt_vpass_final<F, S, false>(g, hl, hh, twp, out_plane, id.ty * g.TH, id.tx * g.TW, twp / 4, g.m_lvl[LEVEL - 1], tid, n, store);
         }
     });
-    }
 }
 
 // Generic fallback (any even F <= 20, level <= 4): runtime taps, one pixel per work item, three buffers.

@@ -3,8 +3,6 @@
 #include <algorithm>
 #include <cmath>
 #include <cstddef>
-#include <cstdio>
-#include <cstdlib>
 
 #include "swt2_core.cuh"
 
@@ -29,7 +27,7 @@ inline void swt_fill_geometry(SwtGeom &g, int th, int tw, bool fast) {
     if (fast) {
         g.nbuf = 2;
         g.off_b = static_cast<int>(kSwtGuard + buf + kSwtGuard);
-        const size_t b_floats = g.rw == 1 ? (g.level > 1 ? buf : 0) : std::max<size_t>(g.level > 1 ? buf : 0, static_cast<size_t>(2) * g.RHv * tw);
+        const size_t b_floats = std::max<size_t>(g.level > 1 ? buf : 0, static_cast<size_t>(2) * g.RHv * tw);
         g.smem_floats = static_cast<int>(g.off_b + b_floats + kSwtGuard);
     } else {
         g.nbuf = 3;
@@ -67,24 +65,19 @@ inline int swt_plan(SwtGeom &g, int B, int C, int H, int W, int F, int level, in
     g.padL = (g.left + 3) / 4 * 4;
     g.threads = 256;
     const int S = 1 << (level - 1);
-    // register-window passes (swt2_core.cuh: swt_rw_*): B200_SWT_RW=0/1 overrides the default
-    // Measured on B200 (round 2, 256x3x520x520 uint8, fraction of the HBM roofline, two-pass -> hybrid): haar level 2
-    // 0.75 -> 0.79, db2 level 2 0.56 -> 0.61, haar level 3 0.53 -> 0.64, db2 level 3 0.40 -> 0.43; the 8-tap filters lose 3-9 %
-    // (the 15 / 8 horizontal FMAs of an 8-row window outweigh the saved shared-memory round trip) and the all-register
-    // form (1) loses everywhere: 128 registers leave 16 warps per SM (db4 level 1: 0.58 -> 0.42).
-    g.rw = (fast && level >= 2 && F <= 4) ? 2 : 0;
-    if (const char *ov = std::getenv("B200_SWT_RW")) g.rw = fast ? std::atoi(ov) : 0;
-    if (g.rw < 0 || g.rw > 2 || (g.rw == 2 && level == 1)) g.rw = 0;
-    // sliding last vertical pass (swt_vpass_final_slide): B200_SWT_VS=0/1 overrides the default.
-    // Measured on B200 (round 2, C4 grid, blocked -> sliding): db4 / sym4 level 1 0.581 -> 0.605 of the HBM roofline (the
-    // 8-tap kernel drops from 80 to 64 registers: 7 % fewer instructions, 36 % fewer shared-memory wavefronts); the short
-    // filters lose (haar level 1 0.81 -> 0.62: their blocked pass has 4 output rows per unit already and twice the
-    // stores per unit), bior4.4 loses (0.52 -> 0.47) and so do levels 2 / 3 with every tile tried (db4 level 2 0.395 ->
-    // 0.33-0.37: TH must be a multiple of 8 * 2^(level-1)).
-    g.vs = (fast && level == 1 && F == 8) ? 1 : 0;
-    if (const char *ov = std::getenv("B200_SWT_VS")) g.vs = (fast && g.rw != 1 && std::atoi(ov) != 0) ? 1 : 0;
-    const int th_unit = fast ? ((g.rw == 1 || g.vs) ? kRwR : kSwtR) * S : 1;
-    static_assert(kRwR == kVsR, "one tile-height unit for both register-window forms");
+    // Pass forms (swt2_core.cuh: swt_rw_form, swt_vs_form), measured on B200 (round 2):
+    // - hybrid (register-window intermediate levels, swt_rw_ll; 256x3x520x520 uint8, fraction of the HBM roofline,
+    //   two-pass -> hybrid): haar level 2 0.75 -> 0.79, db2 level 2 0.56 -> 0.61, haar level 3 0.53 -> 0.64, db2 level 3
+    //   0.40 -> 0.43; the 8-tap filters lose 3-9 % (the 15 / 8 horizontal FMAs of an 8-row window outweigh the saved
+    //   shared-memory round trip).  An all-register form (register-window last level too) lost everywhere: 128
+    //   registers leave 16 warps per SM (db4 level 1: 0.58 -> 0.42).
+    // - sliding last vertical pass (swt_vpass_final_slide; C4 grid, blocked -> sliding): db4 / sym4 level 1 0.581 ->
+    //   0.605 of the HBM roofline (the 8-tap kernel drops from 80 to 64 registers: 7 % fewer instructions, 36 % fewer
+    //   shared-memory wavefronts); the short filters lose (haar level 1 0.81 -> 0.62: their blocked pass has 4 output
+    //   rows per unit already and twice the stores per unit), bior4.4 loses (0.52 -> 0.47) and so do levels 2 / 3 with
+    //   every tile tried (db4 level 2 0.395 -> 0.33-0.37: TH must be a multiple of 8 * 2^(level-1)).
+    const bool vs = fast && swt_vs_form(F, level);
+    const int th_unit = fast ? (vs ? kVsR : kSwtR) * S : 1;
     const long long planes = static_cast<long long>(B) * C;
     double best = 1e30;
     int bth = 0, btw = 0;
@@ -126,24 +119,11 @@ inline int swt_plan(SwtGeom &g, int B, int C, int H, int W, int F, int level, in
             if (cost < best) best = cost, bth = th, btw = tw;
         }
     }
-    // Measured on B200 (tools/swt_sweep.sh, profiles/): small CTAs whose staging / horizontal / vertical phases interleave
+    // Measured on B200 (tile-shape sweeps, profiles/): small CTAs whose staging / horizontal / vertical phases interleave
     // across many resident CTAs beat what the instruction-count model above predicts.  Level 1: 128 threads, 16-row
     // (F <= 4) or 48-row tiles about 112 / 76 columns wide; deeper levels: 256 threads, 48 x ~76 tiles.  The model's
     // choice stays as the fallback when the preferred tile does not fit.
-    if (fast && g.rw == 1) {
-        // one unit (4 columns x 8 rows of a residue class) per thread in the last pass: threads = (TW / 4) * (TH / 8)
-        const int want_th = level == 1 ? 32 : (level == 2 ? 32 : 64), want_tw = 128;
-        const int nx = (W + want_tw - 1) / want_tw;
-        const int tw = ((W + nx - 1) / nx + 3) / 4 * 4;
-        const int th = (std::min(want_th, H) + th_unit - 1) / th_unit * th_unit;
-        SwtGeom t = g;
-        swt_fill_geometry(t, th, tw, fast);
-        if (swt_smem_bytes(t) <= 110 * 1024) {
-            bth = th, btw = tw;
-            const int units = (tw / 4) * (th / kRwR);
-            g.threads = std::min(256, std::max(64, (units + 31) / 32 * 32));
-        }
-    } else if (fast) {
+    if (fast) {
         const int want_th = (level == 1 && F <= 4) ? 16 : ((level == 1 && F == 8) ? 32 : 48);      // db4 level 1: 32x76 0.53, 48x76 0.48
         const int want_tw = (level == 1 && F <= 4) ? 112 : 76;
         const int nx = (W + want_tw - 1) / want_tw;
@@ -156,14 +136,6 @@ inline int swt_plan(SwtGeom &g, int B, int C, int H, int W, int F, int level, in
             g.threads = level == 1 ? 128 : 256;
         }
     }
-    if (const char *ov = std::getenv("B200_SWT_TILE")) {      // tuning override: "TH,TW"
-        int th = 0, tw = 0;
-        if (std::sscanf(ov, "%d,%d", &th, &tw) == 2 && th > 0 && tw > 0 && tw % 4 == 0 && th % th_unit == 0 && th <= 128) {
-            SwtGeom t = g;
-            swt_fill_geometry(t, th, tw, fast);
-            if (swt_smem_bytes(t) <= 220 * 1024) bth = th, btw = tw;
-        }
-    }
     if (bth == 0) return -2;
     swt_fill_geometry(g, bth, btw, fast);
     // uint8 staging units (swt2_core.cuh): 8 pixels per unit, except where rows are 4-byte aligned AND the kernel is a
@@ -171,11 +143,7 @@ inline int swt_plan(SwtGeom &g, int B, int C, int H, int W, int F, int level, in
     // (measured on B200, same box: 224x224 haar 32.7 vs 33.7 us, 520x520 db2 668 vs 680 us; 518-wide rows and long
     // filters gain 5-11 % from the 8-pixel units: db4 983 -> 932 us, bior4.4 1133 -> 1024 us, haar 635 -> 606 us)
     g.u8_stage = in_is_u8 ? ((W % 4 == 0 && level == 1 && F <= 4) ? 0 : 1) : 0;
-    if (const char *ov = std::getenv("B200_SWT_U8STAGE")) {      // A/B override: 0 / 1
-        const int m = std::atoi(ov);
-        if (in_is_u8 && (m == 0 || m == 1)) g.u8_stage = m;
-    }
-    if (fast && g.vs) {
+    if (vs) {
         // the sliding pass has 4 * (TW / 4) * TH / kVsR units: the CTA size that leaves the fewest idle lanes in its sweeps
         const int units = 4 * ((g.TW + 3) / 4) * (g.TH / kVsR);
         double best_eff = 0;
@@ -186,10 +154,6 @@ inline int swt_plan(SwtGeom &g, int B, int C, int H, int W, int F, int level, in
             if (eff > best_eff) best_eff = eff, best_t = t;
         }
         g.threads = best_t;
-    }
-    if (const char *ov = std::getenv("B200_SWT_THREADS")) {
-        const int t = std::atoi(ov);
-        if (t >= 32 && t <= 1024 && t % 32 == 0) g.threads = t;
     }
     return 0;
 }

@@ -96,6 +96,6 @@ def sim_swt(sim, x, lo, hi, level, sms=148):
     x = np.ascontiguousarray(x)
     b, c, h, w = x.shape
     out = np.full((b, c, 4, h, w), np.nan, np.float32)
-    plan = (ctypes.c_int * 7)()
+    plan = (ctypes.c_int * 8)()            # TH, TW, rw form, threads, vs form, RH, RWp, u8_stage
     rc = sim.sim_swt2_fwd(vp(x), int(x.dtype == np.uint8), vp(out), b, c, h, w, vp(lo), vp(hi), len(lo), level, sms, plan)
     return rc, out, list(plan)

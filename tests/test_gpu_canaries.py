@@ -134,23 +134,32 @@ def test_knn_topk_stays_inside_its_buffers(monkeypatch, fused, k, n, top_tie):
         assert torch.equal(idx.view(torch.int64).reshape(nq, k).cpu(), torch.arange(0, 7 * k, 7).expand(nq, k))
 
 
-@pytest.mark.parametrize("rw", ["0", "1", "2"])
-@pytest.mark.parametrize("shape,level,u8", [((2, 3, 70, 518), 1, True), ((1, 2, 136, 200), 2, True), ((1, 1, 256, 256), 3, False), ((1, 1, 8, 8), 3, True)])
-def test_swt_stays_inside_its_output(monkeypatch, rw, shape, level, u8):
+# per level, a short, an 8-tap and a long filter: level 1 two-pass (uint8 in 4- or 8-pixel staging units by W), sliding
+# last pass, two-pass F = 10; levels 2-3 hybrid, two-pass F = 8, two-pass F = 10; level 4 the generic program
+CANARY_FILTERS = {1: ("haar", "db4", "bior4.4"), 2: ("db2", "sym4", "bior4.4"), 3: ("db2", "sym4", "bior4.4"), 4: ("haar", "db2", "db4")}
+
+
+@pytest.mark.parametrize("filt", [0, 1, 2])
+@pytest.mark.parametrize("shape,level,u8", [((2, 3, 70, 518), 1, True), ((1, 2, 136, 200), 2, True), ((1, 1, 256, 256), 3, False),
+                                            ((1, 1, 8, 8), 3, True), ((2, 3, 64, 224), 1, True), ((1, 1, 24, 36), 1, False),
+                                            ((1, 1, 64, 64), 4, False)])
+def test_swt_stays_inside_its_output(filt, shape, level, u8):
+    """Guard bytes around the input and the output of b200_swt2_fwd, for every planned pass form and both uint8 staging
+    forms (filt: index into CANARY_FILTERS[level])."""
     from image_retrieval_wavelet_b200 import _cabi
     from oracle import c_oracle, filters
 
-    monkeypatch.setenv("B200_SWT_RW", rw)
     rng = np.random.default_rng(sum(shape))
     x = rng.integers(0, 256, shape).astype(np.uint8) if u8 else rng.random(shape, dtype=np.float32)
-    lo, hi = filters.filter_bank("db2")
+    lo, hi = filters.filter_bank(CANARY_FILTERS[level][filt])
     b, c, h, w = shape
     xin = Guarded(x.nbytes)
     xin.view(torch.uint8).copy_(torch.from_numpy(x.view(np.uint8).reshape(-1)))
     out = Guarded(b * c * 4 * h * w * 4)
-    flo, fhi = (ctypes.c_float * 4)(*lo), (ctypes.c_float * 4)(*hi)
+    flo, fhi = (ctypes.c_float * len(lo))(*lo), (ctypes.c_float * len(hi))(*hi)
     # the input sits 4096 bytes into an allocation: 16-byte aligned, as the entry point asks
-    _cabi.check(_cabi.load().b200_swt2_fwd(xin.ptr, int(u8), out.ptr, b, c, h, w, flo, fhi, 4, level, _cabi.stream_ptr()), "b200_swt2_fwd")
+    _cabi.check(_cabi.load().b200_swt2_fwd(xin.ptr, int(u8), out.ptr, b, c, h, w, flo, fhi, len(lo), level, _cabi.stream_ptr()),
+                "b200_swt2_fwd")
     torch.cuda.synchronize()
     assert out.intact() and xin.intact()
     ref = c_oracle.swt2(x, lo, hi, level)

@@ -46,6 +46,9 @@ CASES = [
     ((1, 3, 30, 34), "db3", 1, np.float32),
     ((2, 3, 256, 256), "db2", 2, np.float32),       # float32, 16-byte aligned rows: interior tiles staged by cp.async.bulk
     ((2, 2, 520, 520), "haar", 1, np.float32),
+    ((1, 1, 24, 36), "sym4", 1, np.float32),        # sliding last pass: float32, smaller than one tile
+    ((1, 1, 256, 256), "db2", 3, np.float32),       # hybrid, bulk-staged float32
+    ((1, 1, 8, 8), "db2", 3, np.uint8),             # hybrid: smaller than one tile
 ]
 
 
@@ -63,54 +66,61 @@ def test_swt2_matches_oracle(shape, name, level, dtype):
     _check(out, ref, f"{shape} {name} L{level}")
 
 
-@pytest.mark.parametrize("rw", ["0", "1", "2"])
+def _swt_rolled(x, name, level, dy, dx):
+    """x rolled by (dy, dx) through its planned pass form: parity with the rolled oracle and, for a non-zero roll, the
+    rolled sub-bands of x bit for bit (the periodic SWT commutes with circular shifts, and every pixel is computed in the
+    same order wherever tiles, staging units and register windows cut the image)."""
+    from image_retrieval_wavelet_b200.transforms import swt2
+
+    lo, hi = filters.filter_bank(name)
+    xt = torch.from_numpy(x).cuda()
+    out = swt2(torch.roll(xt, (dy, dx), dims=(2, 3)), name, level)
+    _check(out, np.roll(c_oracle.swt2(x, lo, hi, level), (dy, dx), axis=(3, 4)), f"{x.shape} {name} L{level} rolled by {(dy, dx)}")
+    if dy or dx:
+        assert torch.equal(out, torch.roll(swt2(xt, name, level), (dy, dx), dims=(3, 4)))
+    return out
+
+
+@pytest.mark.parametrize("shift", [0, 1, 2])
 @pytest.mark.parametrize("shape,name,level,dtype", [((2, 3, 70, 518), "haar", 1, np.uint8), ((1, 2, 130, 518), "db4", 1, np.uint8),
                                                      ((2, 1, 136, 200), "db2", 2, np.uint8), ((1, 2, 256, 256), "db2", 2, np.float32),
                                                      ((1, 1, 520, 520), "sym4", 3, np.uint8), ((1, 3, 104, 96), "haar", 3, np.float32),
                                                      ((1, 1, 48, 40), "bior4.4", 2, np.uint8), ((1, 1, 8, 8), "db4", 3, np.float32)])
-def test_swt_pass_forms_agree_on_device(monkeypatch, rw, shape, name, level, dtype):
-    """B200_SWT_RW = 0 / 1 / 2 (two-pass levels, register-window passes, hybrid): every form against the oracle."""
-    from image_retrieval_wavelet_b200.transforms import swt2
-
-    monkeypatch.setenv("B200_SWT_RW", rw)
+def test_swt_pass_forms_agree_on_device(shift, shape, name, level, dtype):
+    """Every pass form the planner picks (two-pass, sliding last pass, hybrid) on the image rolled by (shift, shift)."""
     rng = np.random.default_rng(sum(shape) + level)
     x = rng.integers(0, 256, shape).astype(np.uint8) if dtype == np.uint8 else rng.random(shape, dtype=np.float32)
-    lo, hi = filters.filter_bank(name)
-    _check(swt2(torch.from_numpy(x).cuda(), name, level), c_oracle.swt2(x, lo, hi, level), f"rw={rw} {shape} {name} L{level}")
+    _swt_rolled(x, name, level, shift, shift)
 
 
-@pytest.mark.parametrize("vs", ["0", "1"])
+@pytest.mark.parametrize("dx", [0, 1])
 @pytest.mark.parametrize("shape,name,level,dtype", [((2, 3, 70, 518), "haar", 1, np.uint8), ((1, 2, 130, 518), "db4", 1, np.uint8),
                                                      ((2, 3, 518, 518), "sym4", 1, np.uint8), ((2, 1, 136, 200), "db2", 2, np.uint8),
                                                      ((1, 1, 520, 520), "sym4", 3, np.uint8), ((1, 1, 48, 40), "bior4.4", 2, np.uint8),
                                                      ((1, 1, 8, 8), "db4", 3, np.float32), ((1, 2, 224, 224), "db4", 1, np.float32)])
-def test_swt_sliding_last_pass_agrees_on_device(monkeypatch, vs, shape, name, level, dtype):
-    """B200_SWT_VS = 0 / 1 (blocked / sliding last vertical pass): both against the oracle."""
-    from image_retrieval_wavelet_b200.transforms import swt2
-
-    monkeypatch.setenv("B200_SWT_VS", vs)
+def test_swt_sliding_last_pass_agrees_on_device(dx, shape, name, level, dtype):
+    """The last vertical pass (sliding for 8-tap filters at level 1, blocked otherwise) on the image rolled by (0, dx)."""
     rng = np.random.default_rng(sum(shape) + level)
     x = rng.integers(0, 256, shape).astype(np.uint8) if dtype == np.uint8 else rng.random(shape, dtype=np.float32)
-    lo, hi = filters.filter_bank(name)
-    _check(swt2(torch.from_numpy(x).cuda(), name, level), c_oracle.swt2(x, lo, hi, level), f"vs={vs} {shape} {name} L{level}")
+    _swt_rolled(x, name, level, 0, dx)
 
 
-@pytest.mark.parametrize("stage", ["0", "1"])
+@pytest.mark.parametrize("dx", [0, 1])
 @pytest.mark.parametrize("shape,name,level", [((3, 2, 70, 518), "haar", 1), ((2, 3, 130, 518), "db4", 1), ((2, 1, 66, 94), "bior4.4", 1),
-                                              ((2, 1, 40, 36), "db2", 2), ((1, 1, 24, 10), "haar", 1), ((2, 3, 224, 224), "db2", 1)])
-def test_uint8_staging_units_agree(monkeypatch, stage, shape, name, level):
-    """Both uint8 staging forms (B200_SWT_U8STAGE: 4-pixel units / 8-pixel units of three aligned words) on rows that
-    start on every byte alignment, with wrap in x and y: identical bits (the conversion is exact in both) and parity."""
+                                              ((2, 1, 40, 36), "db2", 2), ((1, 1, 24, 10), "haar", 1), ((2, 3, 224, 224), "db2", 1),
+                                              ((2, 3, 130, 518), "db2", 1), ((2, 1, 40, 10), "db2", 1), ((2, 3, 224, 222), "haar", 1)])
+def test_uint8_staging_units_agree(dx, shape, name, level):
+    """uint8 staging on rows that start on every byte alignment (the image rolled by dx), with wrap in x and y.  Where
+    both staging forms apply (level 1, F <= 4) they give identical bits: x (W % 4 = 2) is staged in 8-pixel units of three
+    aligned words, [x, x] side by side (W % 4 = 0) in 4-pixel units, and the periodic transform of [x, x] is
+    [swt(x), swt(x)]."""
     from image_retrieval_wavelet_b200.transforms import swt2
 
-    monkeypatch.setenv("B200_SWT_U8STAGE", stage)
     x = np.random.default_rng(len(name) + shape[3]).integers(0, 256, shape).astype(np.uint8)
-    lo, hi = filters.filter_bank(name)
-    out = swt2(torch.from_numpy(x).cuda(), name, level)
-    _check(out, c_oracle.swt2(x, lo, hi, level), f"stage {stage} {shape} {name} L{level}")
-    monkeypatch.setenv("B200_SWT_U8STAGE", "1" if stage == "0" else "0")
-    other = swt2(torch.from_numpy(x).cuda(), name, level)
-    assert torch.equal(out, other)
+    out = _swt_rolled(x, name, level, 0, dx)
+    if level == 1 and len(filters.filter_bank(name)[0]) <= 4 and shape[3] % 4 == 2:
+        xr = torch.roll(torch.from_numpy(x).cuda(), dx, dims=3)
+        assert torch.equal(swt2(torch.cat([xr, xr], dim=-1), name, 1), torch.cat([out, out], dim=-1))
 
 
 def test_full_size_c4_properties():

@@ -21,6 +21,10 @@ SWT_CASES = [
     ((1, 1, 64, 64), "haar", 4, np.float32),      # level 4: generic program
     ((3, 1, 136, 200), "coif1", 3, np.uint8),
     ((1, 1, 2, 2), "haar", 1, np.uint8),          # minimum size
+    ((1, 1, 24, 36), "sym4", 1, np.float32),      # sliding last pass: float32, smaller than one tile
+    ((1, 1, 66, 94), "bior4.4", 1, np.uint8),     # F = 10 level 1: W % 4 = 2
+    ((2, 1, 40, 36), "db2", 2, np.uint8),         # hybrid, uint8
+    ((1, 1, 8, 8), "db2", 3, np.uint8),           # hybrid: smaller than one tile
 ]
 
 
@@ -38,64 +42,94 @@ def test_swt_tile_program(sim, shape, name, level, dtype):
         assert np.abs(out[:, :, band] - ref[:, :, band]).max() <= tol, (band, plan)
 
 
-@pytest.mark.parametrize("rw", ["0", "1", "2"])
+# (F, level, W, uint8) -> (rw form, vs form, u8_stage); rw -1: the generic program
+FORM_CASES = [
+    ((2, 1, 224, 1), (0, 0, 0)), ((4, 1, 224, 1), (0, 0, 0)), ((6, 1, 224, 1), (0, 0, 1)), ((10, 1, 224, 0), (0, 0, 0)),   # two-pass
+    ((2, 1, 518, 1), (0, 0, 1)), ((4, 1, 518, 0), (0, 0, 0)), ((10, 1, 518, 1), (0, 0, 1)),
+    ((8, 1, 518, 1), (0, 1, 1)), ((8, 1, 224, 1), (0, 1, 1)), ((8, 1, 224, 0), (0, 1, 0)),                                 # sliding
+    ((2, 2, 520, 1), (2, 0, 1)), ((4, 2, 520, 0), (2, 0, 0)), ((2, 3, 520, 1), (2, 0, 1)), ((4, 3, 256, 1), (2, 0, 1)),    # hybrid
+    ((6, 2, 520, 1), (0, 0, 1)), ((8, 2, 520, 1), (0, 0, 1)), ((10, 2, 520, 0), (0, 0, 0)),                                # two-pass
+    ((6, 3, 520, 0), (0, 0, 0)), ((8, 3, 520, 1), (0, 0, 1)), ((10, 3, 520, 1), (0, 0, 1)),
+    ((12, 1, 224, 1), (-1, 0, 1)), ((20, 2, 224, 0), (-1, 0, 0)), ((2, 4, 224, 1), (-1, 0, 1)), ((4, 4, 224, 0), (-1, 0, 0)),  # generic
+]
+
+
+@pytest.mark.parametrize("case,forms", FORM_CASES)
+def test_swt_plan_picks_the_form_of_filter_and_level(sim, case, forms):
+    """The pass form is a function of (F, level) alone: hybrid for levels 2-3 under F <= 4, the sliding last pass for
+    F = 8 at level 1, two-pass otherwise on the fast path; uint8 staging in 4-pixel units only for 4-byte aligned rows
+    under a short level-1 filter."""
+    import ctypes
+
+    F, level, W, u8 = case
+    plan = (ctypes.c_longlong * 10)()
+    assert sim.sim_swt2_plan(4, 3, 224, W, F, level, u8, 148, plan) == 0
+    assert (plan[2], plan[4], plan[9]) == forms, list(plan)
+    if forms[0] >= 0:                                      # fast path: TH is a whole number of vertical units
+        assert plan[0] % ((8 if forms[1] else 4) << (level - 1)) == 0, list(plan)
+
+
+def _swt_rolled(sim, x, name, level, dy, dx):
+    """x rolled by (dy, dx) through its planned pass form: parity with the rolled oracle and, for a non-zero roll, the
+    rolled sub-bands of x bit for bit (the periodic SWT commutes with circular shifts, and every pixel is computed in the
+    same order wherever tiles, staging units and register windows cut the image)."""
+    lo, hi = filters.filter_bank(name)
+    rc, out, plan = sim_swt(sim, np.roll(x, (dy, dx), axis=(2, 3)), lo, hi, level)
+    assert rc == 0
+    assert not np.isnan(out).any(), "some output pixel was never written"
+    ref = np.roll(c_oracle.swt2(x, lo, hi, level), (dy, dx), axis=(3, 4))
+    for band in range(4):
+        assert np.abs(out[:, :, band] - ref[:, :, band]).max() <= 1e-5 * max(np.abs(ref[:, :, band]).max(), 1e-30), (band, plan)
+    if dy or dx:
+        rc0, out0, _ = sim_swt(sim, x, lo, hi, level)
+        assert rc0 == 0 and np.array_equal(np.roll(out0, (dy, dx), axis=(3, 4)).view(np.uint32), out.view(np.uint32)), plan
+    return out, plan
+
+
+@pytest.mark.parametrize("shift", [0, 1, 2])
 @pytest.mark.parametrize("shape,name,level,dtype", [((1, 2, 70, 518), "haar", 1, np.uint8), ((1, 1, 66, 94), "db4", 1, np.uint8),
                                                      ((2, 1, 40, 36), "db2", 2, np.float32), ((1, 1, 72, 88), "sym4", 3, np.uint8),
                                                      ((1, 1, 64, 80), "haar", 3, np.float32), ((1, 2, 48, 36), "bior4.4", 2, np.uint8),
                                                      ((1, 1, 8, 8), "db4", 3, np.float32), ((1, 1, 130, 518), "db2", 1, np.uint8)])
-def test_swt_pass_forms_agree(sim, monkeypatch, rw, shape, name, level, dtype):
-    """B200_SWT_RW: 0 two-pass levels (horizontal outputs through shared memory), 1 register-window passes (a window of F
-    filtered rows per unit, no intermediate planes), 2 register-window intermediate levels + two-pass last level (the
-    default for levels 2-3 under short filters) — same sub-bands, including x / y wrap, W % 4 = 2 and tiny images."""
-    monkeypatch.setenv("B200_SWT_RW", rw)
+def test_swt_pass_forms_agree(sim, shift, shape, name, level, dtype):
+    """Every pass form the planner picks (two-pass, sliding last pass, hybrid: test_swt_plan_picks_the_form_of_filter_and_level)
+    on the image rolled by (shift, shift): same sub-bands as the oracle, including x / y wrap, W % 4 = 2 and tiny images."""
     rng = np.random.default_rng(sum(shape) + level)
     x = rng.integers(0, 256, shape).astype(np.uint8) if dtype == np.uint8 else rng.random(shape, dtype=np.float32)
-    lo, hi = filters.filter_bank(name)
-    rc, out, plan = sim_swt(sim, x, lo, hi, level)
-    assert rc == 0
-    ref = c_oracle.swt2(x, lo, hi, level)
-    assert not np.isnan(out).any(), "some output pixel was never written"
-    for band in range(4):
-        assert np.abs(out[:, :, band] - ref[:, :, band]).max() <= 1e-5 * max(np.abs(ref[:, :, band]).max(), 1e-30), (band, plan)
+    _swt_rolled(sim, x, name, level, shift, shift)
 
 
-@pytest.mark.parametrize("vs", ["0", "1"])
-@pytest.mark.parametrize("rw", ["0", "2"])
+@pytest.mark.parametrize("dx", [0, 1])
+@pytest.mark.parametrize("dy", [0, 2])
 @pytest.mark.parametrize("shape,name,level,dtype", [((1, 2, 70, 518), "haar", 1, np.uint8), ((1, 1, 66, 94), "db4", 1, np.uint8),
                                                      ((2, 1, 40, 36), "db2", 2, np.float32), ((1, 1, 72, 88), "sym4", 3, np.uint8),
                                                      ((1, 2, 48, 36), "bior4.4", 2, np.uint8), ((1, 1, 8, 8), "db4", 3, np.float32),
                                                      ((1, 1, 130, 518), "sym4", 1, np.uint8)])
-def test_swt_sliding_last_pass_agrees(sim, monkeypatch, vs, rw, shape, name, level, dtype):
-    """B200_SWT_VS: 0 blocked last vertical pass (R + F - 1 rows per R outputs, both bands of a half per unit), 1 sliding
-    pass (register window of F rows, one band per unit; the default for 8-tap filters at level 1) — same sub-bands for
-    tiles that overhang the image bottom, W % 4 = 2 rows and images smaller than one tile."""
-    monkeypatch.setenv("B200_SWT_VS", vs)
-    monkeypatch.setenv("B200_SWT_RW", rw)
+def test_swt_sliding_last_pass_agrees(sim, dx, dy, shape, name, level, dtype):
+    """The last vertical pass: sliding (register window of F rows, one band per unit) for 8-tap filters at level 1,
+    blocked (R + F - 1 rows per R outputs, both bands of a half per unit) otherwise — same sub-bands on the image rolled by
+    (dy, dx), for tiles that overhang the image bottom, W % 4 = 2 rows and images smaller than one tile."""
     rng = np.random.default_rng(sum(shape) + level)
     x = rng.integers(0, 256, shape).astype(np.uint8) if dtype == np.uint8 else rng.random(shape, dtype=np.float32)
-    lo, hi = filters.filter_bank(name)
-    rc, out, plan = sim_swt(sim, x, lo, hi, level)
-    assert rc == 0
-    ref = c_oracle.swt2(x, lo, hi, level)
-    assert not np.isnan(out).any(), "some output pixel was never written"
-    for band in range(4):
-        assert np.abs(out[:, :, band] - ref[:, :, band]).max() <= 1e-5 * max(np.abs(ref[:, :, band]).max(), 1e-30), (band, plan)
+    _swt_rolled(sim, x, name, level, dy, dx)
 
 
-@pytest.mark.parametrize("stage", ["0", "1"])
+@pytest.mark.parametrize("dx", [0, 1])
 @pytest.mark.parametrize("shape,name,level", [((1, 2, 70, 518), "haar", 1), ((1, 1, 66, 94), "db4", 1), ((2, 1, 40, 36), "db2", 2),
-                                              ((1, 1, 24, 10), "haar", 1)])
-def test_swt_uint8_staging_units_agree(sim, monkeypatch, stage, shape, name, level):
-    """Both uint8 staging forms (4-pixel units shared with float32, 8-pixel units: three aligned words + funnel shift)
-    on rows that start on every byte alignment, with x/y wrap, narrow images and the short last unit of a row."""
-    monkeypatch.setenv("B200_SWT_U8STAGE", stage)
+                                              ((1, 1, 24, 10), "haar", 1), ((1, 2, 70, 518), "db2", 1), ((2, 1, 40, 10), "db2", 1)])
+def test_swt_uint8_staging_units_agree(sim, dx, shape, name, level):
+    """uint8 staging on rows that start on every byte alignment (the image rolled by dx), with x/y wrap, narrow images and
+    the short last unit of a row.  Where both staging forms apply (level 1, F <= 4) they give identical bits: x (W % 4 = 2)
+    is staged in 8-pixel units of three aligned words, [x, x] side by side (W % 4 = 0) in the 4-pixel units shared with
+    float32, and the periodic transform of [x, x] is [swt(x), swt(x)]."""
     x = np.random.default_rng(len(name) + shape[3]).integers(0, 256, shape).astype(np.uint8)
+    out, plan = _swt_rolled(sim, x, name, level, 0, dx)
     lo, hi = filters.filter_bank(name)
-    rc, out, plan = sim_swt(sim, x, lo, hi, level)
-    assert rc == 0
-    ref = c_oracle.swt2(x, lo, hi, level)
-    assert not np.isnan(out).any()
-    assert np.abs(out - ref).max() <= 1e-5 * np.abs(ref).max(), plan
+    if level == 1 and len(lo) <= 4:
+        xr = np.roll(x, dx, axis=3)
+        rc, out2, plan2 = sim_swt(sim, np.concatenate([xr, xr], axis=-1), lo, hi, 1)
+        assert rc == 0 and plan[7] == 1 and plan2[7] == 0, (plan, plan2)
+        assert np.array_equal(out2.view(np.uint32), np.concatenate([out, out], axis=-1).view(np.uint32))
 
 
 @pytest.mark.parametrize("sms", [1, 16, 148, 1000])

@@ -1,7 +1,7 @@
 #!/bin/bash
 # AddressSanitizer + UBSan over the kernels' tile programs: csrc/hostsim.cpp runs the SAME __host__ __device__ code as the
-# CUDA build (swt2_core.cuh: all three pass forms; hamming_core.cuh: stage A / S / B, stash and walk forms, shard scans),
-# thread by thread, with the shared-memory buffers as exactly-sized heap blocks — so an out-of-range shared / global
+# CUDA build (swt2_core.cuh: every planned pass form and both uint8 staging forms; hamming_core.cuh: stage A / S / B,
+# stash and walk forms, shard scans), thread by thread, with the shared-memory buffers as exactly-sized heap blocks — so an out-of-range shared / global
 # index of those programs is an ASan report here.  compute-sanitizer itself is closed on this project's GPU pool
 # (profiles/r2_sanitizer.md).  Run in the build container:   bash tools/sim_asan.sh
 set -e

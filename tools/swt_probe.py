@@ -1,5 +1,5 @@
-"""SWT C1 / C4 grid (bench.py's cases) with the current planner settings; B200_SWT_RW / B200_SWT_TILE / B200_SWT_THREADS
-are read by the planner.  python tools/swt_probe.py [steps] [filter substring]"""
+"""SWT C1 / C4 grid (bench.py's cases): time and fraction of the HBM roofline per case.  A/B of two builds: run it once
+per library with B200RET_LIB=<path to libb200ret.so>.  python tools/swt_probe.py [steps] [filter substring]"""
 import argparse
 import os
 import sys
