@@ -12,6 +12,22 @@ inline T plan_ceil_div(T a, T b) { return (a + b - 1) / b; }
 template <typename T>
 inline T plan_round_up(T a, T b) { return plan_ceil_div(a, b) * b; }
 
+// largest stash (1 byte + 1 bit per (row, query) pair) a plan carves, in MB
+constexpr size_t kMapStashMaxMB = 24576;
+
+// Tensor-core form of the select pass (hamming_select.cu (A'): tcgen05 filter -> hit masks -> SIMT append; c3 select
+// 0.61 -> 0.53 ms, c5 5.8 -> 3.7 ms) for a select plan: full 128-query groups, e4m3 copies of the codes (rows padded to
+// 128-byte K blocks) and the hit masks (4 B per (32-row group, query)) bounded in the workspace.  Needs only Q, N, B and
+// the query groups, so map_plan_init decides it before the select geometry, which it then fits to the form: 128-query
+// select groups and segments of whole 256-row tiles.  The plan carves the e4m3 + mask block and the launcher runs the form
+// exactly when this holds.
+inline bool plan_select_tc(const b200_map_plan &p) {
+    const size_t bp = static_cast<size_t>((p.B + 127) / 128) * 128;
+    const size_t groups = static_cast<size_t>(plan_ceil_div<long long>(p.N, 256)) * 8;
+    return p.T == 128 && p.Qpad % 128 == 0 && groups * p.Qpad * sizeof(uint32_t) <= (4ull << 30) &&
+           static_cast<size_t>(p.N) * bp <= (8ull << 30);
+}
+
 // waves: how many machine-filling sets of segments to cut the database into (1: one CTA per SM slot; the host-buffer
 // pipeline asks for one wave per H2D chunk so that stage A of a chunk fills the GPU while the next chunk is in flight)
 // allow_select: the caller can run the select pipeline (device library, single shard); the simulator and sub-plans pass false
@@ -57,14 +73,12 @@ inline int map_plan_init(b200_map_plan *plan, int Q, long long N, long long N_to
     const size_t stash_d_bytes = static_cast<size_t>(plan_ceil_div<long long>(N > 0 ? N : 1, 16)) * p.Qpad * 16;
     const size_t stash_r_bytes = static_cast<size_t>(plan_ceil_div<long long>(N > 0 ? N : 1, 32)) * p.Qpad * 4;
     {
-        size_t budget_mb = 24576;
-        if (const char *e = std::getenv("B200_MAP_STASH_MAX_MB")) budget_mb = static_cast<size_t>(std::atoll(e));
         // worth it when most rows are outside the top k (stage B then skips them at 1 byte each).  When k covers the
         // database every row is walked anyway: measured on c3_all, re-scoring in 4-row batches (2.25 ms) beats walking the
         // stash row by row (3.67 ms) and stage A is spared the stores.  B200_MAP_STASH=0/1 forces.
         const char *on = std::getenv("B200_MAP_STASH");
         const bool want = on ? on[0] != '0' : 4 * p.k <= N_total;
-        p.stash = (B <= 254 && N > 0 && want && (stash_d_bytes + stash_r_bytes) / (1024 * 1024) < budget_mb) ? 1 : 0;
+        p.stash = (B <= 254 && N > 0 && want && (stash_d_bytes + stash_r_bytes) / (1024 * 1024) < kMapStashMaxMB) ? 1 : 0;
     }
     const long long seg_unit = p.stash ? 32 : 2;
     long long seg = plan_round_up<long long>(plan_ceil_div<long long>(N > 0 ? N : 1, S), seg_unit);
@@ -84,7 +98,6 @@ inline int map_plan_init(b200_map_plan *plan, int Q, long long N, long long N_to
     p.off_stash_d = carve(p.stash ? stash_d_bytes : 0);
     p.off_stash_r = carve(p.stash ? stash_r_bytes : 0);
     // ---- select mode (see b200ret.h)
-    bool plan_stc = false;
     {
         const char *on = std::getenv("B200_MAP_SELECT");
         const bool forced = on && on[0] != '0';
@@ -105,36 +118,20 @@ inline int map_plan_init(b200_map_plan *plan, int Q, long long N, long long N_to
             // 5-10 % faster, the candidate density differs between query groups and finer CTAs balance it), with segments of
             // >= 1024 rows so that the per-(query, segment) candidate lists stay long (the rank kernel pays per list); when
             // a GPU has few queries (a slice of a multi-GPU run) the groups shrink to 64 / 32 queries instead of the segments
-            // Tensor-core form of the select pass (hamming_select.cu (A'): tcgen05 filter -> hit masks -> SIMT append; c3 select
-            // 0.61 -> 0.53 ms, c5 5.8 -> 3.7 ms): full 128-query groups, 256-row tiles, e4m3 copies of the codes and the hit
-            // masks in the workspace (bounded: 4 B per (32-row group, query)).  B200_SEL_TC=0: the SIMT kernel alone.
-            const char *tc_env = std::getenv("B200_SEL_TC");
-            const size_t stc_bp = static_cast<size_t>((B + 127) / 128) * 128;
-            const size_t stc_groups = static_cast<size_t>(plan_ceil_div<long long>(N, 256)) * 8;
-            const bool stc = !(tc_env && tc_env[0] == '0') && p.T == 128 && p.Qpad % 128 == 0 &&
-                             stc_groups * p.Qpad * sizeof(uint32_t) <= (4ull << 30) && static_cast<size_t>(N) * stc_bp <= (8ull << 30);
-            plan_stc = stc;
-            long long cps = stc ? 20 : 12;       // (the append half is latency-bound: finer CTAs, 12 -> 20 per SM: 0.42 -> 0.37 ms on c3)
-            if (const char *e = std::getenv("B200_SEL_CTAS_PER_SM")) cps = std::atoll(e) > 0 ? std::atoll(e) : cps;
+            const bool stc = plan_select_tc(p);
+            const long long cps = stc ? 20 : 12;       // (the append half is latency-bound: finer CTAs, 12 -> 20 per SM: 0.42 -> 0.37 ms on c3)
             const long long want = static_cast<long long>(num_sms) * cps;
             // (few query groups — a slice of a multi-GPU run: 512-row segments; 628 queries of c3: select 0.102 -> 0.088 ms,
             // rank 0.044 -> 0.050 ms)
-            long long min_seg = (p.Qpad / p.T) * plan_ceil_div<long long>(N, 1024) < 6ll * num_sms ? 512 : 1024;
-            if (const char *e = std::getenv("B200_SEL_MIN_SEG")) min_seg = std::atoll(e) >= 64 ? std::atoll(e) : min_seg;
+            const long long min_seg = (p.Qpad / p.T) * plan_ceil_div<long long>(N, 1024) < 6ll * num_sms ? 512 : 1024;
             const long long cap_s = plan_ceil_div<long long>(N, min_seg);
             int tsel = p.T;
             // (groups shrink to 64 / 32 queries only when full groups could not give every SM one CTA: measured on a 628-
             // query slice of c3, 128 / 64 / 32 queries per CTA: 0.101 / 0.105 / 0.132 ms)
             if (!stc)
                 while (tsel > 32 && (p.Qpad / tsel) * cap_s < num_sms) tsel >>= 1;
-            if (const char *e = std::getenv("B200_SEL_T")) {
-                const int v = std::atoi(e);
-                if ((v == 32 || v == 64 || v == 128) && v <= p.T) tsel = v;
-            }
             p.sel_T = tsel;
             long long sS = plan_ceil_div<long long>(want, p.Qpad / tsel);
-            if (const char *e = std::getenv("B200_SEL_SEGMENTS")) sS = std::atoll(e);
-            if (sS < 1) sS = 1;
             if (sS > cap_s) sS = cap_s;
             long long sseg = plan_round_up<long long>(plan_ceil_div<long long>(N, sS), stc ? 256 : 64);      // (whole 256-row tiles of the tensor-core kernel)
             const long long sseg_cap = stc ? 65280 : 65472;       // row-in-segment is a 16-bit field of a candidate entry
@@ -167,7 +164,6 @@ inline int map_plan_init(b200_map_plan *plan, int Q, long long N, long long N_to
                     if (ratio < best - 1e-9) best = ratio, mS = c;
                 }
             }
-            if (const char *e = std::getenv("B200_SMP_SEGMENTS")) mS = std::atoll(e) > 0 ? std::atoll(e) : mS;
             const long long m_cap = plan_ceil_div<long long>(p.smp_rows, 128);
             if (mS > m_cap) mS = m_cap;
             if (mS < 1) mS = 1;
@@ -185,7 +181,7 @@ inline int map_plan_init(b200_map_plan *plan, int Q, long long N, long long N_to
             p.off_sel_table = carve(static_cast<size_t>(p.Qpad) * p.sel_S * p.sel_maxc * sizeof(uint32_t));
             p.off_sel_pool = carve(static_cast<size_t>(p.sel_pool_chunks) * p.sel_chunk * sizeof(uint32_t));
             p.off_smp_codes = off;                                // == workspace_bytes: no tensor-core form for this plan
-            if (plan_stc && p.sel_T == 128 && p.sel_seg_len % 256 == 0) {
+            if (plan_select_tc(p)) {
                 // e4m3 copies of the codes for the tensor-core filter (rows padded to 128-byte K blocks) + its hit masks: one
                 // uint32 per (32-row group, query), whole 256-row tiles
                 const size_t bp = static_cast<size_t>((B + 127) / 128) * 128;

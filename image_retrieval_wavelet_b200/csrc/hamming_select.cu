@@ -20,8 +20,6 @@
 // (collapsed codes: every row ties) a device flag hands the whole problem to the three-stage path, whose kernels are
 // launched behind that flag and return at once otherwise.  No host synchronisation anywhere: the sequence is
 // CUDA-graph capturable.
-#include <cstdlib>
-
 #include "common.cuh"
 #include "hamming_core.cuh"
 #include "hamming_plan.h"
@@ -369,7 +367,7 @@ __global__ void __launch_bounds__(128) hamming_select_kernel(const __grid_consta
 }
 
 // ------------------------------------------------------------------------------------------------ (A') select on the tensor cores
-// The default where the plan allows it (B200_SEL_TC=0: the SIMT kernel alone).  The scoring moves off the POPC pipe: for +-1 codes <q, r> = B - 2 d, so the distances of 128
+// Runs where the plan allows it (plan_select_tc in hamming_plan.h).  The scoring moves off the POPC pipe: for +-1 codes <q, r> = B - 2 d, so the distances of 128
 // queries x 256 rows are ONE tcgen05.mma chain over the codes expanded to e4m3 bytes (+1 = 0x38, -1 = 0xB8, padding
 // columns 0; float32 accumulation of at most 256 terms of +-1 is exact).  Two kernels:
 //   hamming_select_tc_kernel (FILTER)  warp 0 TMA producer (query tile 128 x 128 B + row tile 256 x 128 B per 128-column K
@@ -432,7 +430,7 @@ struct StcMaps {
 };
 
 __global__ void __launch_bounds__(kStcThreads, 1) hamming_select_tc_kernel(const __grid_constant__ StcMaps maps, const __grid_constant__ SelArgs a,
-                                                                           int B, int nkb, int dbg) {
+                                                                           int B, int nkb) {
     extern __shared__ unsigned char stc_smem_raw[];
     __shared__ uint32_t s_quit;
     volatile uint32_t *vflags = a.flags;
@@ -544,15 +542,9 @@ __global__ void __launch_bounds__(kStcThreads, 1) hamming_select_tc_kernel(const
                 tc_fence_after();
                 const uint32_t taddr = tmem_base + ab * kStcBN + (static_cast<uint32_t>(quarter * 32) << 16);
                 uint32_t ra[32], rb[32];
-                if (dbg & 16) {                                        // probe: TMA + MMA only
-                    tc_fence_before();
-                    mbar_arrive(&acc_empty[ab]);
-                    continue;
-                }
                 tc_ld32(taddr, ra);
                 tc_ld_wait();
                 auto consume = [&](const uint32_t (&r)[32], int c) {
-                    if (dbg & 8) return;                               // probe: TMEM reads only
                     uint32_t h[4] = {0u, 0u, 0u, 0u};                  // four independent chains
 #pragma unroll
                     for (int j = 0; j < 32; ++j)
@@ -616,8 +608,7 @@ constexpr int kStageCap = 12288;                          // most entries of sha
 // list takes the chunked form) in steps of 512 — c3 (k = 5000): 9728 entries = 55 KB per CTA with the counters, FOUR CTAs per
 // SM instead of three
 inline int rank_stage_cap(uint32_t k) {
-    long long cap = (static_cast<long long>(k) * 9 / 5 + 512 + 511) / 512 * 512;
-    if (const char *e = std::getenv("B200_SEL_STAGE_CAP")) cap = std::atoll(e) / 128 * 128;      // A/B
+    const long long cap = (static_cast<long long>(k) * 9 / 5 + 512 + 511) / 512 * 512;
     return static_cast<int>(cap < 1024 ? 1024 : (cap > kStageCap ? kStageCap : cap));
 }
 __host__ __device__ inline int rank_stage_max_blk(int cap) { return cap / 128 + kStageMaxSeg; }
@@ -991,7 +982,7 @@ static sel_fn pick_app(int cw, int lw, bool eq) {        // the MASKED (append-o
     return nullptr;
 }
 
-using stc_fn = void (*)(const StcMaps, const SelArgs, int, int, int);
+using stc_fn = void (*)(const StcMaps, const SelArgs, int, int);
 
 // The select pipeline in three phases, so that a caller whose database arrives in pieces (b200_maphashing_host: row
 // chunks over PCIe) can score the segments of a chunk while the next chunk is still in flight:
@@ -1020,11 +1011,9 @@ static int sel_args(const b200_map_plan *p, const uint64_t *qc, const uint64_t *
     a.maxc = p->sel_maxc, a.bins = p->bins;
     a.pool_chunks = static_cast<uint32_t>(p->sel_pool_chunks), a.k = static_cast<uint32_t>(p->k);
     a.stage = (p->sel_S <= kStageMaxSeg && (p->sel_chunk >> 7) <= 8) ? 1 : 0;
-    if (const char *e = std::getenv("B200_SEL_STAGE")) a.stage = (a.stage && std::atoi(e) != 0) ? 1 : 0;      // A/B
     a.stage_cap = a.stage ? rank_stage_cap(a.k) : 0;
     a.round = 0, a.seg0 = 0, a.mask = nullptr;
     a.nsub = a.pool_chunks >= 64u * kSubPools ? kSubPools : 1u;
-    if (const char *e = std::getenv("B200_SEL_SUBPOOLS")) a.nsub = (std::atoi(e) > 1 && a.pool_chunks >= kSubPools) ? kSubPools : 1u;      // A/B
     a.sub_chunks = a.pool_chunks / a.nsub;
     *out = a;
     return B200_OK;
@@ -1094,15 +1083,12 @@ int select_finish(const b200_map_plan *p, const uint64_t *qc, const uint64_t *ql
     if (int rc = sel_args(p, qc, ql, dc, dl, ws, ap, tsum, rank_idx, rank_dist, status, &a)) return rc;
     sel_fn fn = pick_sel(cw, p->LW, p->label_mode == B200_LABELS_EQUAL);
     if (!fn) return B200_ERR_UNSUPPORTED;
-    // tensor-core form of the select pass (A'): filter kernel -> hit masks -> append kernel; the plan holds its workspace
+    // tensor-core form of the select pass (A'): filter kernel -> hit masks -> append kernel, where the plan carved its
+    // workspace and the caller has not run round 0 already; the SIMT kernel when the driver cannot encode tensor maps
     const int Bp = (p->B + kStcBK - 1) / kStcBK * kStcBK;
     stc_fn tf = hamming_select_tc_kernel;
     sel_fn af = pick_app(cw, p->LW, p->label_mode == B200_LABELS_EQUAL);
-    bool use_tc = !round0_selected && af && a.tile == 256 && p->sel_T == kStcBM && p->sel_seg_len % kStcBN == 0 && p->Qpad % kStcBM == 0 && encode_tiled_fn() != nullptr;
-    {
-        const char *e = std::getenv("B200_SEL_TC");      // the plan decides (it holds the workspace); 0 here switches it off for A/B
-        use_tc = use_tc && !(e && e[0] == '0') && p->off_smp_codes != p->workspace_bytes && p->sel_seg_len <= 65280;
-    }
+    bool use_tc = !round0_selected && plan_select_tc(*p) && encode_tiled_fn() != nullptr;
     StcMaps maps;
     if (use_tc) {
         unsigned char *db8 = reinterpret_cast<unsigned char *>((reinterpret_cast<uintptr_t>(w + p->off_smp_codes) + 1023) & ~static_cast<uintptr_t>(1023));
@@ -1133,7 +1119,7 @@ int select_finish(const b200_map_plan *p, const uint64_t *qc, const uint64_t *ql
             // (the caller's select_segments launches did this round's select pass)
         } else if (use_tc) {
             const int units = (p->Qpad / kStcBM) * p->sel_S, sms = sm_count();
-            tf<<<units < sms ? units : sms, kStcThreads, kStcSmemBytes, st>>>(maps, a, p->B, Bp / kStcBK, std::getenv("B200_STC_DBG") ? std::atoi(std::getenv("B200_STC_DBG")) : 0);
+            tf<<<units < sms ? units : sms, kStcThreads, kStcSmemBytes, st>>>(maps, a, p->B, Bp / kStcBK);
             B200_LAUNCH_CHECK("hamming_select_tc_kernel");
             stage_mark(round ? "filter_round1" : "filter", st);
             af<<<dim3(p->Qpad / p->sel_T, p->sel_S), p->sel_T, smem, st>>>(a);
@@ -1162,18 +1148,13 @@ int hamming_select_run(const b200_map_plan *p, const uint64_t *qc, const uint64_
 extern "C" int b200_map_select_status(const b200_map_plan *plan, const void *workspace, uint32_t *out4, b200_stream_t stream) {
     using namespace b200;
     if (!plan || !workspace || !out4 || !plan->select) return B200_ERR_INVALID_ARG;
-    uint32_t f[8];
+    uint32_t f[64];                                             // the whole flags block, sub-pool cursors included
     B200_CUDA_TRY(cudaMemcpyAsync(f, static_cast<const unsigned char *>(workspace) + plan->off_sel_flags, sizeof(f),
                                   cudaMemcpyDeviceToHost, as_stream(stream)));
     B200_CUDA_TRY(cudaStreamSynchronize(as_stream(stream)));
     const unsigned long long est = static_cast<unsigned long long>(f[kFlagEst]) | (static_cast<unsigned long long>(f[kFlagEst + 1]) << 32);
     out4[0] = f[kFlagCursor], out4[1] = f[kFlagFallback], out4[2] = f[kFlagRetry];
-    {
-        uint32_t sub[kSubPools];
-        B200_CUDA_TRY(cudaMemcpy(sub, static_cast<const unsigned char *>(workspace) + plan->off_sel_flags + kFlagSubCursor * sizeof(uint32_t),
-                                 sizeof(sub), cudaMemcpyDeviceToHost));
-        for (int i = 0; i < kSubPools; ++i) out4[0] += sub[i];
-    }
+    for (int i = 0; i < kSubPools; ++i) out4[0] += f[kFlagSubCursor + i];
     out4[3] = static_cast<uint32_t>(est / static_cast<unsigned long long>(plan->Q > 0 ? plan->Q : 1));
     return B200_OK;
 }

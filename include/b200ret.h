@@ -180,8 +180,7 @@ typedef struct b200_map_plan {
     int bins, T, groups, Qpad, S, seg_len, wide, tile;
     int stash;         /* 1: stage A keeps (distance, relevance) of every (row, query) pair in the workspace and
                           stage B ranks from that stash instead of scoring again.  Chosen when 4k <= N_total,
-                          B <= 254 and the stash fits B200_MAP_STASH_MAX_MB (default 24576); B200_MAP_STASH=0/1
-                          forces it off / on                                                                  */
+                          B <= 254 and the stash takes less than 24576 MB; B200_MAP_STASH=0/1 forces it off / on */
     size_t off_hist, off_tot, off_dstar, off_psum, off_phits, off_stash_d, off_stash_r, workspace_bytes;
     /* Select mode (single shard, 8k <= N_total, B <= 254; B200_MAP_SELECT=0/1 forces): the top k are a small part of the
      * database, so instead of counting every (row, query) pair into per-distance histograms, a sampled histogram
@@ -191,8 +190,8 @@ typedef struct b200_map_plan {
      * query whose list turns out shorter than k is redone with the bound lifted; a pool overflow hands the whole
      * problem to the three-stage path above, whose kernels are otherwise gated off).  b200_hamming_map and
      * b200_hamming_topk take this path by themselves; the staged API (hist / scan / ap) never does.
-     * The one pass has two forms.  Tensor-core form (default when the queries come in groups of 128 and the hit masks fit
-     * 4 GB; B200_SEL_TC=0 at plan time switches it off): the +-1 codes are expanded to e4m3 bytes and a tcgen05 fp8 GEMM
+     * The one pass has two forms, and the plan alone decides which.  Tensor-core form (when the queries come in groups of
+     * 128, the hit masks fit 4 GB and the e4m3 codes 8 GB): the +-1 codes are expanded to e4m3 bytes and a tcgen05 fp8 GEMM
      * (dot = B - 2 distance, exact) writes one hit bit per (row, query) — off_smp_codes then points at the e4m3 copies and
      * the masks, otherwise off_smp_codes == workspace_bytes — and a SIMT kernel scores only the hit rows again and appends
      * them.  SIMT form: XOR + POPC of every pair in the same kernel that appends. */

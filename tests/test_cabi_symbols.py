@@ -86,29 +86,57 @@ def test_select_planner_rules_for_query_slices():
     assert seen[(8, 40000)][0] == 32                            # too few queries for one CTA per SM: the groups shrink
 
 
+def _plan_for(q, n, bits, lw, k):
+    plan = _cabi.MapPlan()
+    assert _cabi.load().b200_map_plan_init(ctypes.byref(plan), q, n, n, bits, lw, 0, k) == 0
+    return plan
+
+
 def test_plan_decides_the_tensor_core_form(monkeypatch):
     """hamming_plan.h: the tensor-core form of the select pass gets its workspace (e4m3 copies + hit masks, off_smp_codes <
-    workspace_bytes) and 256-row tiles when the queries come in groups of 128 and the masks stay below 4 GB; B200_SEL_TC=0,
-    small query sets and huge databases keep the SIMT kernel (off_smp_codes == workspace_bytes)."""
-    lib = _cabi.load()
-
-    def plan_for(q, n, bits, lw, k):
-        plan = _cabi.MapPlan()
-        assert lib.b200_map_plan_init(ctypes.byref(plan), q, n, n, bits, lw, 0, k) == 0
-        return plan
-
-    monkeypatch.delenv("B200_SEL_TC", raising=False)
-    p = plan_for(5000, 117000, 128, 2, 5000)
+    workspace_bytes) and 256-row tiles when the queries come in groups of 128 and the masks stay below 4 GB; small query
+    sets and huge databases keep the SIMT kernel (off_smp_codes == workspace_bytes).  Every plan with that workspace has
+    the geometry the tensor-core kernels are written for."""
+    monkeypatch.delenv("B200_MAP_SELECT", raising=False)
+    monkeypatch.delenv("B200_SEL_STRIDE", raising=False)
+    p = _plan_for(5000, 117000, 128, 2, 5000)
     assert p.select == 1 and p.off_smp_codes < p.workspace_bytes and p.sel_seg_len % 256 == 0 and p.sel_T == 128
     masks = (117000 + 255) // 256 * 8 * p.Qpad * 4
     assert p.workspace_bytes - p.off_smp_codes >= 117000 * 128 + p.Qpad * 128 + masks
-    p64 = plan_for(10000, 1000000, 64, 2, 5000)                     # 64-bit codes are padded to one 128-byte K block
+    p64 = _plan_for(10000, 1000000, 64, 2, 5000)                    # 64-bit codes are padded to one 128-byte K block
     assert p64.off_smp_codes < p64.workspace_bytes and p64.workspace_bytes - p64.off_smp_codes >= 1000000 * 128
-    small = plan_for(40, 70001, 64, 1, 5000)                        # fewer than 128 queries: SIMT kernel
+    small = _plan_for(40, 70001, 64, 1, 5000)                       # fewer than 128 queries: SIMT kernel
     assert small.select == 1 and small.off_smp_codes == small.workspace_bytes
-    huge = plan_for(10000, 50000000, 64, 2, 5000)                   # the hit masks would take 63 GB: SIMT kernel
+    huge = _plan_for(10000, 50000000, 64, 2, 5000)                  # the hit masks would take 63 GB: SIMT kernel
     assert huge.select == 1 and huge.off_smp_codes == huge.workspace_bytes
-    monkeypatch.setenv("B200_SEL_TC", "0")
-    off = plan_for(5000, 117000, 128, 2, 5000)
-    assert off.select == 1 and off.off_smp_codes == off.workspace_bytes and off.sel_seg_len % 64 == 0
-    assert off.workspace_bytes < p.workspace_bytes
+    tc = 0
+    for q in (40, 64, 128, 130, 256, 300, 628, 1252, 5000, 10000):
+        for n in (40000, 70001, 117000, 1000000, 50000000):
+            for bits in (64, 128, 200):
+                for k in (600, 5000):
+                    pl = _plan_for(q, n, bits, 2, k)
+                    if pl.select and pl.off_smp_codes != pl.workspace_bytes:
+                        tc += 1
+                        assert pl.sel_T == 128 and pl.Qpad % 128 == 0, (q, n, bits, k)
+                        assert pl.sel_seg_len % 256 == 0 and pl.sel_seg_len <= 65280, (q, n, bits, k)
+    assert tc >= 100
+
+
+def test_plan_ignores_former_tuning_overrides(monkeypatch):
+    """Only B200_MAP_SELECT, B200_SEL_STRIDE and B200_MAP_STASH reach the planner: the select geometry, the tensor-core
+    form and the stash budget it once let the environment override are set to values that would change every plan
+    below, and the plans stay the same field for field."""
+    for name in ("B200_MAP_SELECT", "B200_SEL_STRIDE", "B200_MAP_STASH"):
+        monkeypatch.delenv(name, raising=False)
+    shapes = ((5000, 117000, 128, 2, 5000), (628, 117000, 128, 2, 5000), (40, 70001, 64, 1, 5000), (10000, 1000000, 64, 2, 5000),
+              (256, 40000, 128, 1, 600))
+    before = [_plan_for(*s) for s in shapes]
+    # B200_ + name: the select CTAs per SM, minimum segment, query group, segment counts, tensor-core switch, stash budget
+    hostile = {"SEL_CTAS_PER_SM": "1", "SEL_MIN_SEG": "64", "SEL_T": "32", "SEL_SEGMENTS": "3", "SMP_SEGMENTS": "1",
+               "SEL_TC": "0", "MAP_STASH_MAX_MB": "0"}
+    for name, value in hostile.items():
+        monkeypatch.setenv("B200_" + name, value)
+    for s, p0 in zip(shapes, before):
+        p1 = _plan_for(*s)
+        for field, _ in _cabi.MapPlan._fields_:
+            assert getattr(p1, field) == getattr(p0, field), (s, field)

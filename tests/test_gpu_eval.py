@@ -361,16 +361,22 @@ def test_host_buffer_entry_point_chunked_pipeline(monkeypatch, chunks, n, k, nla
 
 @pytest.mark.parametrize("streamed", ["1", "0"])
 @pytest.mark.parametrize("chunks", [2, 3, 8])
-@pytest.mark.parametrize("n,k,bits,nlab,collapse", [(70001, 5000, 64, 24, False), (40000, 600, 128, -1, False), (45000, 1000, 64, 24, True)])
-def test_host_buffer_entry_point_streams_the_select_pipeline(monkeypatch, streamed, chunks, n, k, bits, nlab, collapse):
+@pytest.mark.parametrize("nq,n,k,bits,nlab,collapse", [
+    pytest.param(40, 70001, 5000, 64, 24, False, id="70001-5000-64-24-False"),
+    pytest.param(40, 40000, 600, 128, -1, False, id="40000-600-128--1-False"),
+    pytest.param(40, 45000, 1000, 64, 24, True, id="45000-1000-64-24-True"),
+    pytest.param(200, 70001, 5000, 128, 24, False, id="200q-70001-5000-128-24-False"),
+])
+def test_host_buffer_entry_point_streams_the_select_pipeline(monkeypatch, streamed, chunks, nq, n, k, bits, nlab, collapse):
     """Select plans in b200_maphashing_host: the sample rows cross PCIe first (strided 2-D copy), every chunk's segments are
     scored while the next chunk is in flight (B200_HOST_STREAMED=0: the whole database first).  Same integers and AP as
-    the oracle either way — also when the codes collapse (every row ties: pool overflow -> the gated three stages)."""
+    the oracle either way — also when the codes collapse (every row ties: pool overflow -> the gated three stages).  With
+    128 queries or more the streamed round 0 runs the SIMT select kernel on 128-query groups (the unstreamed call runs the
+    tensor-core form there)."""
     from image_retrieval_wavelet_b200 import _cabi
 
     monkeypatch.setenv("B200_HOST_CHUNKS", str(chunks))
     monkeypatch.setenv("B200_HOST_STREAMED", streamed)
-    nq = 40
     q, ql, r, rl = _problem(n + chunks, nq, n, bits, nlab)
     if collapse:
         r[:] = r[0]
@@ -380,6 +386,9 @@ def test_host_buffer_entry_point_streams_the_select_pipeline(monkeypatch, stream
         lq, lr, mode, L = ql.astype(np.float32), rl.astype(np.float32), 0, nlab
     else:
         lq, lr, mode, L = ql.astype(np.float32).reshape(-1, 1).copy(), rl.astype(np.float32).reshape(-1, 1).copy(), 1, 1
+    plan = _cabi.MapPlan()
+    assert _cabi.load().b200_map_plan_init(ctypes.byref(plan), nq, n, n, bits, words(L), mode, k) == 0
+    assert plan.select == 1 and (plan.sel_T == 128 or nq < 128), (plan.select, plan.sel_T)
     rc = _cabi.load().b200_maphashing_host(q.ctypes.data, lq.ctypes.data, r.ctypes.data, lr.ctypes.data, nq, n, bits, L, mode, k,
                                            ap.ctypes.data, ts.ctypes.data, ctypes.addressof(m), ctypes.addressof(bad))
     assert rc == 0 and bad.value == 0

@@ -2,12 +2,14 @@
 candidate lists -> one warp per query.  Same bar as test_gpu_eval.py: hit counts, ranked indices and distances
 bit-exact, AP within 1e-6 — including the cases where the sample misleads (bound lifted for those queries) and where
 the candidate pool overflows (the gated three-stage path takes over)."""
+import ctypes
+
 import numpy as np
 import pytest
 import torch
 
 from oracle import c_oracle, eval_ref
-from simlib import correlated_codes, multi_hot, pm1
+from simlib import correlated_codes, multi_hot, pm1, words
 
 pytestmark = pytest.mark.gpu
 
@@ -169,17 +171,21 @@ def test_c5_scale_out_shape_query_sample():
     assert abs(m.item() - ap.mean().item()) <= 1e-12
 
 
-@pytest.mark.parametrize("tc", ["1", "0"])
-@pytest.mark.parametrize("nq,n,bits,nlab,k", [(300, 6000, 128, 80, 600), (130, 9000, 64, 24, 700), (256, 5000, 200, -1, 512)])
-def test_tensor_core_select_kernel_agrees(monkeypatch, nq, n, bits, nlab, k, tc):
+@pytest.mark.parametrize("nq,n,bits,nlab,k", [(300, 6000, 128, 80, 600), (130, 9000, 64, 24, 700), (256, 5000, 200, -1, 512),
+                                               (64, 6000, 128, 80, 600), (40, 9000, 64, 24, 700), (33, 5000, 200, -1, 512)])
+def test_tensor_core_select_kernel_agrees(monkeypatch, nq, n, bits, nlab, k):
     """The tcgen05 form of the select pass (distances as e4m3 dot products of the +-1 codes, TMA tiles, TMEM accumulators,
-    hit masks, SIMT append; DESIGN 4.2) and the SIMT kernel alone (B200_SEL_TC=0) give the same lists — hit counts
-    bit-exact, AP within 1e-6 — and the tensor-core form really runs where the plan allows it (its "expand" and "filter"
-    stages show up in the stage times)."""
+    hit masks, SIMT append; DESIGN 4.2), which the plan picks for 128-query groups, and the SIMT kernel, which it picks for
+    fewer queries, give the oracle's lists — hit counts bit-exact, AP within 1e-6 — and the form the plan picks is the one
+    that runs (the tensor-core form's "expand" and "filter" stages show up in the stage times)."""
+    from image_retrieval_wavelet_b200 import _cabi
     from image_retrieval_wavelet_b200.engine.map_engine import HammingMapEngine
 
     monkeypatch.setenv("B200_MAP_SELECT", "1")
-    monkeypatch.setenv("B200_SEL_TC", tc)
+    plan = _cabi.MapPlan()
+    assert _cabi.load().b200_map_plan_init(ctypes.byref(plan), nq, n, n, bits, words(max(nlab, 1)), 0 if nlab > 0 else 1, k) == 0
+    tc = plan.off_smp_codes != plan.workspace_bytes
+    assert plan.select == 1 and tc == (nq >= 128), (plan.select, plan.sel_T)
     rng = np.random.default_rng(nq + n + bits)
     q, r = pm1(rng, nq, bits), pm1(rng, n, bits)
     r[:nq] = q
@@ -193,7 +199,7 @@ def test_tensor_core_select_kernel_agrees(monkeypatch, nq, n, bits, nlab, k, tc)
                              torch.from_numpy(rl).cuda(), k)
     stages = eng.stage_ms()
     eng.close()
-    assert ("expand" in stages and "filter" in stages) == (tc == "1"), stages
+    assert ("expand" in stages and "filter" in stages) == tc, stages
     m0, ap0, ts0, _, _ = eval_ref.maphashing_exact(q, ql, r, rl, k, return_details=True)
     assert np.array_equal(ts.cpu().numpy().astype(np.int64), ts0)
     assert np.abs(ap.cpu().numpy() - ap0).max() <= AP_TOL and abs(m - m0) <= AP_TOL
