@@ -576,17 +576,6 @@ __global__ void __launch_bounds__(kStcThreads, 1) hamming_select_tc_kernel(const
     }
 }
 
-static bool make_map_u8(CUtensorMap *map, const void *base, long long rows, int Bp, int box_rows) {
-    EncodeTiledFn fn = encode_tiled_fn();
-    if (!fn) return false;
-    const cuuint64_t dims[2] = {static_cast<cuuint64_t>(Bp), static_cast<cuuint64_t>(rows)};
-    const cuuint64_t strides[1] = {static_cast<cuuint64_t>(Bp)};
-    const cuuint32_t box[2] = {static_cast<cuuint32_t>(kStcBK), static_cast<cuuint32_t>(box_rows)};
-    const cuuint32_t estr[2] = {1, 1};
-    return fn(map, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<void *>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-              CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
 // ------------------------------------------------------------------------------------------------ (B) rank
 // One CTA per query, kRankWarps warps.  Pass 1: every warp histograms a contiguous (index-order) part of the query's
 // candidates by distance; a CTA-wide scan gives each (warp, distance) its rank / ordinal base and the cut-off distance
@@ -1094,7 +1083,8 @@ int select_finish(const b200_map_plan *p, const uint64_t *qc, const uint64_t *ql
         unsigned char *db8 = reinterpret_cast<unsigned char *>((reinterpret_cast<uintptr_t>(w + p->off_smp_codes) + 1023) & ~static_cast<uintptr_t>(1023));
         unsigned char *q8 = db8 + round_up<size_t>(static_cast<size_t>(p->N) * Bp, 1024);
         a.mask = reinterpret_cast<uint32_t *>(q8 + round_up<size_t>(static_cast<size_t>(p->Qpad) * Bp, 1024));
-        if (!make_map_u8(&maps.q, q8, p->Q, Bp, kStcBM) || !make_map_u8(&maps.db, db8, p->N, Bp, kStcBN)) {
+        if (!make_tensor_map(&maps.q, CU_TENSOR_MAP_DATA_TYPE_UINT8, q8, p->Q, Bp, kStcBM) ||
+            !make_tensor_map(&maps.db, CU_TENSOR_MAP_DATA_TYPE_UINT8, db8, p->N, Bp, kStcBN)) {
             use_tc = false;
         } else {
             const int sms = sm_count();

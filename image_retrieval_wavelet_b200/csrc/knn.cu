@@ -4,13 +4,15 @@
 //
 // v0 (this file): exact float32.  (1) a register-tiled SGEMM writes the Q x N score matrix to the caller's
 // workspace, (2) one CTA per query selects the k best by an MSB-first radix select over order-preserving keys and
-// sorts the survivors with a bitonic network; ties go to the smaller index.  The tensor-core (tcgen05) scorer that
-// replaces step (1) lives in knn_tc.cu when built; this exact path stays as its parity reference and as the
-// D % 16 != 0 fallback.
+// sorts the survivors with a bitonic network; ties go to the smaller index.  For inner products the tensor-core
+// (tcgen05) scorer of knn_tc.cu replaces step (1), and where the shape allows (knn_fused_rank) filters candidates in its
+// epilogue instead of writing the matrix.  The exact path serves L2, B200_KNN_TC=0 and drivers without the tensor-map
+// encoder, and is the tensor-core path's parity reference.
 #include <cmath>
 #include <cstdlib>
 
 #include "common.cuh"
+#include "knn_tc.h"
 
 namespace b200 {
 
@@ -33,16 +35,6 @@ __global__ void __launch_bounds__(256) row_sqnorm_kernel(const float *__restrict
     for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
     if (lane == 0) out[warp] = s;
 }
-
-// knn_tc.cu
-size_t knn_tc_extra_workspace(int Q, long long N, int D);
-struct TcContextOpaque {
-    alignas(64) unsigned char bytes[8 * 128 + 64];      // TcContext: eight 128-byte tensor maps + sizes
-};
-int knn_tc_prepare(const float *queries, const float *refs, int Q, long long N, int D, void *extra, long long sample_stride,
-                   TcContextOpaque *ctx, cudaStream_t st);
-int knn_tc_scores(const TcContextOpaque *ctx, int sample, float *S, long long ldS, const float *thr, unsigned long long *cand,
-                  uint32_t *cand_cnt, uint32_t cap, const uint32_t *gate, cudaStream_t st);
 
 // S[q][n] = <Q[q], R[n]>   (l2: sqrt(max(|q|^2 + |r|^2 - 2<q,r>, 0)))     Q: [M][D], R: [N][D], D % 4 == 0; row stride ldS
 __global__ void __launch_bounds__(256) knn_scores_kernel(const float *__restrict__ Qm, const float *__restrict__ Rm,
@@ -138,6 +130,66 @@ __device__ __forceinline__ void radix_pick_digit(const uint32_t *hist, uint32_t 
     }
 }
 
+__host__ __device__ constexpr int pow2_ceil(int k) { int p = 1; while (p < k) p <<= 1; return p; }
+
+// a[0 .. n) descending, n a power of two, by 256 threads (a in shared memory; ends with __syncthreads)
+template <typename T>
+__device__ __forceinline__ void bitonic_sort_desc(T *a, int n, int tid) {
+    for (int size = 2; size <= n; size <<= 1) {
+        for (int st = size >> 1; st > 0; st >>= 1) {
+            for (int i = tid; i < n / 2; i += 256) {
+                const int lo = 2 * i - (i & (st - 1)), hi = lo + st;
+                const bool desc = ((lo & size) == 0);
+                const T x = a[lo], y = a[hi];
+                if ((x < y) == desc) a[lo] = y, a[hi] = x;
+            }
+            __syncthreads();
+        }
+    }
+}
+
+// The k best of cnt distinct (key << 32 | ~idx) pairs in shared memory, best first, to idx_out / score_out [0 .. k): the
+// exact k-th largest pair by an MSB-first radix select, then only the k winners, zero-padded to P = pow2_ceil(k) in
+// top [P], are sorted.  hist [256], need, pref and top_cnt are the caller's shared scratch; 256 threads.
+__device__ __forceinline__ void select_top_pairs(const unsigned long long *pairs, uint32_t cnt, int k, int P, unsigned long long *top,
+                                                 int64_t *idx_out, float *score_out, bool largest, uint32_t *hist, uint32_t *need,
+                                                 unsigned long long *pref, uint32_t *top_cnt, int tid) {
+    if (tid == 0) *pref = 0ull, *need = static_cast<uint32_t>(k);
+    __syncthreads();
+    for (int shift = 56; shift >= 0; shift -= 8) {
+        hist[tid] = 0;
+        __syncthreads();
+        const unsigned long long pf = *pref;
+        for (uint32_t i = tid; i < cnt; i += 256) {
+            const unsigned long long pr = pairs[i];
+            if (shift == 56 || (pr >> (shift + 8)) == (pf >> (shift + 8))) atomicAdd(&hist[(pr >> shift) & 255ull], 1u);
+        }
+        __syncthreads();
+        if (tid < 32) {
+            __shared__ uint32_t s_digit;
+            radix_pick_digit(hist, *need, tid, &s_digit, need);
+            __syncwarp();
+            if (tid == 0) *pref = pf | (static_cast<unsigned long long>(s_digit) << shift);
+        }
+        __syncthreads();
+    }
+    const unsigned long long kth = *pref;
+    if (tid == 0) *top_cnt = 0;
+    for (int i = tid; i < P; i += 256) top[i] = 0ull;
+    __syncthreads();
+    for (uint32_t i = tid; i < cnt; i += 256) {
+        const unsigned long long pr = pairs[i];
+        if (pr >= kth) top[atomicAdd(top_cnt, 1u)] = pr;             // exactly k of them
+    }
+    __syncthreads();
+    bitonic_sort_desc(top, P, tid);
+    for (int i = tid; i < k; i += 256) {
+        const unsigned long long pr = top[i];
+        idx_out[i] = static_cast<int64_t>(0xffffffffu - static_cast<uint32_t>(pr));
+        score_out[i] = rank_key_inv(static_cast<uint32_t>(pr >> 32), largest);
+    }
+}
+
 // One CTA (256 threads) per query row: the k largest keys (rank_key: larger scores first, or smaller distances for L2;
 // NaN last), ties to the smaller index, sorted best-first.
 // Lists longer than kKnnMaxK come out in passes of <= kKnnMaxK ranks: pass p only sees the entries that rank strictly
@@ -157,8 +209,7 @@ __global__ void __launch_bounds__(256) knn_select_kernel(const float *__restrict
     const float *row = S + static_cast<size_t>(blockIdx.x) * ldS;
     int64_t *orow_idx = idx_out + static_cast<size_t>(blockIdx.x) * ldo + k_done;          // where this pass writes its ranks
     float *orow_score = score_out + static_cast<size_t>(blockIdx.x) * ldo + k_done;
-    int P = 1;
-    while (P < k) P <<= 1;
+    const int P = pow2_ceil(k);
     // entries at or before the previous pass' last one are out of the game: their key reads as 0 ... but 0 is also a
     // legal key (NaN), so eligibility is carried separately
     unsigned long long bound = ~0ull;                     // exclusive upper bound on (key << 32 | ~idx)
@@ -179,17 +230,7 @@ __global__ void __launch_bounds__(256) knn_select_kernel(const float *__restrict
         const long long stride = N / kKnnSample;
         for (int i = tid; i < kKnnSample; i += 256) s_samp[i] = key_of(static_cast<long long>(i) * stride);
         __syncthreads();
-        for (int size = 2; size <= kKnnSample; size <<= 1) {
-            for (int st = size >> 1; st > 0; st >>= 1) {
-                for (int i = tid; i < kKnnSample / 2; i += 256) {
-                    const int lo = 2 * i - (i & (st - 1)), hi = lo + st;
-                    const bool desc = ((lo & size) == 0);
-                    const uint32_t a = s_samp[lo], b = s_samp[hi];
-                    if ((a < b) == desc) s_samp[lo] = b, s_samp[hi] = a;
-                }
-                __syncthreads();
-            }
-        }
+        bitonic_sort_desc(s_samp, kKnnSample, tid);
         const uint32_t thr = s_samp[fast_rank - 1];
         if (tid == 0) s_cnt_gt = 0;
         __syncthreads();
@@ -240,55 +281,8 @@ __global__ void __launch_bounds__(256) knn_select_kernel(const float *__restrict
         const uint32_t cnt = s_cnt_gt;
         __syncthreads();
         if (cnt >= static_cast<uint32_t>(k) && cnt <= static_cast<uint32_t>(kKnnCand)) {
-            // exact k-th largest (key, ~index) pair among the candidates: MSB-first radix select over the 64-bit pairs
-            // (all distinct), then only the k winners are sorted
-            unsigned long long *s_top = s_pair + kKnnCand;                 // [P]
             __shared__ unsigned long long s_pref;
-            if (tid == 0) s_pref = 0ull, s_need = static_cast<uint32_t>(k);
-            __syncthreads();
-            for (int shift = 56; shift >= 0; shift -= 8) {
-                s_hist[tid] = 0;
-                __syncthreads();
-                const unsigned long long pref = s_pref;
-                for (uint32_t i = tid; i < cnt; i += 256) {
-                    const unsigned long long pr = s_pair[i];
-                    if (shift == 56 || (pr >> (shift + 8)) == (pref >> (shift + 8))) atomicAdd(&s_hist[(pr >> shift) & 255ull], 1u);
-                }
-                __syncthreads();
-                if (tid < 32) {
-                    __shared__ uint32_t s_digit;
-                    radix_pick_digit(s_hist, s_need, tid, &s_digit, &s_need);
-                    __syncwarp();
-                    if (tid == 0) s_pref = pref | (static_cast<unsigned long long>(s_digit) << shift);
-                }
-                __syncthreads();
-            }
-            const unsigned long long kth = s_pref;
-            if (tid == 0) s_cnt_gt = 0;
-            for (int i = tid; i < P; i += 256) s_top[i] = 0ull;
-            __syncthreads();
-            for (uint32_t i = tid; i < cnt; i += 256) {
-                const unsigned long long pr = s_pair[i];
-                if (pr >= kth) s_top[atomicAdd(&s_cnt_gt, 1u)] = pr;             // exactly k of them
-            }
-            __syncthreads();
-            for (int size = 2; size <= P; size <<= 1) {
-                for (int st = size >> 1; st > 0; st >>= 1) {
-                    for (int i = tid; i < P / 2; i += 256) {
-                        const int lo = 2 * i - (i & (st - 1)), hi = lo + st;
-                        const bool desc = ((lo & size) == 0);
-                        const unsigned long long a = s_top[lo], b = s_top[hi];
-                        if ((a < b) == desc) s_top[lo] = b, s_top[hi] = a;
-                    }
-                    __syncthreads();
-                }
-            }
-            for (int i = tid; i < k; i += 256) {
-                const unsigned long long pr = s_top[i];
-                const uint32_t u = static_cast<uint32_t>(pr >> 32);
-                orow_idx[i] = static_cast<int64_t>(0xffffffffu - static_cast<uint32_t>(pr));
-                orow_score[i] = rank_key_inv(u, !l2);
-            }
+            select_top_pairs(s_pair, cnt, k, P, s_pair + kKnnCand, orow_idx, orow_score, !l2, s_hist, &s_need, &s_pref, &s_cnt_gt, tid);
             return;
         }
     }
@@ -306,10 +300,10 @@ __global__ void __launch_bounds__(256) knn_select_kernel(const float *__restrict
         }
         __syncthreads();
         if (tid < 32) {
-            __shared__ uint32_t s_digit2;
-            radix_pick_digit(s_hist, s_need, tid, &s_digit2, &s_need);   // s_need: keys with this digit (and prefix) still wanted
+            __shared__ uint32_t s_digit;
+            radix_pick_digit(s_hist, s_need, tid, &s_digit, &s_need);     // s_need: keys with this digit (and prefix) still wanted
             __syncwarp();
-            if (tid == 0) s_prefix = prefix | (s_digit2 << shift);
+            if (tid == 0) s_prefix = prefix | (s_digit << shift);
         }
         __syncthreads();
     }
@@ -353,19 +347,7 @@ __global__ void __launch_bounds__(256) knn_select_kernel(const float *__restrict
         __syncthreads();                         // s_scan is rewritten by the next chunk
     }
     __syncthreads();
-    // ---- bitonic sort, descending on the 64-bit pair (padding zeros sink to the end)
-    for (int size = 2; size <= P; size <<= 1) {
-        for (int stride = size >> 1; stride > 0; stride >>= 1) {
-            for (int i = tid; i < P / 2; i += 256) {
-                const int lo = 2 * i - (i & (stride - 1));
-                const int hi = lo + stride;
-                const bool desc = ((lo & size) == 0);
-                const unsigned long long a = s_pair[lo], b = s_pair[hi];
-                if ((a < b) == desc) s_pair[lo] = b, s_pair[hi] = a;
-            }
-            __syncthreads();
-        }
-    }
+    bitonic_sort_desc(s_pair, P, tid);                // padding zeros sink to the end
     for (int i = tid; i < k; i += 256) {
         const unsigned long long pr = s_pair[i];
         const uint32_t u = static_cast<uint32_t>(pr >> 32);
@@ -376,15 +358,14 @@ __global__ void __launch_bounds__(256) knn_select_kernel(const float *__restrict
 }
 
 // Top-k of a candidate list written by the filtering epilogue of the tensor-core scorer (knn_tc.cu): one CTA per query;
-// cnt pairs (key << 32 | ~idx), all distinct.  The exact k-th largest pair by an MSB-first radix select, then only the k
-// winners are sorted.  A list that is too short (threshold above the k-th neighbour) or overflowed raises *fail: the
-// caller's gated launches then redo the whole call through the score matrix.
+// cnt pairs (key << 32 | ~idx), all distinct, staged in shared memory for select_top_pairs.  A list that is too short
+// (threshold above the k-th neighbour) or overflowed raises *fail: the caller's gated launches then redo the whole call
+// through the score matrix.
 __global__ void __launch_bounds__(256) knn_select_cand_kernel(const unsigned long long *__restrict__ cand, const uint32_t *__restrict__ cand_cnt,
                                                               uint32_t cap, int k, int64_t *__restrict__ idx_out,
                                                               float *__restrict__ score_out, uint32_t *__restrict__ fail) {
     extern __shared__ __align__(16) unsigned char knn_smem[];
-    unsigned long long *s_pair = reinterpret_cast<unsigned long long *>(knn_smem);    // [cap]
-    unsigned long long *s_top = s_pair + cap;                                          // [P]
+    unsigned long long *s_pair = reinterpret_cast<unsigned long long *>(knn_smem);    // [cap], then the top array [P]
     __shared__ uint32_t s_hist[256];
     __shared__ uint32_t s_need, s_cnt;
     __shared__ unsigned long long s_pref;
@@ -394,54 +375,11 @@ __global__ void __launch_bounds__(256) knn_select_cand_kernel(const unsigned lon
         if (tid == 0) *fail = 1u;
         return;
     }
-    int P = 1;
-    while (P < k) P <<= 1;
+    const int P = pow2_ceil(k);
     const unsigned long long *list = cand + static_cast<size_t>(blockIdx.x) * cap;
     for (uint32_t i = tid; i < cnt; i += 256) s_pair[i] = list[i];
-    if (tid == 0) s_pref = 0ull, s_need = static_cast<uint32_t>(k);
-    __syncthreads();
-    for (int shift = 56; shift >= 0; shift -= 8) {
-        s_hist[tid] = 0;
-        __syncthreads();
-        const unsigned long long pref = s_pref;
-        for (uint32_t i = tid; i < cnt; i += 256) {
-            const unsigned long long pr = s_pair[i];
-            if (shift == 56 || (pr >> (shift + 8)) == (pref >> (shift + 8))) atomicAdd(&s_hist[(pr >> shift) & 255ull], 1u);
-        }
-        __syncthreads();
-        if (tid < 32) {
-            __shared__ uint32_t s_digit;
-            radix_pick_digit(s_hist, s_need, tid, &s_digit, &s_need);
-            __syncwarp();
-            if (tid == 0) s_pref = pref | (static_cast<unsigned long long>(s_digit) << shift);
-        }
-        __syncthreads();
-    }
-    const unsigned long long kth = s_pref;
-    if (tid == 0) s_cnt = 0;
-    for (int i = tid; i < P; i += 256) s_top[i] = 0ull;
-    __syncthreads();
-    for (uint32_t i = tid; i < cnt; i += 256) {
-        const unsigned long long pr = s_pair[i];
-        if (pr >= kth) s_top[atomicAdd(&s_cnt, 1u)] = pr;             // exactly k of them
-    }
-    __syncthreads();
-    for (int size = 2; size <= P; size <<= 1) {
-        for (int st = size >> 1; st > 0; st >>= 1) {
-            for (int i = tid; i < P / 2; i += 256) {
-                const int lo = 2 * i - (i & (st - 1)), hi = lo + st;
-                const bool desc = ((lo & size) == 0);
-                const unsigned long long a = s_top[lo], b = s_top[hi];
-                if ((a < b) == desc) s_top[lo] = b, s_top[hi] = a;
-            }
-            __syncthreads();
-        }
-    }
-    for (int i = tid; i < k; i += 256) {
-        const unsigned long long pr = s_top[i];
-        idx_out[static_cast<size_t>(blockIdx.x) * k + i] = static_cast<int64_t>(0xffffffffu - static_cast<uint32_t>(pr));
-        score_out[static_cast<size_t>(blockIdx.x) * k + i] = rank_key_inv(static_cast<uint32_t>(pr >> 32), true);
-    }
+    select_top_pairs(s_pair, cnt, k, P, s_pair + cap, idx_out + static_cast<size_t>(blockIdx.x) * k,
+                     score_out + static_cast<size_t>(blockIdx.x) * k, true, s_hist, &s_need, &s_pref, &s_cnt, tid);
 }
 
 // thr[q] = rank-th largest score of the sample row (the last of the sorted top-`rank` list the select kernel wrote)
@@ -500,8 +438,7 @@ static int knn_select_passes(const float *S, long long N, long long ldS, int Q, 
                                        static_cast<int>((kKnnCand + kKnnMaxK) * sizeof(unsigned long long))));
     for (int done = 0; done < k; done += kKnnMaxK) {
         const int kp = k - done < kKnnMaxK ? k - done : kKnnMaxK;
-        int P = 1;
-        while (P < kp) P <<= 1;
+        const int P = pow2_ceil(kp);
         // one-pass threshold path: sample rank r such that P(threshold above the last wanted rank) ~ 4 sigma, and the
         // expected number of eligible keys >= threshold (plus 4 sigma) fits the candidate buffer; else the radix select alone
         int fast_rank = 0;
@@ -548,40 +485,36 @@ int b200_knn_topk(const float *refs, const float *queries, int Q, long long N, i
     unsigned char *fz = w + off;                               // fused scratch: sample top list (idx, score), thr, counters
     off += round_up<size_t>(static_cast<size_t>(Q) * (kKnnMaxK * 12 + 16), 256) + 256;
     void *extra = w + off;
-    const uint32_t *gate = nullptr;
     if (knn_use_tc(metric_l2)) {
-        TcContextOpaque ctx;
-        const int rank = getenv("B200_KNN_FUSED") && getenv("B200_KNN_FUSED")[0] == '0' ? 0 : knn_fused_rank(N, k);
-        int rc = knn_tc_prepare(queries, refs, Q, N, D, extra, rank ? kKnnSampleStride : 0, &ctx, st);
-        if (rc == B200_OK && rank) {
-            // ---- fused path: threshold from a sampled pass, then the full GEMM keeps only the candidates
-            const long long ns = N / kKnnSampleStride, lds = knn_ld(ns);
-            int64_t *top_idx = reinterpret_cast<int64_t *>(fz);
-            float *top_score = reinterpret_cast<float *>(fz + static_cast<size_t>(Q) * rank * 8);
-            float *thr = top_score + static_cast<size_t>(Q) * rank;
-            uint32_t *cand_cnt = reinterpret_cast<uint32_t *>(thr + Q);
-            uint32_t *fail = cand_cnt + Q;
-            if (int e = knn_tc_scores(&ctx, 1, S, lds, nullptr, nullptr, nullptr, 0, nullptr, st)) return e;      // sample scores in S
-            if (int e = knn_select_passes(S, ns, lds, Q, rank, 0, top_idx, top_score, nullptr, st)) return e;
-            knn_threshold_kernel<<<ceil_div(Q, 256), 256, 0, st>>>(top_score, rank, Q, thr, cand_cnt, fail);
-            B200_LAUNCH_CHECK("knn_threshold_kernel");
-            if (int e = knn_tc_scores(&ctx, 0, nullptr, 0, thr, cand, cand_cnt, kKnnFusedCap, nullptr, st)) return e;
-            int P = 1;
-            while (P < k) P <<= 1;
-            const size_t smem = (static_cast<size_t>(kKnnFusedCap) + P) * sizeof(unsigned long long);
-            B200_CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void *>(knn_select_cand_kernel),
-                                               cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                               static_cast<int>((kKnnFusedCap + kKnnMaxK) * sizeof(unsigned long long))));
-            knn_select_cand_kernel<<<Q, 256, smem, st>>>(cand, cand_cnt, kKnnFusedCap, k, idx, score, fail);
-            B200_LAUNCH_CHECK("knn_select_cand_kernel");
-            // any list too short / overflowed: the launches below redo the call through the score matrix, else they return at once
-            gate = fail;
+        TcContext ctx;
+        const int rank = knn_fused_rank(N, k);
+        const int rc = knn_tc_prepare(queries, refs, Q, N, D, extra, rank ? kKnnSampleStride : 0, &ctx, st);
+        if (rc == B200_OK) {
+            const uint32_t *gate = nullptr;
+            if (rank) {
+                // ---- fused path: threshold from a sampled pass, then the full GEMM keeps only the candidates
+                const long long ns = N / kKnnSampleStride, lds = knn_ld(ns);
+                int64_t *top_idx = reinterpret_cast<int64_t *>(fz);
+                float *top_score = reinterpret_cast<float *>(fz + static_cast<size_t>(Q) * rank * 8);
+                float *thr = top_score + static_cast<size_t>(Q) * rank;
+                uint32_t *cand_cnt = reinterpret_cast<uint32_t *>(thr + Q);
+                uint32_t *fail = cand_cnt + Q;
+                if (int e = knn_tc_scores(&ctx, 1, S, lds, nullptr, nullptr, nullptr, 0, nullptr, st)) return e;      // sample scores in S
+                if (int e = knn_select_passes(S, ns, lds, Q, rank, 0, top_idx, top_score, nullptr, st)) return e;
+                knn_threshold_kernel<<<ceil_div(Q, 256), 256, 0, st>>>(top_score, rank, Q, thr, cand_cnt, fail);
+                B200_LAUNCH_CHECK("knn_threshold_kernel");
+                if (int e = knn_tc_scores(&ctx, 0, nullptr, 0, thr, cand, cand_cnt, kKnnFusedCap, nullptr, st)) return e;
+                const size_t smem = (static_cast<size_t>(kKnnFusedCap) + pow2_ceil(k)) * sizeof(unsigned long long);
+                B200_CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void *>(knn_select_cand_kernel),
+                                                   cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                   static_cast<int>((kKnnFusedCap + kKnnMaxK) * sizeof(unsigned long long))));
+                knn_select_cand_kernel<<<Q, 256, smem, st>>>(cand, cand_cnt, kKnnFusedCap, k, idx, score, fail);
+                B200_LAUNCH_CHECK("knn_select_cand_kernel");
+                // any list too short / overflowed: the launches below redo the call through the score matrix, else they return at once
+                gate = fail;
+            }
             if (int e = knn_tc_scores(&ctx, 0, S, ldS, nullptr, nullptr, nullptr, 0, gate, st)) return e;
             return knn_select_passes(S, N, ldS, Q, k, 0, idx, score, gate, st);
-        }
-        if (rc == B200_OK) {
-            if (int e = knn_tc_scores(&ctx, 0, S, ldS, nullptr, nullptr, nullptr, 0, nullptr, st)) return e;
-            return knn_select_passes(S, N, ldS, Q, k, 0, idx, score, nullptr, st);
         }
         if (rc != B200_ERR_UNSUPPORTED) return rc;
     }

@@ -16,6 +16,7 @@
 #include <cuda_bf16.h>
 
 #include "common.cuh"
+#include "knn_tc.h"
 #include "tc_common.cuh"
 
 namespace b200 {
@@ -48,10 +49,6 @@ __global__ void __launch_bounds__(256) knn_split_bf16_kernel(const float *__rest
 // kind::f16: D float32, A/B bfloat16, both K-major, M = 128, N = 256
 constexpr uint32_t kTcIdesc = (1u << 4) | (1u << 7) | (1u << 10) | (static_cast<uint32_t>(kTcBN >> 3) << 17) |
                               (static_cast<uint32_t>(kTcBM >> 4) << 24);
-
-struct TcMaps {
-    CUtensorMap q_hi, q_lo, r_hi, r_lo;
-};
 
 // Epilogue modes: `filt.thr == nullptr`: the score tile is stored to S (row stride ldS).  Otherwise the scores never
 // reach memory: a score that reaches its query's threshold thr[m] is appended — (order-preserving key << 32 | ~index) —
@@ -212,51 +209,13 @@ __global__ void __launch_bounds__(kTcThreads, 1) knn_scores_tc_kernel(const __gr
 }
 
 // ---- host side ---------------------------------------------------------------------------------------------------
-static bool make_map(CUtensorMap *map, const void *base, long long rows, int Dp, int box_rows) {
-    EncodeTiledFn fn = encode_tiled_fn();
-    if (!fn) return false;
-    const cuuint64_t dims[2] = {static_cast<cuuint64_t>(Dp), static_cast<cuuint64_t>(rows)};
-    const cuuint64_t strides[1] = {static_cast<cuuint64_t>(Dp) * 2};
-    const cuuint32_t box[2] = {static_cast<cuuint32_t>(kTcBK), static_cast<cuuint32_t>(box_rows)};
-    const cuuint32_t estr[2] = {1, 1};
-    return fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void *>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-              CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
 size_t knn_tc_extra_workspace(int Q, long long N, int D) {
     const size_t Dp = round_up<size_t>(D, kTcBK);
     return round_up<size_t>(2 * (static_cast<size_t>(Q) + static_cast<size_t>(N)) * Dp * sizeof(__nv_bfloat16), 1024) + 1024;
 }
 
-// bf16 hi / lo copies of both operands + their tensor maps; `r_*_s` read every `sample_stride`-th reference row (a tensor
-// map with a longer row stride: no gather pass).
-struct TcContext {
-    TcMaps full, sample;
-    int Q, Dp;
-    long long N, Ns;
-};
-
-static bool make_map_strided(CUtensorMap *map, const void *base, long long rows, int Dp, int box_rows, long long row_stride_rows) {
-    EncodeTiledFn fn = encode_tiled_fn();
-    if (!fn) return false;
-    const cuuint64_t dims[2] = {static_cast<cuuint64_t>(Dp), static_cast<cuuint64_t>(rows)};
-    const cuuint64_t strides[1] = {static_cast<cuuint64_t>(Dp) * 2 * static_cast<cuuint64_t>(row_stride_rows)};
-    const cuuint32_t box[2] = {static_cast<cuuint32_t>(kTcBK), static_cast<cuuint32_t>(box_rows)};
-    const cuuint32_t estr[2] = {1, 1};
-    return fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void *>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-              CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
-// Splits both operands into bf16 hi + lo (two launches) and builds the tensor maps.  sample_stride > 0 also builds maps
-// over every sample_stride-th reference row.  B200_ERR_UNSUPPORTED when the tensor-map entry point is unavailable.
-struct TcContextOpaque {
-    alignas(64) unsigned char bytes[8 * 128 + 64];
-};
-static_assert(sizeof(TcContext) <= sizeof(TcContextOpaque), "TcContextOpaque (knn.cu) must hold a TcContext");
-
 int knn_tc_prepare(const float *queries, const float *refs, int Q, long long N, int D, void *extra, long long sample_stride,
-                   TcContextOpaque *opaque, cudaStream_t st) {
-    TcContext *ctx = reinterpret_cast<TcContext *>(opaque);
+                   TcContext *ctx, cudaStream_t st) {
     const int Dp = static_cast<int>(round_up<size_t>(D, kTcBK));
     unsigned char *base = reinterpret_cast<unsigned char *>((reinterpret_cast<uintptr_t>(extra) + 1023) & ~static_cast<uintptr_t>(1023));
     __nv_bfloat16 *q_hi = reinterpret_cast<__nv_bfloat16 *>(base);
@@ -264,14 +223,15 @@ int knn_tc_prepare(const float *queries, const float *refs, int Q, long long N, 
     __nv_bfloat16 *r_hi = q_lo + static_cast<size_t>(Q) * Dp;
     __nv_bfloat16 *r_lo = r_hi + static_cast<size_t>(N) * Dp;
     ctx->Q = Q, ctx->Dp = Dp, ctx->N = N, ctx->Ns = 0;
-    if (!make_map(&ctx->full.q_hi, q_hi, Q, Dp, kTcBM) || !make_map(&ctx->full.q_lo, q_lo, Q, Dp, kTcBM) ||
-        !make_map(&ctx->full.r_hi, r_hi, N, Dp, kTcBN) || !make_map(&ctx->full.r_lo, r_lo, N, Dp, kTcBN))
+    const CUtensorMapDataType bf16 = CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+    if (!make_tensor_map(&ctx->full.q_hi, bf16, q_hi, Q, Dp, kTcBM) || !make_tensor_map(&ctx->full.q_lo, bf16, q_lo, Q, Dp, kTcBM) ||
+        !make_tensor_map(&ctx->full.r_hi, bf16, r_hi, N, Dp, kTcBN) || !make_tensor_map(&ctx->full.r_lo, bf16, r_lo, N, Dp, kTcBN))
         return B200_ERR_UNSUPPORTED;
     if (sample_stride > 0) {
         ctx->Ns = N / sample_stride;
         ctx->sample.q_hi = ctx->full.q_hi, ctx->sample.q_lo = ctx->full.q_lo;
-        if (!make_map_strided(&ctx->sample.r_hi, r_hi, ctx->Ns, Dp, kTcBN, sample_stride) ||
-            !make_map_strided(&ctx->sample.r_lo, r_lo, ctx->Ns, Dp, kTcBN, sample_stride))
+        if (!make_tensor_map(&ctx->sample.r_hi, bf16, r_hi, ctx->Ns, Dp, kTcBN, sample_stride) ||
+            !make_tensor_map(&ctx->sample.r_lo, bf16, r_lo, ctx->Ns, Dp, kTcBN, sample_stride))
             return B200_ERR_UNSUPPORTED;
     }
     const int sms = sm_count();
@@ -284,11 +244,8 @@ int knn_tc_prepare(const float *queries, const float *refs, int Q, long long N, 
     return B200_OK;
 }
 
-// One pass of the scorer: sample != 0 scores the sampled reference rows (Ns columns), else all N.  thr == nullptr: the
-// score matrix goes to S; otherwise the epilogue filters (see TcFilter).
-int knn_tc_scores(const TcContextOpaque *opaque, int sample, float *S, long long ldS, const float *thr, unsigned long long *cand,
+int knn_tc_scores(const TcContext *ctx, int sample, float *S, long long ldS, const float *thr, unsigned long long *cand,
                   uint32_t *cand_cnt, uint32_t cap, const uint32_t *gate, cudaStream_t st) {
-    const TcContext *ctx = reinterpret_cast<const TcContext *>(opaque);
     const long long n = sample ? ctx->Ns : ctx->N;
     const int sms = sm_count();
     const long long tiles = static_cast<long long>((ctx->Q + kTcBM - 1) / kTcBM) * ((n + kTcBN - 1) / kTcBN);

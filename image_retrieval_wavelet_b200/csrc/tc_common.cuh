@@ -72,4 +72,20 @@ inline EncodeTiledFn encode_tiled_fn() {
     return fn;
 }
 
+// 2-D tensor map over `rows` rows of `row_elems` elements (bf16 or u8), row i at base + i * row_stride_rows rows, 128-byte
+// swizzle; the box is one 128-byte swizzle row wide (64 bf16 or 128 u8) by box_rows.  False when the driver's encoder is
+// unavailable or rejects the map.
+inline bool make_tensor_map(CUtensorMap *map, CUtensorMapDataType type, const void *base, long long rows, int row_elems, int box_rows,
+                            long long row_stride_rows = 1) {
+    EncodeTiledFn fn = encode_tiled_fn();
+    if (!fn) return false;
+    const cuuint64_t esize = type == CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 ? 2 : 1;
+    const cuuint64_t dims[2] = {static_cast<cuuint64_t>(row_elems), static_cast<cuuint64_t>(rows)};
+    const cuuint64_t strides[1] = {static_cast<cuuint64_t>(row_elems) * esize * static_cast<cuuint64_t>(row_stride_rows)};
+    const cuuint32_t box[2] = {static_cast<cuuint32_t>(128 / esize), static_cast<cuuint32_t>(box_rows)};
+    const cuuint32_t estr[2] = {1, 1};
+    return fn(map, type, 2, const_cast<void *>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
+              CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+}
+
 }  // namespace b200

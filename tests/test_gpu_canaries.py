@@ -99,16 +99,16 @@ def test_select_pool_overflow_stays_inside_the_pool(monkeypatch):
     assert int(ts.view(torch.int32)[3]) == hits and abs(float(ap.view(torch.float64)[3]) - want) <= 1e-6
 
 
-@pytest.mark.parametrize("fused,k,n,top_tie", [pytest.param("1", 1000, 70000, False, id="1-1000-70000"),
-                                               pytest.param("0", 1000, 70000, False, id="0-1000-70000"),
-                                               pytest.param("1", 5000, 20000, False, id="1-5000-20000"),
-                                               pytest.param("1", 2048, 70001, True, id="1-2048-70001-top_tie")])
-def test_knn_topk_stays_inside_its_buffers(monkeypatch, fused, k, n, top_tie):
-    """top_tie: every 7th row is the best row of every query (integer inputs, 10 001 exact ties): the fused path's
-    candidate lists and the select kernel's candidate buffer overflow, and the fallbacks run."""
+@pytest.mark.parametrize("k,n,top_tie", [pytest.param(1000, 70000, False, id="1000-70000"),
+                                         pytest.param(1000, 65535, False, id="1000-65535"),
+                                         pytest.param(5000, 20000, False, id="5000-20000"),
+                                         pytest.param(2048, 70001, True, id="2048-70001-top_tie")])
+def test_knn_topk_stays_inside_its_buffers(k, n, top_tie):
+    """N = 70 000 takes the fused path, N = 65 535 (one row below it) and k = 5000 the score matrix.  top_tie: every
+    7th row is the best row of every query (integer inputs, 10 001 exact ties): the fused path's candidate lists and the
+    select kernel's candidate buffer overflow, and the fallbacks run."""
     from image_retrieval_wavelet_b200 import _cabi
 
-    monkeypatch.setenv("B200_KNN_FUSED", fused)
     g = torch.Generator().manual_seed(n)
     nq, d = 70, 64
     if top_tie:

@@ -100,9 +100,10 @@ def bits_equal(a, b):
 
 # ------------------------------------------------------------------------------------------------ routes + probe
 COSINE_ROUTES = {
-    "tc": {"B200_KNN_TC": "1", "B200_KNN_FUSED": "0"},      # tcgen05 scorer, score matrix, knn_select_kernel
-    "fused": {"B200_KNN_TC": "1", "B200_KNN_FUSED": "1"},   # sampled threshold, filtering epilogue, knn_select_cand_kernel
-    "simt": {"B200_KNN_TC": "0", "B200_KNN_FUSED": "1"},    # exact float32 FMA scorer, score matrix
+    # tcgen05 scorer: where fused_rank(N, k) > 0 the sampled threshold, filtering epilogue and knn_select_cand_kernel (with
+    # the score matrix as fallback), elsewhere the score matrix and knn_select_kernel
+    "tc": {"B200_KNN_TC": "1"},
+    "simt": {"B200_KNN_TC": "0"},                            # exact float32 FMA scorer, score matrix
 }
 
 
@@ -168,11 +169,10 @@ def run_routes(monkeypatch, q, r, k, metric):
     routes = COSINE_ROUTES if metric == "cosine" else {"l2": {}}
     out = {name: knn_call(monkeypatch, env, refs, qs, k, metric) for name, env in routes.items()}
     for name, (_, _, probe) in out.items():
-        if probe is not None and name != "fused":
+        if probe is not None and name != "tc":
             assert probe[0] == POISON, f"{name}: the fused path ran"
     if metric == "cosine":
-        for name in ("fused", "simt"):
-            assert bits_equal(out[name][0], out["tc"][0]) and bits_equal(out[name][1], out["tc"][1]), f"{name} != tc"
+        assert bits_equal(out["simt"][0], out["tc"][0]) and bits_equal(out["simt"][1], out["tc"][1]), "simt != tc"
     return out
 
 
@@ -234,7 +234,7 @@ def test_route_probe_mirrors_the_workspace_layout():
 
 
 # ------------------------------------------------------------------------------------------------ GPU: every route
-# (Q, N, D, k, bound, pattern, fused fail word expected on the fused route: 0, 1 or None = either)
+# (Q, N, D, k, bound, pattern, fused fail word expected on the "tc" route where the fused path applies: 0, 1 or None = either)
 CASES = [
     (1, 257, 4, 257, 2, "dense", None),               # k = N; scores in [-16, 16]
     (129, 4099, 12, 4097, 3, "dense", None),          # ties straddle rank k and the 4096-rank pass boundary
@@ -259,21 +259,20 @@ def test_every_route_returns_the_exact_list(monkeypatch, metric, nq, n, d, k, bo
     want_s, want_i = oracle(q, r, k, metric)
     for name, (score, idx, probe) in run_routes(monkeypatch, q, r, k, metric).items():
         assert_exact(score, idx, want_s, want_i, name)
-        if name == "fused" and fused_rank(n, k):
+        if name == "tc" and fused_rank(n, k):
             check_fused_probe(probe, k, fail)
 
 
 @pytest.mark.gpu
 def test_c3_shape_every_route_exact(monkeypatch):
     """BASELINE configs[2] shape (5000 x 117000 x 768, k = 2048) on integers |x| <= 15: the fused path (which must have
-    produced the answer), the tensor-core matrix path and the SIMT path agree bit for bit on all queries, and a
-    48-query sample equals the oracle."""
+    produced the answer) and the SIMT path agree bit for bit on all queries, and a 48-query sample equals the oracle."""
     q, r = make_case(3, 5000, 117000, 768, 15, "dense", "cosine")
     out = run_routes(monkeypatch, q, r, 2048, "cosine")
-    check_fused_probe(out["fused"][2], 2048, 0)
+    check_fused_probe(out["tc"][2], 2048, 0)
     sub = np.random.default_rng(4).choice(5000, 48, replace=False)
     want_s, want_i = oracle(q[sub], r, 2048, "cosine")
-    assert_exact(out["fused"][0].cpu()[sub], out["fused"][1].cpu()[sub], want_s, want_i, "c3")
+    assert_exact(out["tc"][0].cpu()[sub], out["tc"][1].cpu()[sub], want_s, want_i, "c3")
 
 
 # ------------------------------------------------------------------------------------------------ GPU: edges
