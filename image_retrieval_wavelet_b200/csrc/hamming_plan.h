@@ -140,7 +140,8 @@ inline int map_plan_init(b200_map_plan *plan, int Q, long long N, long long N_to
             if (sS > 65535) p.select = 0;
             p.sel_S = static_cast<int>(sS), p.sel_seg_len = static_cast<int>(sseg);
             p.sel_maxc = 64;                                      // chunks a list can have
-            int ch = 128;                                         // a warp reads a chunk 128 entries at a time
+            int ch = 128;                                         // a warp reads a chunk 128 entries at a time (and the
+                                                                  // tensor-core append opens at most one chunk per 128 entries)
             while (static_cast<long long>(ch) * p.sel_maxc < sseg) ch <<= 1;
             p.sel_chunk = ch;
             // pool: half a chunk of slack per (query, segment) list + 4k candidates per query + 16 lifted-bound retries

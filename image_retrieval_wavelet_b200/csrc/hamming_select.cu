@@ -222,9 +222,7 @@ __device__ __forceinline__ bool label_rel(const uint32_t *s_labs, int j, const u
 // Measured alternative (round 2, kept out): lanes = rows, loop over queries, one ballot per 32 pairs and a
 // warp-uniform append per non-empty ballot — 13 instructions per 32 pairs to score, but 45 per append with only ~2
 // candidate lanes each (87 % of the ballots are non-empty at 6 % candidates): 1.69 ms against 0.73 ms on c3.
-// MASKED: the append half of the tensor-core form (A') — which rows are within the bound comes from the filter kernel's hit
-// masks; only those rows are scored here (the distance their list entry carries).
-template <int CW, int LW, bool EQ, bool MASKED = false>
+template <int CW, int LW, bool EQ>
 __global__ void __launch_bounds__(128) hamming_select_kernel(const __grid_constant__ SelArgs a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     uint32_t *s_codes = reinterpret_cast<uint32_t *>(smem_raw);
@@ -286,7 +284,7 @@ __global__ void __launch_bounds__(128) hamming_select_kernel(const __grid_consta
             const int i = __ffs(static_cast<int>(m)) - 1;
             m &= m - 1u;
             const int j = row0 + i;
-            const uint32_t d = MASKED ? code_dist<CW>(s_codes, j, qc) : static_cast<uint32_t>(s_d[i]);
+            const uint32_t d = static_cast<uint32_t>(s_d[i]);
             const bool rel = label_rel<LW, EQ>(s_labs, j, ql);
             if ((fill & chmask) == 0u) {
                 uint32_t c;
@@ -316,11 +314,6 @@ __global__ void __launch_bounds__(128) hamming_select_kernel(const __grid_consta
 
     for (int tile0 = seg_begin; tile0 < seg_end; tile0 += a.tile) {
         const int n = a.tile < seg_end - tile0 ? a.tile : seg_end - tile0;
-        uint32_t mw[8];                       // MASKED: this query's hit masks of the tile's (<= 8) 32-row groups, requested ahead of the staging
-        if constexpr (MASKED) {
-#pragma unroll
-            for (int g = 0; g < 8; ++g) mw[g] = 32 * g < n ? a.mask[static_cast<size_t>((tile0 >> 5) + g) * a.Qpad + q] : 0u;
-        }
         {
             const uint4 *gc = reinterpret_cast<const uint4 *>(a.db_codes + static_cast<size_t>(tile0) * CW);
             const uint4 *gl = reinterpret_cast<const uint4 *>(a.db_labels + static_cast<size_t>(tile0) * LW);
@@ -329,11 +322,7 @@ __global__ void __launch_bounds__(128) hamming_select_kernel(const __grid_consta
             for (int i = t; i < nl; i += T) reinterpret_cast<uint4 *>(s_labs)[i] = ldg_stream_u4(gl + i);
         }
         __syncthreads();
-        if constexpr (MASKED) {
-#pragma unroll
-            for (int g = 0; g < 8; ++g)
-                if (mw[g]) append(mw[g], 32 * g, tile0 - seg_begin);
-        } else if (warp_active) {
+        if (warp_active) {
             int j = 0;
             for (; j + 32 <= n; j += 32) {
                 uint32_t m = 0, w[8];
@@ -376,10 +365,10 @@ __global__ void __launch_bounds__(128) hamming_select_kernel(const __grid_consta
 //               lane), tcgen05.ld 32 columns at a time, dot >= B - 2 bound -> one bit; the 32-bit hit mask of every
 //               (32-row group, query) goes to mask[group][Qpad] (a warp stores 128 contiguous bytes).  Persistent over
 //               work units (query tile, segment), query tile fastest: the CTAs running together share a segment's rows in L2.
-//   hamming_select_append_kernel (APPEND)  the SIMT select kernel above with its scoring loop replaced by a read of the
-//               thread's hit masks: only the rows within the bound (4-6 % on c3) are scored again (XOR + POPC from the
-//               staged tile: the distance the list entry carries), label-tested and appended — in row order, to the same
-//               lists, so the rank kernel does not know which form ran.
+//   hamming_select_append_kernel (APPEND)  the hit rows (4-6 % on c3) are scored again (XOR + POPC from the staged tile:
+//               the distance the list entry carries), label-tested and appended — in row order, to the same lists, so the
+//               rank kernel does not know which form ran.  Same grid and tile staging as the SIMT kernel, but a warp
+//               compacts its 32 queries' hits of a 32-row group and each LANE handles one candidate (see the kernel).
 // First form (measured, replaced): the appends in the filter's epilogue — 4 warps per SM (one per TMEM lane quarter) with
 // nothing to hide the latency of the per-candidate chain: 1.42 ms on c3 against 0.64 ms for the SIMT kernel (DESIGN 4.2).
 constexpr int kStcBM = 128, kStcBN = 256, kStcBK = 128;
@@ -574,6 +563,197 @@ __global__ void __launch_bounds__(kStcThreads, 1) hamming_select_tc_kernel(const
         tc_fence_after();
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
     }
+}
+
+// Position (0-based) of the k-th set bit of m, k < popc(m): bisection on the halves, quarters, ... of the word.
+__device__ __forceinline__ uint32_t nth_set_bit(uint32_t m, uint32_t k) {
+    uint32_t p = 0, c = __popc(m & 0xffffu);
+    if (k >= c) k -= c, p = 16;
+    c = __popc((m >> p) & 0xffu);
+    if (k >= c) k -= c, p += 8;
+    c = __popc((m >> p) & 0xfu);
+    if (k >= c) k -= c, p += 4;
+    c = __popc((m >> p) & 0x3u);
+    if (k >= c) k -= c, p += 2;
+    return p + (k >= ((m >> p) & 1u) ? 1u : 0u);
+}
+
+template <int NW>
+__device__ __forceinline__ void lds_words(const uint32_t *p, uint32_t (&x)[NW]) {
+    if constexpr (NW == 2) {
+        const U32x2 v = *reinterpret_cast<const U32x2 *>(p);
+        x[0] = v.x, x[1] = v.y;
+    } else {
+#pragma unroll
+        for (int i = 0; i < NW / 4; ++i) {
+            const U32x4 v = reinterpret_cast<const U32x4 *>(p)[i];
+            x[4 * i] = v.x, x[4 * i + 1] = v.y, x[4 * i + 2] = v.z, x[4 * i + 3] = v.w;
+        }
+    }
+}
+
+// (A') append.  The tile's rows and the CTA's 128 query codes and labels are staged in shared memory, so any lane can
+// score any (query, row) pair.  A warp (32 queries) takes the tile's 8 groups of 32 rows in passes of kAppendGroups
+// groups: lane L counts its query's hits c_L in the pass's masks; a warp scan of c_L gives every hit a slot (lane L's
+// hits are slots off_L .. off_L + c_L - 1, row order); each lane first allocates the one pool chunk its list may need
+// for the pass; then the warp runs ceil(hits / 32) rounds in which lane i takes slot 32 r + i: its owner query
+// (bisection of the offsets by shuffles), its group and row (the owner's running hit counts per group, then the
+// matching set bit of that group's mask), distance, relevance, and its pool position (list fill + rank in row order: the
+// lists come out in row order, and the lanes of one owner store adjacent words).
+// Measured on c3 / c5 (B200 at a 1000 W power limit, bench.py stage times, alternating runs against the parent): the
+// first form of this kernel — the SIMT kernel's loop, a thread walking its own query's hit bits at ~15 of 32 lanes —
+// 0.36-0.38 / 1.58 ms; one group per pass 0.32 / 2.29 ms (c5 has ~8 hits per warp and group: a round with 3/4 of its
+// lanes idle, plus a scan, for every group); four groups per pass 0.28 / 1.36 ms.
+// Four groups add at most 128 entries to a list and a chunk holds at least 128 (hamming_plan.h), so a list needs at most
+// one new chunk per pass.
+constexpr int kAppendGroups = 4;
+constexpr uint32_t kAppendMinChunk = 128;                   // the planner's smallest sel_chunk
+static_assert(32 * kAppendGroups <= kAppendMinChunk, "a pass may need more than one new chunk per list");
+// CTAs per SM the registers must allow: as many as for the SIMT kernel's form of the loop (48 / 56 / 64 registers)
+constexpr int append_min_blocks(int cw, int lw) { return cw + lw >= 8 ? 8 : (cw + lw >= 6 ? 9 : 10); }
+
+template <int CW, int LW, bool EQ>
+__global__ void __launch_bounds__(128, append_min_blocks(CW, LW)) hamming_select_append_kernel(const __grid_constant__ SelArgs a) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    uint32_t *s_codes = reinterpret_cast<uint32_t *>(smem_raw);                   // [tile][2 CW]
+    uint32_t *s_labs = s_codes + static_cast<size_t>(a.tile) * 2 * CW;          // [tile][2 LW]
+    uint32_t *s_qc = s_labs + static_cast<size_t>(a.tile) * 2 * LW;             // [blockDim][2 CW] the CTA's queries
+    uint32_t *s_ql = s_qc + static_cast<size_t>(blockDim.x) * 2 * CW;           // [blockDim][2 LW]
+    uint32_t *s_mask = s_ql + static_cast<size_t>(blockDim.x) * 2 * LW;         // [8][blockDim] the queries' hit masks of the tile's groups
+    const int T = blockDim.x, t = threadIdx.x, lane = t & 31;
+    const int q = blockIdx.x * T + t, seg = blockIdx.y + a.seg0;
+    volatile uint32_t *vflags = a.flags;
+    {
+        // one thread decides for the CTA (another CTA may raise the fallback flag at any moment)
+        bool quit = false;
+        if (t == 0) {
+            quit = vflags[kFlagFallback] != 0u;
+            if (a.round == 0) {
+                const unsigned long long est = *reinterpret_cast<volatile unsigned long long *>(a.flags + kFlagEst);
+                if (est > a.est_cap) {         // the lists would not fit the pool: every CTA sees the same total and leaves
+                    vflags[kFlagFallback] = 1u;
+                    if (a.status) *a.status = 1u;
+                    quit = true;
+                }
+            } else if (vflags[kFlagRetry] == 0u) {
+                quit = true;
+            }
+        }
+        if (__syncthreads_or(quit)) return;
+    }
+    const uint32_t bw = a.bound[q];
+    const bool active = a.round == 0 ? !(bw & kBoundInactive) : (bw & kBoundRetry) != 0;
+    if (!__syncthreads_or(active)) return;
+    {
+        const int qq = q < a.Q ? q : a.Q - 1;
+        const uint32_t *pc = reinterpret_cast<const uint32_t *>(a.q_codes) + static_cast<size_t>(qq) * 2 * CW;
+        const uint32_t *pl = reinterpret_cast<const uint32_t *>(a.q_labels) + static_cast<size_t>(qq) * 2 * LW;
+#pragma unroll
+        for (int i = 0; i < 2 * CW; ++i) s_qc[t * 2 * CW + i] = pc[i];
+#pragma unroll
+        for (int i = 0; i < 2 * LW; ++i) s_ql[t * 2 * LW + i] = pl[i];
+    }                                           // (read after the first tile's barrier)
+    const uint32_t *w_qc = s_qc + (t & ~31) * 2 * CW, *w_ql = s_ql + (t & ~31) * 2 * LW;     // this warp's 32 queries
+    const int seg_begin = seg * a.seg_len;
+    const int seg_end = seg_begin + a.seg_len < a.N ? seg_begin + a.seg_len : a.N;
+    const uint32_t chmask = (1u << a.ch_shift) - 1u;
+    uint32_t fill = 0, first = 0, base = 0;     // this lane's list: entries so far, its first chunk, the pool entry of its current chunk
+    bool dead = false;
+
+    for (int tile0 = seg_begin; tile0 < seg_end; tile0 += a.tile) {
+        const int n = a.tile < seg_end - tile0 ? a.tile : seg_end - tile0;
+        uint32_t mw[8];                         // this query's hit masks of the tile's (<= 8) 32-row groups, requested ahead of the staging
+#pragma unroll
+        for (int g = 0; g < 8; ++g) mw[g] = 32 * g < n ? a.mask[static_cast<size_t>((tile0 >> 5) + g) * a.Qpad + q] : 0u;
+        {
+            const uint4 *gc = reinterpret_cast<const uint4 *>(a.db_codes + static_cast<size_t>(tile0) * CW);
+            const uint4 *gl = reinterpret_cast<const uint4 *>(a.db_labels + static_cast<size_t>(tile0) * LW);
+            const int nc = (n * CW + 1) / 2, nl = (n * LW + 1) / 2;
+            for (int i = t; i < nc; i += T) reinterpret_cast<uint4 *>(s_codes)[i] = ldg_stream_u4(gc + i);
+            for (int i = t; i < nl; i += T) reinterpret_cast<uint4 *>(s_labs)[i] = ldg_stream_u4(gl + i);
+        }
+#pragma unroll
+        for (int g = 0; g < 8; ++g) s_mask[g * T + t] = mw[g];      // (out of the registers of the loop below)
+        __syncthreads();
+#pragma unroll 1
+        for (int g0 = 0; g0 < 8; g0 += kAppendGroups) {
+            // this lane's hits in the pass's groups: c in all, byte b of cum: in groups g0 .. g0 + b
+            uint32_t c = 0, cum = 0;
+#pragma unroll
+            for (int b = 0; b < kAppendGroups; ++b) {
+                c += __popc(s_mask[(g0 + b) * T + t]);
+                if (b < kAppendGroups - 1) cum |= c << (8 * b);
+            }
+            uint32_t incl = c;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const uint32_t v = __shfl_up_sync(0xffffffffu, incl, o);
+                if (lane >= o) incl += v;
+            }
+            const uint32_t hits = __shfl_sync(0xffffffffu, incl, 31);
+            if (hits == 0u) continue;
+            // the list's next c (<= 128) entries: the first `room` fill its current chunk, the rest open one new chunk
+            const uint32_t room = (0u - fill) & chmask;
+            uint32_t nbase = 0;
+            if (c > room && !dead) {
+                uint32_t ch;
+                if (a.nsub > 1) {
+                    const uint32_t sub = (static_cast<uint32_t>(seg) * gridDim.x + blockIdx.x) & (kSubPools - 1);
+                    const uint32_t local = atomicAdd(a.flags + kFlagSubCursor + sub, 1u);
+                    ch = local < a.sub_chunks ? sub * a.sub_chunks + local : 0xffffffffu;
+                } else {
+                    ch = atomicAdd(a.flags + kFlagCursor, 1u);
+                }
+                if (ch >= a.pool_chunks) {
+                    dead = true;
+                    vflags[kFlagFallback] = 1u;
+                    if (a.status) *a.status = 1u;
+                } else {
+                    const uint32_t at = fill + room;
+                    if (at == 0u)
+                        first = ch;
+                    else
+                        a.table[(static_cast<size_t>(q) * a.S + seg) * a.maxc + (at >> a.ch_shift)] = ch;
+                    nbase = ch << a.ch_shift;
+                }
+            }
+            // entry i (< c) of this lane's pass goes to old_at + i (i < room) or new_at + i; key: slot offset | dead | room
+            // (room < sel_chunk <= 0x8000: checked by the launcher)
+            const uint32_t old_at = base + (fill & chmask), new_at = nbase - room;
+            const uint32_t key = ((incl - c) << 16) | (dead ? 0x8000u : 0u) | room;
+            if (c > room && !dead) base = nbase;
+            fill += c;
+            for (uint32_t s0 = 0; s0 < hits; s0 += 32u) {
+                const uint32_t s = s0 + static_cast<uint32_t>(lane);
+                int o = 0;                      // owner: the last lane whose first slot is <= s
+#pragma unroll
+                for (int b = 16; b > 0; b >>= 1)
+                    if ((__shfl_sync(0xffffffffu, key, o + b) >> 16) <= s) o += b;
+                const uint32_t ko = __shfl_sync(0xffffffffu, key, o), co = __shfl_sync(0xffffffffu, cum, o);
+                const uint32_t oa = __shfl_sync(0xffffffffu, old_at, o), na = __shfl_sync(0xffffffffu, new_at, o);
+                if (s < hits && !(ko & 0x8000u)) {
+                    const uint32_t i = s - (ko >> 16);
+                    uint32_t gb = 0, below = 0;     // the group of the owner's i-th hit, and the owner's hits in the groups before it
+#pragma unroll
+                    for (int b = 0; b < kAppendGroups - 1; ++b) {
+                        const uint32_t v = (co >> (8 * b)) & 0xffu;
+                        if (i >= v) gb = b + 1, below = v;
+                    }
+                    const int g = g0 + static_cast<int>(gb);
+                    const int j = 32 * g + static_cast<int>(nth_set_bit(s_mask[g * T + (t & ~31) + o], i - below));
+                    uint32_t qc[2 * CW], ql[2 * LW];
+                    lds_words<2 * CW>(w_qc + o * 2 * CW, qc);
+                    lds_words<2 * LW>(w_ql + o * 2 * LW, ql);
+                    const uint32_t d = code_dist<CW>(s_codes, j, qc);
+                    const bool rel = label_rel<LW, EQ>(s_labs, j, ql);
+                    const uint32_t pos = i < (ko & 0x7fffu) ? oa + i : na + i;
+                    a.pool[pos] = static_cast<uint32_t>(tile0 - seg_begin + j) | (d << 16) | (static_cast<uint32_t>(rel) << 24);
+                }
+            }
+        }
+        __syncthreads();
+    }
+    if (active) a.head[static_cast<size_t>(q) * a.S + seg] = U32x2{dead ? 0u : fill, first};
 }
 
 // ------------------------------------------------------------------------------------------------ (B) rank
@@ -953,20 +1133,20 @@ static sel_fn pick_sel(int cw, int lw, bool eq) {
     return nullptr;
 }
 template <int CW>
-static sel_fn pick_app2(int lw, bool eq) {
-    if (eq) return hamming_select_kernel<CW, 1, true, true>;
+static sel_fn pick_append2(int lw, bool eq) {
+    if (eq) return hamming_select_append_kernel<CW, 1, true>;
     switch (lw) {
-        case 1: return hamming_select_kernel<CW, 1, false, true>;
-        case 2: return hamming_select_kernel<CW, 2, false, true>;
-        case 4: return hamming_select_kernel<CW, 4, false, true>;
+        case 1: return hamming_select_append_kernel<CW, 1, false>;
+        case 2: return hamming_select_append_kernel<CW, 2, false>;
+        case 4: return hamming_select_append_kernel<CW, 4, false>;
     }
     return nullptr;
 }
-static sel_fn pick_app(int cw, int lw, bool eq) {        // the MASKED (append-only) form
+static sel_fn pick_append(int cw, int lw, bool eq) {
     switch (cw) {
-        case 1: return pick_app2<1>(lw, eq);
-        case 2: return pick_app2<2>(lw, eq);
-        case 4: return pick_app2<4>(lw, eq);
+        case 1: return pick_append2<1>(lw, eq);
+        case 2: return pick_append2<2>(lw, eq);
+        case 4: return pick_append2<4>(lw, eq);
     }
     return nullptr;
 }
@@ -1076,8 +1256,10 @@ int select_finish(const b200_map_plan *p, const uint64_t *qc, const uint64_t *ql
     // workspace and the caller has not run round 0 already; the SIMT kernel when the driver cannot encode tensor maps
     const int Bp = (p->B + kStcBK - 1) / kStcBK * kStcBK;
     stc_fn tf = hamming_select_tc_kernel;
-    sel_fn af = pick_app(cw, p->LW, p->label_mode == B200_LABELS_EQUAL);
+    sel_fn af = pick_append(cw, p->LW, p->label_mode == B200_LABELS_EQUAL);
     bool use_tc = !round0_selected && plan_select_tc(*p) && encode_tiled_fn() != nullptr;
+    // the append kernel packs a list's room in its current chunk into 15 bits and opens at most one chunk per pass
+    if (use_tc && (p->sel_chunk < static_cast<int>(kAppendMinChunk) || p->sel_chunk > 0x8000)) return B200_ERR_UNSUPPORTED;
     StcMaps maps;
     if (use_tc) {
         unsigned char *db8 = reinterpret_cast<unsigned char *>((reinterpret_cast<uintptr_t>(w + p->off_smp_codes) + 1023) & ~static_cast<uintptr_t>(1023));
@@ -1098,6 +1280,7 @@ int select_finish(const b200_map_plan *p, const uint64_t *qc, const uint64_t *ql
         }
     }
     const size_t smem = static_cast<size_t>(p->tile) * (cw + p->LW) * 8 + static_cast<size_t>(32) * p->sel_T;      // tile + parked distances
+    const size_t asmem = static_cast<size_t>(p->tile + p->sel_T) * (cw + p->LW) * 8 + static_cast<size_t>(32) * p->sel_T;      // tile + queries + masks
     const bool emit = rank_idx != nullptr || rank_dist != nullptr;
     sel_fn rf = emit ? hamming_select_rank_kernel<true> : hamming_select_rank_kernel<false>;
     const size_t rsmem = rank_smem_bytes(p->bins, a.k, a.stage_cap);
@@ -1112,8 +1295,8 @@ int select_finish(const b200_map_plan *p, const uint64_t *qc, const uint64_t *ql
             tf<<<units < sms ? units : sms, kStcThreads, kStcSmemBytes, st>>>(maps, a, p->B, Bp / kStcBK);
             B200_LAUNCH_CHECK("hamming_select_tc_kernel");
             stage_mark(round ? "filter_round1" : "filter", st);
-            af<<<dim3(p->Qpad / p->sel_T, p->sel_S), p->sel_T, smem, st>>>(a);
-            B200_LAUNCH_CHECK("hamming_select_kernel (append)");
+            af<<<dim3(p->Qpad / p->sel_T, p->sel_S), p->sel_T, asmem, st>>>(a);
+            B200_LAUNCH_CHECK("hamming_select_append_kernel");
         } else {
             fn<<<dim3(p->Qpad / p->sel_T, p->sel_S), p->sel_T, smem, st>>>(a);
             B200_LAUNCH_CHECK("hamming_select_kernel");

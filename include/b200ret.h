@@ -193,8 +193,8 @@ typedef struct b200_map_plan {
      * The one pass has two forms, and the plan alone decides which.  Tensor-core form (when the queries come in groups of
      * 128, the hit masks fit 4 GB and the e4m3 codes 8 GB): the +-1 codes are expanded to e4m3 bytes and a tcgen05 fp8 GEMM
      * (dot = B - 2 distance, exact) writes one hit bit per (row, query) — off_smp_codes then points at the e4m3 copies and
-     * the masks, otherwise off_smp_codes == workspace_bytes — and a SIMT kernel scores only the hit rows again and appends
-     * them.  SIMT form: XOR + POPC of every pair in the same kernel that appends. */
+     * the masks, otherwise off_smp_codes == workspace_bytes — and an append kernel, one lane per hit, scores only the hit
+     * rows again and appends them.  SIMT form: XOR + POPC of every pair in the same kernel that appends. */
     int select, sel_stride, sel_S, sel_seg_len, sel_chunk, sel_maxc, smp_S, smp_seg_len, sel_T;
     long long smp_rows, sel_pool_chunks;
     size_t off_sel_flags, off_sel_bound, off_sel_count, off_sel_table, off_sel_pool, off_smp_codes, off_smp_hist;
