@@ -7,6 +7,10 @@
 //   b200_resize_crop_u8 <- that eval transform, Resize(size) -> CenterCrop(crop) of torchvision on every PIL image of a
 //                      batch, for a ragged batch of decoded HWC images in one launch: only the crop window of each resized
 //                      image is computed (resize_crop_kernel below).
+//   b200_resize_random_crop_u8 <- the training transform, Resize(size) -> RandomResizedCrop(crop) -> RandomHorizontalFlip of
+//                      torchvision on every PIL image of a batch, with the boxes and flips drawn by the caller: two launches
+//                      of resize_crop_kernel, the box of each resized image (a window of the first resize), then a full
+//                      resize of that box to the crop size stored mirrored where the flip is drawn.
 //
 // The arithmetic is Pillow's (third-party, pinned `pillow==8.2.0` in requirements.txt:5; src/libImaging/Resample.c, the
 // 8-bit path, unchanged through the 12.x release installed here), restated:
@@ -333,11 +337,13 @@ static ResizeLayout resize_layout(long long planes, int H, int W, int Hout, int 
     return l;
 }
 
-// ---- resize + center crop of a ragged batch (torchvision Resize(size) -> CenterCrop(crop) on PIL images).  A crop of a
-// resize is the resize evaluated inside the crop window only: output (y, x) of image i is resized sample
+// ---- resize + crop of a ragged batch: torchvision Resize(size) -> CenterCrop(crop) (b200_resize_crop_u8) and the two
+// resamplings of Resize(size) -> RandomResizedCrop(crop) -> RandomHorizontalFlip (b200_resize_random_crop_u8) on PIL
+// images.  A crop of a resize is the resize evaluated inside the crop window: output (y, x) of image i is resized sample
 // (top_i + y, left_i + x), whose window and weights are those rows of the full-axis tables.  So the host builds just the
-// Hc (Wc) table rows of each axis, shared by every image with the same (input size, resized size, crop origin), and one
-// launch covers the batch: a regular [n][C][Hc][Wc] output, one CTA per kRcTH x kRcTW tile of one channel.  The CTA walks its tile in sub-blocks of sub_h x sub_w output samples, chosen per
+// Hc_i (Wc_i) table rows of each axis, shared by every image with the same (input size, resized size, crop origin, crop
+// size), and one launch covers the batch: image i's planar [C][Hc_i][Wc_i] output at its own byte offset, one CTA per
+// kRcTH x kRcTW tile of one channel.  The CTA walks its tile in sub-blocks of sub_h x sub_w output samples, chosen per
 // image on the host as the one that stages the fewest source bytes per output sample within kRcSmemBudget: one sub-block
 // (the whole tile) for reductions up to ~2x, tall narrow ones for large photos (a short sub-block would recompute the
 // horizontal pass of its vertical window for every few output rows).  Per sub-block: stage channel c of the source window in
@@ -345,18 +351,22 @@ static ResizeLayout resize_layout(long long planes, int H, int W, int Hout, int 
 // shared uint8 intermediate, vertical pass, store.  The grid is one-dimensional: images in descending order of staged
 // bytes (a large photo's tiles start in the first wave instead of trailing behind the small images), then tiles, then
 // channels, so the C CTAs of a tile are adjacent and the interleaved source words they all load come from L2 after the
-// first.
+// first.  Images may have different output sizes, so each descriptor records its first CTA and a CTA finds its descriptor
+// by a binary search over them.  With `flip` set the vertical pass stores output column x at Wc - 1 - x
+// (RandomHorizontalFlip): the output is mirrored, never the source, as Pillow's weight tables need not be bit-symmetric.
 constexpr int kRcTH = 32, kRcTW = 128, kRcThreads = 256;
 constexpr int kRcSmemBudget = 32 * 1024;
 
 struct CropDesc {
     long long in_off;         // byte offset of the image in `in`
+    long long out_off;        // byte offset of the image's planar [C][Hc][Wc] output in `out`
+    int cta0;                 // first CTA of the image (descriptors in launch order: ascending)
     int W;                    // input width (row pitch W * C bytes)
+    int Hc, Wc, flip;         // output size; flip: output column x is stored at Wc - 1 - x
     int hb, hk, ksh;          // tables (int index into the table block): bounds / weights of crop column 0, taps
     int vb, vk, ksv;          // the same for crop row 0
     int sub_h, sub_w;         // sub-block of the tile (powers of two dividing kRcTH / kRcTW; sub_w >= 4)
     int max_rows, stride;     // staged source rows / bytes per staged row, upper bounds over the image's sub-blocks
-    int img;                  // output image
 };
 
 __host__ __device__ inline size_t crop_smem_bytes(int sub_h, int sub_w, int ksh, int ksv, int max_rows, int stride) {
@@ -364,16 +374,40 @@ __host__ __device__ inline size_t crop_smem_bytes(int sub_h, int sub_w, int ksh,
            static_cast<size_t>(max_rows) * (stride + sub_w);
 }
 
-template <int C>
+// kGeneral = false: every crop of the launch is Hc_all x Wc_all and none is mirrored (every eval launch).  That form is
+// the launch-argument kernel the eval path always had: the descriptor search, the shared-memory stash of the store
+// operands and the mirrored stores are compiled out, so the eval transform keeps its speed.
+template <int C, bool kGeneral>
 __global__ void __launch_bounds__(kRcThreads, 4) resize_crop_kernel(const uint8_t *__restrict__ in, uint8_t *__restrict__ out,
                                                                  const CropDesc *__restrict__ descs, const int *__restrict__ tab,
-                                                                 int Hc, int Wc, int tiles_x, int tiles_y) {
+                                                                 int n, int Hc_all, int Wc_all) {
     extern __shared__ __align__(16) unsigned char rc_smem[];
-    const unsigned cta = blockIdx.x, t = cta / C, tt = t / tiles_x;
-    const int c = static_cast<int>(cta - t * C), bx = static_cast<int>(t - tt * tiles_x);
-    const int by = static_cast<int>(tt % tiles_y), rank = static_cast<int>(tt / tiles_y);
+    const int cta = static_cast<int>(blockIdx.x);
+    int Hc = Hc_all, Wc = Wc_all, rank, c, bx, by;
+    if (!kGeneral || Hc_all > 0) {
+        // one crop size for the launch: the tile and channel follow from the CTA index and the launch arguments alone,
+        // without waiting for the descriptor
+        const int tiles_x = (Wc + kRcTW - 1) / kRcTW, tiles_y = (Hc + kRcTH - 1) / kRcTH;
+        const unsigned t = static_cast<unsigned>(cta) / C, tt = t / tiles_x;
+        c = static_cast<int>(cta - t * C), bx = static_cast<int>(t - tt * tiles_x);
+        by = static_cast<int>(tt % tiles_y), rank = static_cast<int>(tt / tiles_y);
+    } else {
+        // the last descriptor whose first CTA is <= cta lies in [lo, lo + span): each warp narrows it 32-fold per step
+        // (its lanes probe 32 evenly spaced descriptors at once), two dependent loads for up to 1024 descriptors
+        const int lane = static_cast<int>(threadIdx.x) & 31;
+        int lo = 0, span = n;
+        while (span > 1) {
+            const int step = (span + 31) >> 5, probe = lo + lane * step;
+            const unsigned le = __ballot_sync(0xffffffffu, probe < lo + span && __ldg(&descs[probe].cta0) <= cta);
+            const int k = 31 - __clz(le);                                // lane 0 holds: descs[lo].cta0 <= cta
+            lo += k * step, span = min(step, span - k * step);
+        }
+        rank = lo, Hc = descs[lo].Hc, Wc = descs[lo].Wc;
+        const int tiles_x = (Wc + kRcTW - 1) / kRcTW;
+        const unsigned local = static_cast<unsigned>(cta - descs[lo].cta0), t = local / C, tt = t / tiles_x;
+        c = static_cast<int>(local - t * C), bx = static_cast<int>(t - tt * tiles_x), by = static_cast<int>(tt);
+    }
     const CropDesc &d = descs[rank];
-    const size_t plane = static_cast<size_t>(d.img) * C + c;
     const int2 *hb = reinterpret_cast<const int2 *>(tab + d.hb), *vb = reinterpret_cast<const int2 *>(tab + d.vb);
     const int *hk = tab + d.hk, *vk = tab + d.vk;
     const int sh = d.sub_h, sw = d.sub_w, ksh = d.ksh, ksv = d.ksv, stride = d.stride, max_rows = d.max_rows;
@@ -385,6 +419,12 @@ __global__ void __launch_bounds__(kRcThreads, 4) resize_crop_kernel(const uint8_
     uint8_t *s_in = reinterpret_cast<uint8_t *>(s_vk + sh * ksv);        // [max_rows][stride] channel c of the window
     uint8_t *s_tmp = s_in + max_rows * stride;                           // [max_rows][sw] horizontal pass
     const int tid = static_cast<int>(threadIdx.x), lane = tid & 31, warp = tid >> 5;
+    // general form: what only the stores need waits in shared memory, not in registers: the kernel is at its 64-register
+    // cap (4 CTAs per SM), and values live across the staging and horizontal loops slow them down
+    __shared__ uint8_t *s_out;
+    __shared__ int s_wc, s_flip;
+    if (kGeneral && tid == 0) s_out = out + d.out_off + static_cast<size_t>(c) * Hc * Wc, s_wc = Wc, s_flip = d.flip;
+    const size_t plane_off = kGeneral ? 0 : static_cast<size_t>(d.out_off) + static_cast<size_t>(c) * Hc * Wc;
     const int x0 = bx * kRcTW, y0 = by * kRcTH;
     const int nx = Wc - x0 < kRcTW ? Wc - x0 : kRcTW, ny = Hc - y0 < kRcTH ? Hc - y0 : kRcTH;
     const int sw_log = __ffs(sw) - 1, ng = sw >> 2, ng_log = sw_log - 2;
@@ -445,6 +485,9 @@ __global__ void __launch_bounds__(kRcThreads, 4) resize_crop_kernel(const uint8_
             {
                 const int g4 = 4 * (tid & (ng - 1));
                 if (g4 < mw) {
+                    uint8_t *const out_plane = kGeneral ? s_out : out + plane_off;
+                    const int wo = kGeneral ? s_wc : Wc, flip = kGeneral ? s_flip : 0;
+                    const int xo = xa + g4, xs = flip ? wo - 4 - xo : xo;       // first column / lowest address of the 4
                     for (int yy = tid >> ng_log; yy < mh; yy += kRcThreads >> ng_log) {
                         const int2 b = s_vb[yy];
                         const int *k = s_vk + yy * ksv;
@@ -458,12 +501,13 @@ __global__ void __launch_bounds__(kRcThreads, 4) resize_crop_kernel(const uint8_
                             acc[0] += static_cast<int>(v & 0xffu) * w, acc[1] += static_cast<int>((v >> 8) & 0xffu) * w;
                             acc[2] += static_cast<int>((v >> 16) & 0xffu) * w, acc[3] += static_cast<int>(v >> 24) * w;
                         }
-                        uint8_t *dst = out + (plane * Hc + ya + yy) * Wc + xa + g4;
-                        if (g4 + 3 < mw && (reinterpret_cast<uintptr_t>(dst) & 3) == 0) {
-                            *reinterpret_cast<uint32_t *>(dst) =
-                                resize_clip8(acc[0]) | (resize_clip8(acc[1]) << 8) | (resize_clip8(acc[2]) << 16) | (resize_clip8(acc[3]) << 24);
+                        const uint32_t v = resize_clip8(acc[0]) | (resize_clip8(acc[1]) << 8) | (resize_clip8(acc[2]) << 16) |
+                                           (resize_clip8(acc[3]) << 24);
+                        uint8_t *row = out_plane + static_cast<size_t>(ya + yy) * wo;
+                        if (g4 + 3 < mw && (reinterpret_cast<uintptr_t>(row + xs) & 3) == 0) {
+                            *reinterpret_cast<uint32_t *>(row + xs) = flip ? __byte_perm(v, 0, 0x0123) : v;
                         } else {
-                            for (int e = 0; e < 4 && g4 + e < mw; ++e) dst[e] = static_cast<uint8_t>(resize_clip8(acc[e]));
+                            for (int e = 0; e < 4 && g4 + e < mw; ++e) row[flip ? wo - 1 - xo - e : xo + e] = static_cast<uint8_t>(v >> (8 * e));
                         }
                     }
                 }
@@ -472,13 +516,13 @@ __global__ void __launch_bounds__(kRcThreads, 4) resize_crop_kernel(const uint8_
     }
 }
 
-using resize_crop_fn = void (*)(const uint8_t *, uint8_t *, const CropDesc *, const int *, int, int, int, int);
-static resize_crop_fn resize_pick_crop(int C) {
+using resize_crop_fn = void (*)(const uint8_t *, uint8_t *, const CropDesc *, const int *, int, int, int);
+static resize_crop_fn resize_pick_crop(int C, bool general) {
     switch (C) {
-        case 1: return resize_crop_kernel<1>;
-        case 2: return resize_crop_kernel<2>;
-        case 3: return resize_crop_kernel<3>;
-        default: return resize_crop_kernel<4>;
+        case 1: return general ? resize_crop_kernel<1, true> : resize_crop_kernel<1, false>;
+        case 2: return general ? resize_crop_kernel<2, true> : resize_crop_kernel<2, false>;
+        case 3: return general ? resize_crop_kernel<3, true> : resize_crop_kernel<3, false>;
+        default: return general ? resize_crop_kernel<4, true> : resize_crop_kernel<4, false>;
     }
 }
 
@@ -489,8 +533,30 @@ struct CropAxisKey {
 };
 static int crop_ksize(int in_size, int out_size, int filter) { return in_size == out_size ? 1 : resize_ksize(in_size, out_size, filter); }
 
-// Host-side layout of a call: the descriptor block, then one table block per distinct axis key (bounds, then weights;
-// every table starts on a 16-byte boundary).  geom rows: H, W, RH, RW, top, left.
+// One output image of a launch: the source image (H x W, at byte in_off of the input), its resized size, the crop window
+// (top, left, Hc, Wc) inside the resized image, and where its planar output goes.
+struct CropGeom {
+    int H, W, RH, RW, top, left, Hc, Wc, flip;
+    long long in_off, out_off;
+};
+
+// B200_OK, or the error the entry points return for this image (no CUDA call).
+static int crop_check_geom(const CropGeom &g, int C, int filter) {
+    if (g.H < 1 || g.W < 1 || g.RH < 1 || g.RW < 1 || g.top < 0 || g.left < 0 || g.Hc < 1 || g.Wc < 1) return B200_ERR_INVALID_ARG;
+    if (g.top > g.RH - g.Hc || g.left > g.RW - g.Wc) return B200_ERR_INVALID_ARG;      // the crop must lie inside the resized image
+    if (static_cast<long long>(g.W) * C > 0x7fffffffLL) return B200_ERR_UNSUPPORTED;
+    if (crop_ksize(g.W, g.RW, filter) > kResizeMaxTaps || crop_ksize(g.H, g.RH, filter) > kResizeMaxTaps) return B200_ERR_UNSUPPORTED;
+    return B200_OK;
+}
+
+static long long crop_ctas(const std::vector<CropGeom> &g, int C) {
+    long long ctas = 0;
+    for (const CropGeom &e : g) ctas += static_cast<long long>(C) * ceil_div(e.Wc, kRcTW) * ceil_div(e.Hc, kRcTH);
+    return ctas;
+}
+
+// Host-side layout of one launch: the descriptor block, then one table block per distinct axis key (bounds, then weights;
+// every table starts on a 16-byte boundary).
 struct CropLayout {
     std::vector<CropAxisKey> keys;
     std::vector<int> key_off, key_ks;   // int offset of each key's bounds in the table block, its window length
@@ -511,7 +577,110 @@ static int crop_find_or_add(CropLayout &l, std::map<std::tuple<int, int, int, in
     return static_cast<int>(l.keys.size()) - 1;
 }
 
-// Host-side argument check (no CUDA call): B200_OK, or the error the entry points return.
+static CropLayout crop_layout(const std::vector<CropGeom> &g, int filter) {
+    CropLayout l;
+    std::map<std::tuple<int, int, int, int>, int> seen;
+    const size_t n = g.size();
+    l.h_key.resize(n), l.v_key.resize(n);
+    for (size_t i = 0; i < n; ++i) {
+        l.h_key[i] = crop_find_or_add(l, seen, CropAxisKey{g[i].W, g[i].RW, g[i].left, g[i].Wc}, filter);
+        l.v_key[i] = crop_find_or_add(l, seen, CropAxisKey{g[i].H, g[i].RH, g[i].top, g[i].Hc}, filter);
+    }
+    l.off_tab = round_up<size_t>(n * sizeof(CropDesc), 256);
+    l.bytes = l.off_tab + l.table_ints * 4;
+    return l;
+}
+
+// The tables, staging plans and descriptors of one launch, written to `stage` (l.bytes, zeroed): descriptors in launch
+// order, the images that stage the most source bytes first.  Returns the dynamic shared memory the launch needs, or 0
+// when no sub-block of some image fits kRcSmemBudget.
+static size_t crop_stage(const std::vector<CropGeom> &g, int C, int filter, const CropLayout &l, unsigned char *stage) {
+    const int n = static_cast<int>(g.size());
+    int *tab = reinterpret_cast<int *>(stage + l.off_tab);
+    std::vector<std::vector<int>> key_bounds(l.keys.size());
+    for (size_t k = 0; k < l.keys.size(); ++k) {
+        const CropAxisKey &key = l.keys[k];
+        std::vector<int> kk;
+        if (key.in_size == key.out_size) {
+            key_bounds[k].resize(static_cast<size_t>(key.count) * 2);
+            kk.assign(key.count, 1 << kResizePrecisionBits);
+            for (int i = 0; i < key.count; ++i) key_bounds[k][2 * i] = key.first + i, key_bounds[k][2 * i + 1] = 1;
+        } else {
+            resize_coeffs(key.in_size, key.out_size, filter, l.key_ks[k], key_bounds[k], kk, key.first, key.count);
+        }
+        std::memcpy(tab + l.key_off[k], key_bounds[k].data(), key_bounds[k].size() * 4);
+        std::memcpy(tab + l.key_off[k] + round_up<size_t>(static_cast<size_t>(key.count) * 2, 4), kk.data(), kk.size() * 4);
+    }
+    // staging plan per (horizontal, vertical) key pair: the sub-block that fits kRcSmemBudget and stages the fewest source
+    // bytes per output sample (then the larger one)
+    std::map<std::pair<int, int>, std::pair<CropDesc, double>> plans;
+    std::vector<std::pair<double, int>> order(n);                       // (-staged bytes of the image, image)
+    std::vector<CropDesc> by_image(n);
+    size_t smem = 0;
+    for (int i = 0; i < n; ++i) {
+        const int hk = l.h_key[i], vk = l.v_key[i], Hc = g[i].Hc, Wc = g[i].Wc;
+        auto it = plans.find(std::make_pair(hk, vk));
+        if (it == plans.end()) {
+            CropDesc p{};
+            p.hb = l.key_off[hk], p.hk = l.key_off[hk] + static_cast<int>(round_up<size_t>(static_cast<size_t>(Wc) * 2, 4));
+            p.vb = l.key_off[vk], p.vk = l.key_off[vk] + static_cast<int>(round_up<size_t>(static_cast<size_t>(Hc) * 2, 4));
+            p.ksh = l.key_ks[hk], p.ksv = l.key_ks[vk];
+            double best = 0.0;
+            for (int sw = kRcTW; sw >= 4; sw /= 2) {
+                const int stride = round_up(resize_max_window(key_bounds[hk], Wc, sw), 4);
+                for (int sh = kRcTH; sh >= 1; sh /= 2) {
+                    const int rows = resize_max_window(key_bounds[vk], Hc, sh);
+                    if (crop_smem_bytes(sh, sw, p.ksh, p.ksv, rows, stride) > static_cast<size_t>(kRcSmemBudget)) continue;
+                    const double per_sample = static_cast<double>(rows) * stride / (static_cast<double>(sh) * sw);
+                    if (best == 0.0 || per_sample < best)
+                        best = per_sample, p.sub_h = sh, p.sub_w = sw, p.max_rows = rows, p.stride = stride;
+                }
+            }
+            if (best == 0.0) return 0;
+            it = plans.emplace(std::make_pair(hk, vk), std::make_pair(p, best)).first;
+        }
+        CropDesc d = it->second.first;
+        d.in_off = g[i].in_off, d.out_off = g[i].out_off, d.W = g[i].W, d.Hc = Hc, d.Wc = Wc, d.flip = g[i].flip;
+        by_image[i] = d;
+        order[i] = std::make_pair(-it->second.second * Hc * Wc, i);
+        const size_t need = crop_smem_bytes(d.sub_h, d.sub_w, d.ksh, d.ksv, d.max_rows, d.stride);
+        if (need > smem) smem = need;
+    }
+    std::stable_sort(order.begin(), order.end());
+    CropDesc *descs = reinterpret_cast<CropDesc *>(stage);
+    int cta = 0;
+    for (int r = 0; r < n; ++r) {
+        CropDesc &d = descs[r];
+        d = by_image[order[r].second];
+        d.cta0 = cta;
+        cta += C * ceil_div(d.Wc, kRcTW) * ceil_div(d.Hc, kRcTH);
+    }
+    return smem;
+}
+
+// One launch over descriptors and tables already in device memory at `block` (descriptors at 0, tables at off_tab).  When
+// all crops of the launch have one size, it goes to the kernel as launch arguments; the general form of the kernel runs
+// unless that holds and no crop is mirrored.
+static int crop_launch(int C, const uint8_t *in, uint8_t *out, const unsigned char *block, size_t off_tab,
+                       const std::vector<CropGeom> &g, long long ctas, size_t smem, cudaStream_t st) {
+    const int n = static_cast<int>(g.size());
+    int Hc = g[0].Hc, Wc = g[0].Wc;
+    bool flip = false;
+    for (const CropGeom &e : g) {
+        if (e.Hc != Hc || e.Wc != Wc) Hc = Wc = 0;
+        flip = flip || e.flip;
+    }
+    resize_crop_fn fn = resize_pick_crop(C, Hc == 0 || flip);
+    B200_CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void *>(fn), cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       static_cast<int>(smem)));
+    fn<<<static_cast<unsigned>(ctas), kRcThreads, smem, st>>>(in, out, reinterpret_cast<const CropDesc *>(block),
+                                                              reinterpret_cast<const int *>(block + off_tab), n,
+                                                              Hc, Wc);
+    B200_LAUNCH_CHECK("resize_crop_kernel");
+    return B200_OK;
+}
+
+// ---- b200_resize_crop_u8: geom rows H, W, RH, RW, top, left; every crop Hc x Wc, none mirrored.
 static int crop_check(int n, const int *geom, int C, int Hc, int Wc, int filter) {
     if (n < 0 || C < 1 || C > 4 || Hc < 1 || Wc < 1) return B200_ERR_INVALID_ARG;
     if (filter != B200_RESIZE_BICUBIC && filter != B200_RESIZE_BILINEAR) return B200_ERR_INVALID_ARG;
@@ -519,27 +688,63 @@ static int crop_check(int n, const int *geom, int C, int Hc, int Wc, int filter)
     if (static_cast<long long>(n) * C > 0x7fffffffLL) return B200_ERR_UNSUPPORTED;
     for (int i = 0; i < n; ++i) {
         const int *g = geom + 6 * i;
-        const int H = g[0], W = g[1], RH = g[2], RW = g[3], top = g[4], left = g[5];
-        if (H < 1 || W < 1 || RH < 1 || RW < 1 || top < 0 || left < 0) return B200_ERR_INVALID_ARG;
-        if (top > RH - Hc || left > RW - Wc) return B200_ERR_INVALID_ARG;          // the crop must lie inside the resized image
-        if (static_cast<long long>(W) * C > 0x7fffffffLL) return B200_ERR_UNSUPPORTED;
-        if (crop_ksize(W, RW, filter) > kResizeMaxTaps || crop_ksize(H, RH, filter) > kResizeMaxTaps) return B200_ERR_UNSUPPORTED;
+        const int rc = crop_check_geom(CropGeom{g[0], g[1], g[2], g[3], g[4], g[5], Hc, Wc, 0, 0, 0}, C, filter);
+        if (rc != B200_OK) return rc;
     }
     return B200_OK;
 }
 
-static CropLayout crop_layout(int n, const int *geom, int Hc, int Wc, int filter) {
-    CropLayout l;
-    std::map<std::tuple<int, int, int, int>, int> seen;
-    l.h_key.resize(n), l.v_key.resize(n);
+static std::vector<CropGeom> crop_geoms(int n, const int *geom, const long long *offsets, int C, int Hc, int Wc) {
+    std::vector<CropGeom> g(n);
     for (int i = 0; i < n; ++i) {
-        const int *g = geom + 6 * i;
-        l.h_key[i] = crop_find_or_add(l, seen, CropAxisKey{g[1], g[3], g[5], Wc}, filter);
-        l.v_key[i] = crop_find_or_add(l, seen, CropAxisKey{g[0], g[2], g[4], Hc}, filter);
+        const int *r = geom + 6 * i;
+        g[i] = CropGeom{r[0], r[1], r[2], r[3], r[4], r[5], Hc, Wc, 0, offsets ? offsets[i] : 0,
+                        static_cast<long long>(i) * C * Hc * Wc};
     }
-    l.off_tab = round_up<size_t>(static_cast<size_t>(n) * sizeof(CropDesc), 256);
-    l.bytes = l.off_tab + l.table_ints * 4;
-    return l;
+    return g;
+}
+
+// ---- b200_resize_random_crop_u8: geom rows H, W, RH, RW, top, left, h, w, flip.  Launch 1 computes each image's window
+// (top, left, h, w) of the first resize into a planar [C][h][w] uint8 intermediate (each image 4-byte aligned); launch 2
+// resizes every intermediate plane in full to Ho x Wo as a one-channel image, mirrored when flip is set.
+static int random_crop_check(int n, const int *geom, int C, int Ho, int Wo, int filter) {
+    if (n < 0 || C < 1 || C > 4 || Ho < 1 || Wo < 1) return B200_ERR_INVALID_ARG;
+    if (filter != B200_RESIZE_BICUBIC && filter != B200_RESIZE_BILINEAR) return B200_ERR_INVALID_ARG;
+    if (n > 0 && !geom) return B200_ERR_INVALID_ARG;
+    if (static_cast<long long>(n) * C > 0x7fffffffLL) return B200_ERR_UNSUPPORTED;
+    for (int i = 0; i < n; ++i) {
+        const int *g = geom + 9 * i;
+        if (g[8] != 0 && g[8] != 1) return B200_ERR_INVALID_ARG;
+        int rc = crop_check_geom(CropGeom{g[0], g[1], g[2], g[3], g[4], g[5], g[6], g[7], 0, 0, 0}, C, filter);
+        if (rc == B200_OK) rc = crop_check_geom(CropGeom{g[6], g[7], Ho, Wo, 0, 0, Ho, Wo, 0, 0, 0}, 1, filter);
+        if (rc != B200_OK) return rc;
+    }
+    return B200_OK;
+}
+
+struct RandomCropLayout {
+    std::vector<CropGeom> g1, g2;       // launch 1 (one per image, C channels), launch 2 (one per image and channel)
+    CropLayout l1, l2;
+    size_t off_l2 = 0, off_tmp = 0, bytes = 0;
+};
+static RandomCropLayout random_crop_layout(int n, const int *geom, const long long *offsets, int C, int Ho, int Wo, int filter) {
+    RandomCropLayout r;
+    r.g1.resize(n), r.g2.resize(static_cast<size_t>(n) * C);
+    long long tmp = 0;
+    for (int i = 0; i < n; ++i) {
+        const int *g = geom + 9 * i;
+        const int h = g[6], w = g[7];
+        r.g1[i] = CropGeom{g[0], g[1], g[2], g[3], g[4], g[5], h, w, 0, offsets ? offsets[i] : 0, tmp};
+        for (int c = 0; c < C; ++c)
+            r.g2[static_cast<size_t>(i) * C + c] = CropGeom{h, w, Ho, Wo, 0, 0, Ho, Wo, g[8], tmp + static_cast<long long>(c) * h * w,
+                                                            (static_cast<long long>(i) * C + c) * Ho * Wo};
+        tmp += round_up<long long>(static_cast<long long>(C) * h * w, 4);
+    }
+    r.l1 = crop_layout(r.g1, filter), r.l2 = crop_layout(r.g2, filter);
+    r.off_l2 = round_up<size_t>(r.l1.bytes, 256);
+    r.off_tmp = round_up<size_t>(r.off_l2 + r.l2.bytes, 256);
+    r.bytes = r.off_tmp + static_cast<size_t>(tmp);
+    return r;
 }
 
 }  // namespace b200
@@ -634,7 +839,7 @@ int b200_resize_u8(const uint8_t *in, uint8_t *out, long long planes, int H, int
 
 size_t b200_resize_crop_workspace_bytes(int n, const int *geom_host, int C, int Hc, int Wc, int filter) {
     if (n < 1 || crop_check(n, geom_host, C, Hc, Wc, filter) != B200_OK) return 0;
-    return crop_layout(n, geom_host, Hc, Wc, filter).bytes;
+    return crop_layout(crop_geoms(n, geom_host, nullptr, C, Hc, Wc), filter).bytes;
 }
 
 int b200_resize_crop_u8(const uint8_t *in, const long long *offsets_host, const int *geom_host, int n, int C, int Hc, int Wc,
@@ -648,77 +853,55 @@ int b200_resize_crop_u8(const uint8_t *in, const long long *offsets_host, const 
         if (offsets_host[i] < 0) return B200_ERR_INVALID_ARG;
         if (offsets_host[i] & 3) return B200_ERR_ALIGNMENT;
     }
-    const int tiles_x = ceil_div(Wc, kRcTW), tiles_y = ceil_div(Hc, kRcTH);
-    if (static_cast<long long>(n) * C * tiles_x * tiles_y > 0x7fffffffLL) return B200_ERR_UNSUPPORTED;
-    const CropLayout l = crop_layout(n, geom_host, Hc, Wc, filter);
+    const std::vector<CropGeom> g = crop_geoms(n, geom_host, offsets_host, C, Hc, Wc);
+    const long long ctas = crop_ctas(g, C);
+    if (ctas > 0x7fffffffLL) return B200_ERR_UNSUPPORTED;
+    const CropLayout l = crop_layout(g, filter);
     if (l.table_ints > 0x7fffffffULL) return B200_ERR_UNSUPPORTED;              // descriptors index the tables with int
     if (!workspace || workspace_bytes < l.bytes) return B200_ERR_WORKSPACE;
     // descriptors + tables, staged on the host and copied with one cudaMemcpyAsync (a pageable-source copy stages the host
     // data before it returns, so the vector may die at scope exit)
     std::vector<unsigned char> stage(l.bytes, 0);
-    int *tab = reinterpret_cast<int *>(stage.data() + l.off_tab);
-    std::vector<std::vector<int>> key_bounds(l.keys.size());
-    for (size_t k = 0; k < l.keys.size(); ++k) {
-        const CropAxisKey &key = l.keys[k];
-        std::vector<int> kk;
-        if (key.in_size == key.out_size) {
-            key_bounds[k].resize(static_cast<size_t>(key.count) * 2);
-            kk.assign(key.count, 1 << kResizePrecisionBits);
-            for (int i = 0; i < key.count; ++i) key_bounds[k][2 * i] = key.first + i, key_bounds[k][2 * i + 1] = 1;
-        } else {
-            resize_coeffs(key.in_size, key.out_size, filter, l.key_ks[k], key_bounds[k], kk, key.first, key.count);
-        }
-        std::memcpy(tab + l.key_off[k], key_bounds[k].data(), key_bounds[k].size() * 4);
-        std::memcpy(tab + l.key_off[k] + round_up<size_t>(static_cast<size_t>(key.count) * 2, 4), kk.data(), kk.size() * 4);
-    }
-    // staging plan per (horizontal, vertical) key pair: the sub-block that fits kRcSmemBudget and stages the fewest source
-    // bytes per output sample (then the larger one)
-    std::map<std::pair<int, int>, std::pair<CropDesc, double>> plans;
-    std::vector<std::pair<double, int>> order(n);                       // (staged bytes of the image, image)
-    std::vector<CropDesc> by_image(n);
-    size_t smem = 0;
-    for (int i = 0; i < n; ++i) {
-        const int hk = l.h_key[i], vk = l.v_key[i];
-        auto it = plans.find(std::make_pair(hk, vk));
-        if (it == plans.end()) {
-            CropDesc p{};
-            p.hb = l.key_off[hk], p.hk = l.key_off[hk] + static_cast<int>(round_up<size_t>(static_cast<size_t>(Wc) * 2, 4));
-            p.vb = l.key_off[vk], p.vk = l.key_off[vk] + static_cast<int>(round_up<size_t>(static_cast<size_t>(Hc) * 2, 4));
-            p.ksh = l.key_ks[hk], p.ksv = l.key_ks[vk];
-            double best = 0.0;
-            for (int sw = kRcTW; sw >= 4; sw /= 2) {
-                const int stride = round_up(resize_max_window(key_bounds[hk], Wc, sw), 4);
-                for (int sh = kRcTH; sh >= 1; sh /= 2) {
-                    const int rows = resize_max_window(key_bounds[vk], Hc, sh);
-                    if (crop_smem_bytes(sh, sw, p.ksh, p.ksv, rows, stride) > static_cast<size_t>(kRcSmemBudget)) continue;
-                    const double per_sample = static_cast<double>(rows) * stride / (static_cast<double>(sh) * sw);
-                    if (best == 0.0 || per_sample < best)
-                        best = per_sample, p.sub_h = sh, p.sub_w = sw, p.max_rows = rows, p.stride = stride;
-                }
-            }
-            if (best == 0.0) return B200_ERR_UNSUPPORTED;
-            it = plans.emplace(std::make_pair(hk, vk), std::make_pair(p, best)).first;
-        }
-        CropDesc d = it->second.first;
-        d.in_off = offsets_host[i], d.W = geom_host[6 * i + 1], d.img = i;
-        by_image[i] = d;
-        order[i] = std::make_pair(-it->second.second, i);
-        const size_t need = crop_smem_bytes(d.sub_h, d.sub_w, d.ksh, d.ksv, d.max_rows, d.stride);
-        if (need > smem) smem = need;
-    }
-    std::stable_sort(order.begin(), order.end());
-    CropDesc *descs = reinterpret_cast<CropDesc *>(stage.data());
-    for (int r = 0; r < n; ++r) descs[r] = by_image[order[r].second];
+    const size_t smem = crop_stage(g, C, filter, l, stage.data());
+    if (smem == 0) return B200_ERR_UNSUPPORTED;
     cudaStream_t st = as_stream(stream);
     unsigned char *w = static_cast<unsigned char *>(workspace);
     B200_CUDA_TRY(cudaMemcpyAsync(w, stage.data(), stage.size(), cudaMemcpyHostToDevice, st));
-    resize_crop_fn fn = resize_pick_crop(C);
-    B200_CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void *>(fn), cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       static_cast<int>(smem)));
-    fn<<<static_cast<unsigned>(static_cast<long long>(n) * C * tiles_x * tiles_y), kRcThreads, smem, st>>>(
-        in, out, reinterpret_cast<const CropDesc *>(w), reinterpret_cast<const int *>(w + l.off_tab), Hc, Wc, tiles_x, tiles_y);
-    B200_LAUNCH_CHECK("resize_crop_kernel");
-    return B200_OK;
+    return crop_launch(C, in, out, w, l.off_tab, g, ctas, smem, st);
+}
+
+size_t b200_resize_random_crop_workspace_bytes(int n, const int *geom_host, int C, int Ho, int Wo, int filter) {
+    if (n < 1 || random_crop_check(n, geom_host, C, Ho, Wo, filter) != B200_OK) return 0;
+    return random_crop_layout(n, geom_host, nullptr, C, Ho, Wo, filter).bytes;
+}
+
+int b200_resize_random_crop_u8(const uint8_t *in, const long long *offsets_host, const int *geom_host, int n, int C, int Ho,
+                               int Wo, int filter, uint8_t *out, void *workspace, size_t workspace_bytes, b200_stream_t stream) {
+    const int rc = random_crop_check(n, geom_host, C, Ho, Wo, filter);
+    if (rc != B200_OK) return rc;
+    if (n == 0) return B200_OK;
+    if (!in || !out || !offsets_host) return B200_ERR_INVALID_ARG;
+    if (reinterpret_cast<uintptr_t>(in) & 3) return B200_ERR_ALIGNMENT;
+    for (int i = 0; i < n; ++i) {
+        if (offsets_host[i] < 0) return B200_ERR_INVALID_ARG;
+        if (offsets_host[i] & 3) return B200_ERR_ALIGNMENT;
+    }
+    const RandomCropLayout r = random_crop_layout(n, geom_host, offsets_host, C, Ho, Wo, filter);
+    const long long ctas1 = crop_ctas(r.g1, C), ctas2 = crop_ctas(r.g2, 1);
+    if (ctas1 > 0x7fffffffLL || ctas2 > 0x7fffffffLL) return B200_ERR_UNSUPPORTED;
+    if (r.l1.table_ints > 0x7fffffffULL || r.l2.table_ints > 0x7fffffffULL) return B200_ERR_UNSUPPORTED;
+    if (!workspace || workspace_bytes < r.bytes) return B200_ERR_WORKSPACE;
+    // both launches' descriptors and tables in one staging buffer and one cudaMemcpyAsync; the intermediate follows them
+    std::vector<unsigned char> stage(r.off_l2 + r.l2.bytes, 0);
+    const size_t smem1 = crop_stage(r.g1, C, filter, r.l1, stage.data());
+    const size_t smem2 = crop_stage(r.g2, 1, filter, r.l2, stage.data() + r.off_l2);
+    if (smem1 == 0 || smem2 == 0) return B200_ERR_UNSUPPORTED;
+    cudaStream_t st = as_stream(stream);
+    unsigned char *w = static_cast<unsigned char *>(workspace);
+    B200_CUDA_TRY(cudaMemcpyAsync(w, stage.data(), stage.size(), cudaMemcpyHostToDevice, st));
+    const int rc1 = crop_launch(C, in, w + r.off_tmp, w, r.l1.off_tab, r.g1, ctas1, smem1, st);
+    if (rc1 != B200_OK) return rc1;
+    return crop_launch(1, w + r.off_tmp, out, w + r.off_l2, r.l2.off_tab, r.g2, ctas2, smem2, st);
 }
 
 }  // extern "C"

@@ -117,6 +117,23 @@ size_t b200_resize_crop_workspace_bytes(int n, const int *geom_host, int C, int 
 int b200_resize_crop_u8(const uint8_t *in, const long long *offsets_host, const int *geom_host, int n, int C, int Hc, int Wc,
                         int filter, uint8_t *out, void *workspace, size_t workspace_bytes, b200_stream_t stream);
 
+/* Resize + random resized crop + horizontal flip of a ragged batch: the training transform Resize(size) ->
+ * RandomResizedCrop(crop) -> RandomHorizontalFlip (config/transform/basic_swt.yaml) applied to every image, bit-identical
+ * to torchvision on PIL images for the boxes and flips it drew (the caller draws them with torchvision's RNG calls).
+ * in, offsets  : as b200_resize_crop_u8 (HWC uint8 images at 4-byte-aligned byte offsets of one device buffer).
+ * geom_host    : HOST int [n][9] = H, W, RH, RW, top, left, h, w, flip per image: the resized size (Pillow's Image.resize
+ *                with `filter`), the box inside it (0 <= top <= RH - h, 0 <= left <= RW - w; B200_ERR_INVALID_ARG
+ *                otherwise) and flip in {0, 1}.  The box of the resized image is rounded to uint8 and resized in full to
+ *                Ho x Wo (Pillow's Image.resize again), its columns mirrored when flip is 1.
+ * out          : device uint8 [n][C][Ho][Wo] (planar, the layout b200_swt2_fwd takes);  C in 1..4.
+ * workspace    : device scratch of b200_resize_random_crop_workspace_bytes(): the descriptors and weight tables of both
+ *                launches (built on the host per call, one H2D copy) and the planar uint8 boxes between them.
+ * B200_ERR_UNSUPPORTED when a window of either resize is wider than 64 taps.  All argument checks precede any CUDA call;
+ * n = 0 is a no-op; the workspace query returns 0 for n < 1 and for arguments the call rejects. */
+size_t b200_resize_random_crop_workspace_bytes(int n, const int *geom_host, int C, int Ho, int Wo, int filter);
+int b200_resize_random_crop_u8(const uint8_t *in, const long long *offsets_host, const int *geom_host, int n, int C, int Ho,
+                               int Wo, int filter, uint8_t *out, void *workspace, size_t workspace_bytes, b200_stream_t stream);
+
 /* ---- the decimated transform next to the SWT (SURVEY.md §8 f4)
  * DWTTransform._apply_wavelet, main/transforms/custom_transforms.py:196-200: pywt.wavedec2(channel, wavelet, level)
  * in PyWavelets' default 'symmetric' mode, keeping the coarsest level: out [planes][4][H_L][W_L] = (cA, cH, cV, cD),
