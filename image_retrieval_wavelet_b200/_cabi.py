@@ -52,6 +52,8 @@ SIGNATURES = {
     "b200_resize_random_crop_workspace_bytes": (c_size_t, [c_int, c_void_p, c_int, c_int, c_int, c_int]),
     "b200_resize_random_crop_u8": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p,
                                            c_size_t, c_void_p]),
+    "b200_jpeg_decode_workspace_bytes": (c_size_t, [c_void_p, c_void_p, c_size_t, c_int]),
+    "b200_jpeg_decode_u8": (c_int, [c_void_p, c_void_p, c_void_p, c_size_t, c_int, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "b200_dwt2_workspace_bytes": (c_size_t, [c_ll, c_int, c_int, c_int, c_int]),
     "b200_dwt2_fwd": (c_int, [c_void_p, c_int, c_void_p, c_ll, c_int, c_int, c_void_p, c_void_p, c_int, c_int, c_void_p, c_size_t,
                               c_void_p]),

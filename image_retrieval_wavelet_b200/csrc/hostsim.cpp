@@ -12,6 +12,7 @@
 #include "b200ret.h"
 #include "hamming_core.cuh"
 #include "hamming_plan.h"
+#include "jpeg_plan.h"
 #include "swt2_plan.h"
 
 namespace b200 {
@@ -389,6 +390,46 @@ int sim_ap_finalize(const uint64_t *sums, const uint32_t *hits, int n_parts, lon
         total += ap[q];
     }
     if (map_out) *map_out = Q ? total / Q : 0.0;
+    return B200_OK;
+}
+
+// b200_jpeg_decode_u8 on host buffers: the same planner and the same per-subsequence / block / pixel programs as the
+// three kernels, with subsequences of `sub_bits` bits (short ones make the synchronisation take several rounds).
+// *rounds_out: synchronisation rounds; *subs_out (may be NULL): subsequences.
+int sim_jpeg_decode(const uint8_t *in, const b200_jpeg_desc *desc, const void *tables, size_t tables_bytes, int n, uint8_t *out,
+                    const long long *out_offsets, unsigned sub_bits, int *rounds_out, long long *subs_out) {
+    JpegPlan p;
+    const int rc = jpeg_plan(desc, static_cast<const unsigned char *>(tables), tables_bytes, n, out_offsets, sub_bits, p);
+    if (rc != B200_OK) return rc;
+    std::vector<unsigned char> stage, ws(p.bytes, 0xCD);           // poison: only the cleared range may be relied on
+    std::memset(ws.data(), 0, p.zero_bytes);
+    jpeg_stage(p, static_cast<const unsigned char *>(tables), tables_bytes, stage);
+    std::memcpy(ws.data() + p.off_images, stage.data(), stage.size());
+    const JpegArgs a = jpeg_args(p, in, out, ws.data(), sub_bits);
+    for (long long i = 0; i < a.n_sub; ++i) jpeg_sub_init(a, i);
+    int rounds = 0;
+    for (bool changed = a.n_sub > 0; changed; ++rounds) {
+        for (long long i = 0; i < a.n_sub; ++i) jpeg_sub_speculate(a, i);
+        changed = false;
+        for (long long i = 0; i < a.n_sub; ++i) changed |= jpeg_sub_sync(a, i);
+    }
+    unsigned run[4] = {0, 0, 0, 0};
+    for (long long i = 0; i < a.n_sub; ++i)
+        for (int j = 0; j < 4; ++j) {
+            const unsigned t = a.sums[4 * i + j];
+            a.sums[4 * i + j] = run[j];
+            run[j] += t;
+        }
+    for (long long i = 0; i < a.n_sub; ++i) jpeg_sub_write(a, i);
+    for (long long g = 0; g < a.n_blocks; ++g) {
+        const JpegBlockRef r = jpeg_block(a, g);
+        int w[64];
+        for (int col = 0; col < 8; ++col) jpeg_idct_col(r.coef, r.q, col, w);
+        for (int row = 0; row < 8; ++row) jpeg_idct_row(w, row, r.dst + static_cast<size_t>(row) * r.pitch);
+    }
+    for (long long q = 0; q < a.n_pix; ++q) jpeg_out_pixel(a, q);
+    if (rounds_out) *rounds_out = rounds;
+    if (subs_out) *subs_out = a.n_sub;
     return B200_OK;
 }
 

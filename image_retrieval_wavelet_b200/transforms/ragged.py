@@ -247,9 +247,15 @@ def collate_ragged_train(samples, key="image", size=256, scale=(0.08, 1.0), rati
     identically seeded DataLoader gives the same boxes and flips.  Other parameters: ``functools.partial``."""
     batch = collate_ragged(samples, key)
     images = batch[key] if isinstance(batch, dict) else batch
-    params = [random_resized_crop_params(h, w, size, scale, ratio, p) + resized_size(h, w, size) for h, w in images.sizes.tolist()]
-    images.crop_params = torch.tensor(params, dtype=torch.int64).reshape(len(images), 7)
+    images.crop_params = draw_crop_params(images.sizes, size, scale, ratio, p)
     return batch
+
+
+def draw_crop_params(sizes, size=256, scale=(0.08, 1.0), ratio=(3 / 4, 4 / 3), p=0.5):
+    """``random_resized_crop_params`` and the resized size of every image of a batch (``sizes``: ``[B, 2]`` = H, W), drawn
+    in image order: the ``crop_params`` (int64 ``[B, 7]``) of a training batch."""
+    params = [random_resized_crop_params(h, w, size, scale, ratio, p) + resized_size(h, w, size) for h, w in sizes.tolist()]
+    return torch.tensor(params, dtype=torch.int64).reshape(len(params), 7)
 
 
 def resize_random_crop_flip(images, size=256, crop=224, interpolation="bilinear"):

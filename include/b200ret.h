@@ -134,6 +134,41 @@ size_t b200_resize_random_crop_workspace_bytes(int n, const int *geom_host, int 
 int b200_resize_random_crop_u8(const uint8_t *in, const long long *offsets_host, const int *geom_host, int n, int C, int Ho,
                                int Wo, int filter, uint8_t *out, void *workspace, size_t workspace_bytes, b200_stream_t stream);
 
+/* ---- JPEG decoding of a ragged batch: Image.open(f).convert("RGB") of Pillow (libjpeg-turbo, libjpeg 6.2 API) on every
+ * file, bit for bit: Huffman decode, dequantisation + integer "islow" IDCT, fancy upsampling and fixed-point YCbCr -> RGB.
+ * The caller (transforms/jpeg.py, in the DataLoader workers) parses the markers, builds the tables and strips byte stuffing
+ * and restart markers; files outside the envelope below arrive already decoded (kind B200_JPEG_RAW) and are copied.
+ * in           : device; image i's bytes at desc[i].in_offset: its clean entropy-coded segment (kind B200_JPEG_HUFFMAN)
+ *                or HWC RGB pixels (kind B200_JPEG_RAW, in_bytes = height * width * 3).
+ * desc_host    : HOST b200_jpeg_desc [n].  Huffman kind: 1 component (grayscale, written as R = G = B) or 3 YCbCr
+ *                components with component-0 sampling hmax x vmax in {1x1, 2x1, 2x2} and 1x1 chroma
+ *                (B200_ERR_UNSUPPORTED otherwise); restart_interval MCUs per interval (0: none).
+ * tables_host  : HOST block of tables_bytes the descriptors point into (byte offsets): Huffman records of 1024 bytes
+ *                (uint16 look[256] = (length << 8) | symbol per 8-bit prefix, int32 maxcode[18], int32 valoffset[18],
+ *                uint8 huffval[256]), quantisation records (uint16 [64], natural order) and per image the int64 byte
+ *                offsets of its restart intervals in its clean segment (the first is 0).
+ * out          : device; image i as HWC uint8 [height][width][3] at byte out_offsets_host[i].
+ * workspace    : device scratch of b200_jpeg_decode_workspace_bytes(): descriptors, tables, per-subsequence decoder
+ *                states, coefficients and sample planes; after the call its first uint32 holds the number of
+ *                synchronisation rounds the parallel Huffman decode took.
+ * All argument checks precede any CUDA call (B200_ERR_INVALID_ARG for inconsistent descriptors or tables); descriptors,
+ * intervals and tables go to the device in one cudaMemcpyAsync; n = 0 is a no-op; the workspace query returns 0 for
+ * n < 1 and for arguments the call rejects. */
+#define B200_JPEG_HUFFMAN 0
+#define B200_JPEG_RAW 1
+typedef struct b200_jpeg_desc {
+    long long kind, height, width;
+    long long in_offset, in_bytes;
+    long long ncomp, hmax, vmax;
+    long long restart_interval;
+    long long intervals;                 /* byte offset in tables of the interval starts           */
+    long long quant[3], dc[3], ac[3];    /* byte offsets in tables of each component's tables      */
+} b200_jpeg_desc;
+size_t b200_jpeg_decode_workspace_bytes(const b200_jpeg_desc *desc_host, const void *tables_host, size_t tables_bytes, int n);
+int b200_jpeg_decode_u8(const uint8_t *in, const b200_jpeg_desc *desc_host, const void *tables_host, size_t tables_bytes, int n,
+                        uint8_t *out, const long long *out_offsets_host, void *workspace, size_t workspace_bytes,
+                        b200_stream_t stream);
+
 /* ---- the decimated transform next to the SWT (SURVEY.md §8 f4)
  * DWTTransform._apply_wavelet, main/transforms/custom_transforms.py:196-200: pywt.wavedec2(channel, wavelet, level)
  * in PyWavelets' default 'symmetric' mode, keeping the coarsest level: out [planes][4][H_L][W_L] = (cA, cH, cV, cD),
