@@ -105,6 +105,7 @@ SIGNATURES = {
     "b200_comm_status_word": (c_void_p, [c_void_p]),
     "b200_comm_destroy": (c_int, [c_void_p]),
     "b200_select_topk_f32": (c_int, [c_void_p, c_int, c_ll, c_ll, c_int, c_int, c_void_p, c_void_p, c_void_p]),
+    "b200_real_hamming_dist": (c_int, [c_void_p, c_void_p, c_int, c_ll, c_int, c_int, c_void_p, c_ll, c_void_p]),
     "b200_maphashing_host_packed": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_ll, c_int, c_int, c_int, c_ll, c_void_p,
                                             c_void_p, c_void_p]),
     "b200_maphashing_host": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_ll, c_int, c_int, c_int, c_ll, c_void_p,

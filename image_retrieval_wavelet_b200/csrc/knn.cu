@@ -8,6 +8,8 @@
 // (tcgen05) scorer of knn_tc.cu replaces step (1), and where the shape allows (knn_fused_rank) filters candidates in its
 // epilogue instead of writing the matrix.  The exact path serves L2, B200_KNN_TC=0 and drivers without the tensor-map
 // encoder, and is the tensor-core path's parity reference.
+// The same scorer with the kEpiRealHamming epilogue is b200_real_hamming_dist: the reference's float32
+// 0.5 * (B - q @ r.T) of real-valued codes (accuracy_calculator.py:183-186), in a summation order a CPU oracle restates.
 #include <cmath>
 #include <cstdlib>
 
@@ -36,10 +38,19 @@ __global__ void __launch_bounds__(256) row_sqnorm_kernel(const float *__restrict
     if (lane == 0) out[warp] = s;
 }
 
-// S[q][n] = <Q[q], R[n]>   (l2: sqrt(max(|q|^2 + |r|^2 - 2<q,r>, 0)))     Q: [M][D], R: [N][D], D % 4 == 0; row stride ldS
+// Epilogue modes of knn_scores_kernel.  The mode is a template parameter so that kEpiScore (inner product, or L2 when
+// the runtime flag l2 is set) compiles to the same code whether or not the other mode exists.
+enum KnnEpilogue : int {
+    kEpiScore = 0,          // S = <q,r>   (l2: sqrt(max(|q|^2 + |r|^2 - 2<q,r>, 0)))
+    kEpiRealHamming = 1,    // S = 0.5f * ((float)nbits - <q,r>): calc_hamming_dist of real-valued codes
+};
+
+// S[q][n] from acc = <Q[q], R[n]>, one fmaf chain over the dimensions in index order (the k0 tiles, then kk ascending),
+// starting from +0.0f.     Q: [M][D], R: [N][D], D % 4 == 0; row stride ldS.  nbits: kEpiRealHamming only.
+template <int kEpi>
 __global__ void __launch_bounds__(256) knn_scores_kernel(const float *__restrict__ Qm, const float *__restrict__ Rm,
                                                          float *__restrict__ S, int M, long long N, long long ldS, int D, int l2,
-                                                         const float *__restrict__ qn, const float *__restrict__ rn) {
+                                                         const float *__restrict__ qn, const float *__restrict__ rn, float nbits) {
     __shared__ __align__(16) float As[kBK][kBM + 4];
     __shared__ __align__(16) float Bs[kBK][kBN + 4];
     const int tid = threadIdx.x;
@@ -90,7 +101,9 @@ __global__ void __launch_bounds__(256) knn_scores_kernel(const float *__restrict
             const long long n = n0 + tx * 8 + j;
             if (n >= N) continue;
             float v = acc[i][j];
-            if (l2) {
+            if (kEpi == kEpiRealHamming) {
+                v = __fmul_rn(0.5f, __fsub_rn(nbits, v));       // two roundings, as the reference's float32 ops
+            } else if (l2) {
                 const float d2 = qn[m] + rn[n] - 2.f * v;
                 v = d2 != d2 ? d2 : sqrtf(fmaxf(d2, 0.f));        // fmaxf would turn NaN into distance 0
             }
@@ -525,9 +538,24 @@ int b200_knn_topk(const float *refs, const float *queries, int Q, long long N, i
         B200_LAUNCH_CHECK("row_sqnorm_kernel");
     }
     const dim3 grid(static_cast<unsigned>(ceil_div<long long>(N, kBN)), ceil_div(Q, kBM));
-    knn_scores_kernel<<<grid, 256, 0, st>>>(queries, refs, S, Q, N, ldS, D, metric_l2, qn, rn);
+    knn_scores_kernel<kEpiScore><<<grid, 256, 0, st>>>(queries, refs, S, Q, N, ldS, D, metric_l2, qn, rn, 0.f);
     B200_LAUNCH_CHECK("knn_scores_kernel");
     return knn_select_passes(S, N, ldS, Q, k, metric_l2, idx, score, nullptr, st);
+}
+
+int b200_real_hamming_dist(const float *q, const float *db, int Q, long long N, int D, int nbits, float *dist, long long ldS,
+                           b200_stream_t stream) {
+    if (Q < 0 || N < 0 || D < 1 || nbits < 1 || nbits > D || ldS < N) return B200_ERR_INVALID_ARG;
+    if (Q > 0 && N > 0 && (!q || !db || !dist)) return B200_ERR_INVALID_ARG;
+    if ((D & 3) || ceil_div(Q, kBM) > 65535) return B200_ERR_UNSUPPORTED;
+    if ((ldS & 3) || ((reinterpret_cast<uintptr_t>(q) | reinterpret_cast<uintptr_t>(db) | reinterpret_cast<uintptr_t>(dist)) & 15))
+        return B200_ERR_ALIGNMENT;
+    if (Q == 0 || N == 0) return B200_OK;
+    const dim3 grid(static_cast<unsigned>(ceil_div<long long>(N, kBN)), ceil_div(Q, kBM));
+    knn_scores_kernel<kEpiRealHamming><<<grid, 256, 0, as_stream(stream)>>>(q, db, dist, Q, N, ldS, D, 0, nullptr, nullptr,
+                                                                             static_cast<float>(nbits));
+    B200_LAUNCH_CHECK("knn_scores_kernel");
+    return B200_OK;
 }
 
 }  // extern "C"

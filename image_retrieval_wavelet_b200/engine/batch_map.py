@@ -2,9 +2,13 @@
 fast-evaluation subset, :39-91).
 
 In training mode the reference feeds *raw logits* here (``multi_dino_attention.py:750`` only applies ``sign`` in eval
-mode), which makes its "Hamming distance" a real-valued proxy.  A bit-packed evaluator cannot represent that, so this
-mirror binarises explicitly (``on_nonbinary='sign'``: bit = logit > 0) — i.e. it reports the mAP the codes would have
-after ``sign()``.  That is a documented deviation (DESIGN.md §6), not a silent one.
+mode), which makes its "Hamming distance" a real-valued proxy, ``0.5 * (B - q @ r.T)`` in float32.
+``build_batch_map_calculator(..., on_nonbinary=...)`` picks how logits are ranked:
+
+* ``'sign'`` (default): binarise with bit = logit > 0 and rank by the packed Hamming distance — the mAP the codes would
+  have after ``sign()``, a documented deviation from the reference (DESIGN.md §1);
+* ``'real'``: rank by the reference's float32 distance (``hamming.real_hamming_map``), so ``compute_batch_map`` on raw
+  logits reports the reference's number; batches of exact +-1 codes still take the packed path.
 """
 import random
 
@@ -14,10 +18,10 @@ from .accuracy_calculator import CustomCalculator
 from .make_subset import make_subset
 
 
-def build_batch_map_calculator(distance_metric, device):
+def build_batch_map_calculator(distance_metric, device, on_nonbinary="sign"):
     metric_name = "maphashing" if distance_metric == "hamming" else "map"
     calculator = CustomCalculator(exclude=["NMI", "AMI"], k="max_bin_count", with_faiss=False,
-                                  distance_metric=distance_metric, device=device, on_nonbinary="sign")
+                                  distance_metric=distance_metric, device=device, on_nonbinary=on_nonbinary)
     return calculator, metric_name
 
 

@@ -45,7 +45,8 @@ def pack_codes(codes, device=None, on_nonbinary="raise"):
 
     Entries that are not exactly +1/-1 (``sign(0) == 0``, raw logits, NaN) have no Hamming distance in the reference's
     sense (its ``0.5 * (B - q @ r.T)`` turns fractional); ``on_nonbinary='raise'`` (default) rejects them with
-    ValueError, ``'sign'`` binarises with ``x > 0`` first.
+    ValueError, ``'sign'`` binarises with ``x > 0`` first, and ``'real'`` returns None for them (and for codes wider
+    than the packed format), so that the caller ranks the codes as floats (:func:`real_hamming_map`).
     """
     _cabi.require_cuda()
     t = _as_cuda(codes, device)
@@ -55,6 +56,8 @@ def pack_codes(codes, device=None, on_nonbinary="raise"):
     if b < 1:
         raise ValueError("codes need at least one bit")
     if b > _cabi.MAX_CODE_BITS:
+        if on_nonbinary == "real":
+            return None
         raise NotImplementedError(f"codes wider than {_cabi.MAX_CODE_BITS} bits are not supported")
     t = t.to(torch.float32).contiguous()
     cw = _cabi.code_words(b)
@@ -65,11 +68,13 @@ def pack_codes(codes, device=None, on_nonbinary="raise"):
         with torch.cuda.device(t.device):
             rc = _cabi.load().b200_pack_codes(_cabi.ptr(t), n, b, _cabi.ptr(words), _cabi.ptr(bad), _cabi.stream_ptr())
         _cabi.check(rc, "b200_pack_codes")
-        if on_nonbinary == "raise":
+        if on_nonbinary in ("raise", "real"):
             nbad = int(bad.item())
+            if nbad and on_nonbinary == "real":
+                return None
             if nbad:
                 raise ValueError(f"{nbad} code entries are not +-1: Hamming ranking is undefined for them "
-                                 "(binarise with torch.sign and resolve zeros, or pass on_nonbinary='sign')")
+                                 "(binarise with torch.sign and resolve zeros, or pass on_nonbinary='sign' or 'real')")
     return PackedCodes(words, n, b)
 
 
@@ -317,4 +322,92 @@ def ranked_ap(idx, ql, dl, query_mask=None):
         rc = _cabi.load().b200_ranked_ap(_cabi.ptr(idx), 1, q, k, _cabi.ptr(ql.words), _cabi.ptr(dl.words), ql.lw, ql.mode,
                                          _cabi.ptr(mask), _cabi.ptr(ap), _cabi.ptr(hits), _cabi.ptr(m), _cabi.stream_ptr())
     _cabi.check(rc, "b200_ranked_ap")
+    return m, ap, hits
+
+
+# ------------------------------------------------------------------------------------------------ real-valued codes
+REAL_CHUNK_BUDGET = 1 << 30     # bytes of per-chunk scratch of real_hamming_map: distances [chunk, ldS] + top-k lists
+
+
+def _real_codes(x, device=None):
+    """float32 ``[rows, D]`` on the device, columns zero-padded to D % 4 == 0 (zeros add nothing to the fmaf chain)."""
+    t = _as_cuda(x, device)
+    if t.dim() != 2:
+        raise ValueError("codes must be [N, B]")
+    t = t.to(torch.float32)
+    if t.shape[1] % 4:
+        t = torch.nn.functional.pad(t, (0, 4 - t.shape[1] % 4))
+    return t.contiguous()
+
+
+def _real_dist_into(qp, rp, nbits, out):
+    """``b200_real_hamming_dist`` of padded codes into ``out`` ``[Q, ldS]`` (columns ``[0, N)`` written)."""
+    with torch.cuda.device(out.device):
+        rc = _cabi.load().b200_real_hamming_dist(_cabi.ptr(qp), _cabi.ptr(rp), int(qp.shape[0]), int(rp.shape[0]), int(qp.shape[1]),
+                                                 int(nbits), _cabi.ptr(out), int(out.shape[1]), _cabi.stream_ptr())
+    _cabi.check(rc, "b200_real_hamming_dist")
+
+
+def real_hamming_dist(q, r, nbits):
+    """``calc_hamming_dist`` of real-valued codes: float32 ``[Q, N]`` = ``0.5 * (nbits - q @ r.T)`` as the reference
+    computes it in float32, with the inner product summed in dimension order (one fmaf chain, ``b200_real_hamming_dist``).
+    Raw logits, zeros, +-inf and NaN are all accepted; +-1 codes give the exact integer Hamming distances."""
+    _cabi.require_cuda()
+    qp = _real_codes(q)
+    rp = _real_codes(r, qp.device)
+    if qp.shape[1] != rp.shape[1]:
+        raise ValueError("code widths differ")
+    n = int(rp.shape[0])
+    ld = (n + 3) // 4 * 4
+    out = torch.empty((int(qp.shape[0]), ld), dtype=torch.float32, device=qp.device)
+    _real_dist_into(qp, rp, nbits, out)
+    return out if ld == n else out[:, :n]
+
+
+def real_hamming_map(q, ql, r, rl, k, chunk=None):
+    """mAP@k of real-valued codes ``q`` ``[Q, B]`` against ``r`` ``[N, B]`` ranked by :func:`real_hamming_dist` (B = the
+    code width), with packed labels ``ql`` / ``rl``: ``(map, ap [Q], hits [Q])`` device tensors like :func:`hamming_map`.
+
+    The ranking is ascending (distance, database index), NaN last.  Per chunk of queries: the distances into one
+    ``[chunk, ldS]`` buffer, ``b200_select_topk_f32`` (smallest first) on it, ``b200_ranked_ap`` on the index list; then one
+    ``b200_mean_f64`` over all queries, so no result depends on ``chunk``.  ``chunk`` (default: all queries) is capped so
+    that the per-chunk scratch stays within ``REAL_CHUNK_BUDGET``.  ``k``: None or > N means N; < 1 gives zeros."""
+    _cabi.require_cuda()
+    qp = _real_codes(q)
+    rp = _real_codes(r, qp.device)
+    nbits = int(torch.as_tensor(q).shape[1])
+    if qp.shape[1] != rp.shape[1]:
+        raise ValueError(f"query codes have {nbits} bits, database codes {int(torch.as_tensor(r).shape[1])}")
+    if ql.mode != rl.mode or ql.lw != rl.lw:
+        raise ValueError("query and database labels must both be multi-hot with the same width, or both 1-D")
+    nq, n = int(qp.shape[0]), int(rp.shape[0])
+    if ql.rows != nq or rl.rows != n:
+        raise ValueError("codes and labels must have the same number of rows")
+    if nq == 0:
+        raise ValueError("no queries")
+    dev = qp.device
+    ap = torch.zeros(nq, dtype=torch.float64, device=dev)
+    hits = torch.zeros(nq, dtype=torch.int32, device=dev)
+    m = torch.zeros((), dtype=torch.float64, device=dev)
+    k = n if k is None else min(int(k), n)
+    if k < 1:
+        return m, ap, hits
+    ld = (n + 3) // 4 * 4
+    per_row = 4 * ld + 12 * k                      # distances, int64 indices, float32 scores
+    c = max(1, min(nq if chunk is None else int(chunk), REAL_CHUNK_BUDGET // per_row))
+    dist = torch.empty((c, ld), dtype=torch.float32, device=dev)
+    idx = torch.empty((c, k), dtype=torch.int64, device=dev)
+    score = torch.empty((c, k), dtype=torch.float32, device=dev)
+    lib = _cabi.load()
+    with torch.cuda.device(dev):
+        for q0 in range(0, nq, c):
+            rows = min(c, nq - q0)
+            _real_dist_into(qp[q0:q0 + rows], rp, nbits, dist)
+            rc = lib.b200_select_topk_f32(_cabi.ptr(dist), rows, n, ld, k, 0, _cabi.ptr(idx), _cabi.ptr(score), _cabi.stream_ptr())
+            _cabi.check(rc, "b200_select_topk_f32")
+            rc = lib.b200_ranked_ap(_cabi.ptr(idx), 1, rows, k, _cabi.ptr(ql.words[q0:]), _cabi.ptr(rl.words), ql.lw, ql.mode,
+                                    None, _cabi.ptr(ap[q0:]), _cabi.ptr(hits[q0:]), None, _cabi.stream_ptr())
+            _cabi.check(rc, "b200_ranked_ap")
+        rc = lib.b200_mean_f64(_cabi.ptr(ap), None, nq, _cabi.ptr(m), _cabi.stream_ptr())
+    _cabi.check(rc, "b200_mean_f64")
     return m, ap, hits

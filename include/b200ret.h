@@ -413,6 +413,19 @@ int b200_comm_destroy(b200_comm *comm);
 int b200_select_topk_f32(const float *S, int Q, long long N, long long ldS, int k, int largest, int64_t *idx, float *score,
                          b200_stream_t stream);
 
+/* calc_hamming_dist of real-valued codes, accuracy_calculator.py:183-186: dist[q][n] = 0.5f * ((float)nbits - s) in
+ * float32, s = <q_q, db_n> accumulated as one fmaf chain over the dimensions 0 .. D-1 in index order, starting from +0.0f
+ * (a fixed order a CPU oracle restates; raw logits, sign(0) = 0, +-inf and NaN entries are all legal).  This is how
+ * calculate_maphashing ranks codes that are not all +-1: b200_select_topk_f32 (largest = 0) on `dist`, then
+ * b200_ranked_ap on the index list.
+ *   q float32 [Q][D], db float32 [N][D] device, 16-byte aligned; D % 4 == 0 (B200_ERR_UNSUPPORTED): the caller zero-pads
+ *   the columns nbits .. D-1.  nbits (1 <= nbits <= D) is the code width that enters the formula.
+ *   dist float32 [Q][ldS] device, ldS >= N; ldS % 4 == 0 and a 16-byte-aligned dist (B200_ERR_ALIGNMENT), so that the
+ *   result feeds b200_select_topk_f32 as it is.  Columns [0, N) of each row are written, nothing else.
+ * All argument checks precede any CUDA call; Q = 0 or N = 0 is a no-op.  No width limit besides D. */
+int b200_real_hamming_dist(const float *q, const float *db, int Q, long long N, int D, int nbits, float *dist, long long ldS,
+                           b200_stream_t stream);
+
 /* Host-buffer evaluator: CustomCalculator.calculate_maphashing as the reference calls it (float32 +-1 codes
  * and float32 labels in host memory).  labels: multi-hot [.,L] when label_mode == OVERLAP, [.,1] when EQUAL.
  * Does H2D, pack, the three stages and D2H; ap_out[Q] (may be NULL), *map_out = mean AP.
